@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- converged penalty-SQP problems per second (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B] [--dump-outputs DIR]
 
 Own arm (default): one "step" = one pass of the hot path (sco_solve_batch: closest feasible
 point, convexification, penalty-QP assembly, ADMM, merit / trust-region state machine) over a
@@ -268,6 +268,29 @@ def admm_flops(st, stats):
     return float(stats[:, 2].astype(np.float64).sum() * per_iter), per_iter
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 128  # what np.save puts before the data of a float64 array of up to two axes
+
+
+def dump_outputs(out_dir, batches):
+    """`--dump-outputs`: batches = {prefix: (problem numbers, {field: result array, one row per problem})} -> one
+    out_dir/<prefix><field>.npy per field, in float64 (the integer fields -- verdict, stats, nonconverged -- are exact in
+    it), and out_dir/<prefix>problem.npy, the problem number of every row.  If the files would exceed DUMP_LIMIT_BYTES
+    in all, every batch keeps the same share of its problems: a subset fixed by a seed, so that two runs with the same
+    arguments write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    files = sum(1 + len(fields) for _, fields in batches.values())
+    total = sum(8 * len(idx) * (1 + sum(a[:1].size for a in fields.values())) for idx, fields in batches.values())
+    share = min(1.0, (DUMP_LIMIT_BYTES - NPY_HEADER_BYTES * files) / total) if total else 1.0
+    for prefix, (idx, fields) in batches.items():
+        rows = np.arange(len(idx))
+        if share < 1.0:
+            rows = np.sort(np.random.default_rng(0).permutation(len(idx))[:int(len(idx) * share)])
+        np.save(os.path.join(out_dir, prefix + "problem.npy"), np.asarray(idx, dtype=np.float64)[rows])
+        for name, a in fields.items():
+            np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64)[rows])
+
+
 def load_peaks():
     try:
         return json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -422,7 +445,7 @@ def time_config(args, name, B, steps, warmup, dev, local, rank, world, dist, sam
     verdict, stats = host["verdict"], host["stats"]
     converged = reduce(float((verdict == 1).sum()), dist.ReduceOp.SUM if world > 1 else None)
     res = dict(st=st, eng=eng, host=host, ms_local=ms_local, ms_total=ms_total, clocks=clocks, converged=converged,
-               value=converged * steps / (ms_total * 1e-3), t_gen=t_gen, n_streams=n_streams, B=B)
+               value=converged * steps / (ms_total * 1e-3), t_gen=t_gen, n_streams=n_streams, B=B, first=shard * B)
 
     if e2e:
         # end-to-end: host buffers through the C ABI (sco_solve_batch_host_async), the H2D copy of every step's
@@ -554,6 +577,8 @@ def run_b200_arm(args):
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"": (main["first"] + np.arange(B), host)})
 
     import ctypes
     tf = ctypes.c_double(0.0)
@@ -736,6 +761,8 @@ def run_mixed(args):
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"bucket%d_" % bk["bucket"]: (bk["indices"], bk["host"]) for bk in buckets})
     per_rank = [a.cpu().tolist() for a in allt]
     ms_total = max(v[0] for v in per_rank)
     converged = sum(v[1] for v in per_rank)
@@ -852,7 +879,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU pass (audit and cpu_baseline)")
     ap.add_argument("--no-other-configs", action="store_true", help="skip detail.other_configs (C2 / C3)")
     ap.add_argument("--no-warm-start", action="store_true", help="skip detail.warm_start (the opt-in warm-start mode)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (rank 0's problems) as DIR/<name>.npy, float64, at "
+                         "most 64 MB in all, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's results; the reference arm has no timed steps")
     args.cpu_cores = args.cpu_cores or None
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1:

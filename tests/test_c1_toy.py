@@ -161,7 +161,7 @@ def test_oracle_reaches_the_reference_answers_sym(name):
     assert np.allclose(r["x"], x_true, atol=5e-4), (name, r["x"])
 
 
-@pytest.mark.skipif(not ref_builder.reference_available(), reason="/root/reference only exists in the build container")
+@pytest.mark.skipif(not ref_builder.reference_available(), reason="needs an upstream sco_py checkout at SCO_REFERENCE_ROOT")
 @pytest.mark.parametrize("name", ["prob1", "prob4", "prob7", "prob8"])
 def test_port_equals_the_unmodified_reference_on_black_box_objectives(name):
     """The unmodified reference (Solver.solve on the shims) on the same functions as Python callables."""
@@ -209,7 +209,7 @@ def test_vm_family_values_and_fd_jacobians_match_the_oracle(name):
 
 
 # ------------------------------------------------------------------ analytic derivatives (Expr(f, grad)) and the Hessian stage
-@pytest.mark.skipif(not ref_builder.reference_available(), reason="/root/reference only exists in the build container")
+@pytest.mark.skipif(not ref_builder.reference_available(), reason="needs an upstream sco_py checkout at SCO_REFERENCE_ROOT")
 @pytest.mark.parametrize("name", ["prob1", "prob4", "prob7", "prob8"])
 def test_port_equals_the_unmodified_reference_with_analytic_gradients(name):
     """The same functions handed to the unmodified reference as Expr(f, grad) with exact gradients."""

@@ -55,7 +55,7 @@ def test_groups_compile_to_masks_and_overlap():
     assert np.allclose(v, [sums[0], sums[0] + sums[1]])
 
 
-@pytest.mark.skipif(not ref_builder.reference_available(), reason="/root/reference only exists in the build container")
+@pytest.mark.skipif(not ref_builder.reference_available(), reason="needs an upstream sco_py checkout at SCO_REFERENCE_ROOT")
 @pytest.mark.parametrize("i", [0, 1, 2])
 def test_port_equals_the_unmodified_reference_with_groups(i):
     prob, _ = build(i)

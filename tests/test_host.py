@@ -85,6 +85,32 @@ def test_result_gather_world_size_2_gloo():
     assert res == [(0, True), (1, True)]
 
 
+def test_dump_outputs_writes_float64_rows_within_the_limit(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: every field as float64 with the problem number of each row; past the size limit the
+    same seeded subset of problems in every field and in every run."""
+    import bench
+    B = 1000
+    host = dict(x=np.random.default_rng(1).normal(size=(B, 20)), verdict=np.arange(B, dtype=np.int32) % 3 - 1,
+                stats=np.arange(4 * B, dtype=np.int32).reshape(B, 4))
+    bench.dump_outputs(str(tmp_path / "all"), {"": (500 + np.arange(B), host)})
+    for name, a in host.items():
+        d = np.load(tmp_path / "all" / (name + ".npy"))
+        assert d.dtype == np.float64 and np.array_equal(d, a)
+    assert np.array_equal(np.load(tmp_path / "all" / "problem.npy"), 500 + np.arange(B))
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 8 * 25 * B // 4)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"": (np.arange(B), host), "second_": (np.arange(B), host)})
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_LIMIT_BYTES
+    rows = np.load(tmp_path / "a" / "problem.npy").astype(int)
+    assert 0 < len(rows) < B
+    for f in files:
+        d = np.load(tmp_path / "a" / f)
+        assert np.array_equal(d, np.load(tmp_path / "b" / f))
+        if not f.endswith("problem.npy"):
+            assert np.array_equal(d, host[f[:-4].replace("second_", "")][rows])
+
+
 def test_reference_arm_prints_one_line_within_its_budget_single_and_under_torchrun():
     """`bench.py --impl reference` (the CPU arm the driver times next to the GPU arm): one JSON line with the contract's
     keys inside a wall-clock budget, also when the time runs out mid-problem; under torchrun rank 0 alone works and
