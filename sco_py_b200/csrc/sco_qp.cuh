@@ -706,23 +706,25 @@ struct QPSolver {
   //   ROLE 0: v = x zb yb, d = dx dyb          ROLE 1: v = z y, d = dy
   //   ROLE 2: v = zp yp s1 zs1 ys1 s2 zs2 ys2, d = dyp dss1 dys1 dss2 dys2
   template <int ROLE>
-  __device__ __noinline__ int fast_flush(int id, int act, int eq, int can_check, QPResult &res, double v0, double v1,
-                                         double v2, double v3, double v4, double v5, double v6, double v7, double d0,
-                                         double d1, double d2, double d3, double d4) {
+  // `store_d`: the deltas go to shared memory too -- at a tested iteration and at the last one, whose final tests
+  // (QPSolver::solve) evaluate the certificates on the deltas of that iteration, as OSQP does
+  __device__ __noinline__ int fast_flush(int id, int act, int eq, int can_check, int store_d, QPResult &res, double v0,
+                                         double v1, double v2, double v3, double v4, double v5, double v6, double v7,
+                                         double d0, double d1, double d2, double d3, double d4) {
     const QPW &wq = this->w;
     const int ms = this->ms;
     if (act) {
       if (ROLE == 0) {
         wq.x[id] = v0; wq.zb[id] = v1; wq.yb[id] = v2;
-        if (can_check) { wq.dxv[id] = d0; wq.dyb[id] = d1; }
+        if (store_d) { wq.dxv[id] = d0; wq.dyb[id] = d1; }
       } else if (ROLE == 1) {
         wq.zl[id] = v0; wq.yl[id] = v1;
-        if (can_check) wq.dyl[id] = d0;
+        if (store_d) wq.dyl[id] = d0;
       } else if (ROLE == 2) {
         wq.zp[id] = v0; wq.yp[id] = v1;
         wq.s[id] = v2; wq.zs[id] = v3; wq.ys[id] = v4;
         if (eq) { wq.s[ms + id] = v5; wq.zs[ms + id] = v6; wq.ys[ms + id] = v7; }
-        if (can_check) {
+        if (store_d) {
           wq.dyp[id] = d0; wq.dss[id] = d1; wq.dys[id] = d2;
           if (eq) { wq.dss[ms + id] = d3; wq.dys[ms + id] = d4; }
         }
@@ -1124,14 +1126,14 @@ struct QPSolver {
         }
       }
       // ---- the tested (and not waved through) or the last iteration.  Iterates (+ deltas) -> shared memory, then check().
-      const int can_check = tested ? 1 : 0;
+      const int can_check = tested ? 1 : 0, store_d = tested || iter >= max_iter ? 1 : 0;
 #ifdef SCO_TIMING
       long long tph = clock64();
 #endif
-      if (ROLE == 0) status = fast_flush<0>(id, act, 0, can_check, res, x, zb, yb, 0, 0, 0, 0, 0, d0, d1, 0, 0, 0);
-      else if (ROLE == 1) status = fast_flush<1>(id, act, 0, can_check, res, z, y, 0, 0, 0, 0, 0, 0, d0, 0, 0, 0, 0);
-      else if (PEN) status = fast_flush<2>(id, act, eq, can_check, res, z, y, s1, zs1, ys1, s2, zs2, ys2, d0, d1, d2, d3, d4);
-      else status = fast_flush<3>(id, 0, 0, can_check, res, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0);
+      if (ROLE == 0) status = fast_flush<0>(id, act, 0, can_check, store_d, res, x, zb, yb, 0, 0, 0, 0, 0, d0, d1, 0, 0, 0);
+      else if (ROLE == 1) status = fast_flush<1>(id, act, 0, can_check, store_d, res, z, y, 0, 0, 0, 0, 0, 0, d0, 0, 0, 0, 0);
+      else if (PEN) status = fast_flush<2>(id, act, eq, can_check, store_d, res, z, y, s1, zs1, ys1, s2, zs2, ys2, d0, d1, d2, d3, d4);
+      else status = fast_flush<3>(id, 0, 0, can_check, store_d, res, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0);
       checked = can_check != 0;
       SCO_PH(4)
       if (status != 0) break;
@@ -1261,6 +1263,8 @@ struct QPSolver {
       const bool can_check = st.check_termination && (iter % st.check_termination == 0);
       const bool do_rho = st.adaptive_rho && interval && (iter % interval == 0);
       const bool want_delta = can_check || do_rho;
+      // the deltas of the last iteration also feed the final tests after the loop (QPSolver::solve)
+      const bool keep_delta = want_delta || iter == st.max_iter;
 #ifdef SCO_TIMING
       long long tph = clock64();
 #endif
@@ -1335,7 +1339,7 @@ struct QPSolver {
         const double dy = W_rb[j] * (vv - zn);
         W_yb[j] += dy;
         W_zb[j] = zn;
-        if (want_delta) { W_dxv[j] = xn - xo; W_dyb[j] = dy; }
+        if (keep_delta) { W_dxv[j] = xn - xo; W_dyb[j] = dy; }
       }
       sync();
       SCO_PH(2)
@@ -1347,7 +1351,7 @@ struct QPSolver {
         const double dy = W_rl[r] * (vv - zn);
         W_yl[r] += dy;
         W_zl[r] = zn;
-        if (want_delta) W_dyl[r] = dy;
+        if (keep_delta) W_dyl[r] = dy;
       }
       for (int i = tid; i < m_nl; i += TEAM) {
         const double t = pen_row_dot(i, W_xt2);
@@ -1366,14 +1370,14 @@ struct QPSolver {
           const double dys = W_rs[si] * (vs - zns);
           W_ys[si] += dys;
           W_zs[si] = zns;
-          if (want_delta) { W_dss[si] = sn - so; W_dys[si] = dys; }
+          if (keep_delta) { W_dss[si] = sn - so; W_dys[si] = dys; }
         }
         const double vv = alpha * zt + oma * W_zp[i];
         const double zn = clampd(vv + W_yp[i] / W_rp[i], W_lp[i], W_up[i]);
         const double dy = W_rp[i] * (vv - zn);
         W_yp[i] += dy;
         W_zp[i] = zn;
-        if (want_delta) W_dyp[i] = dy;
+        if (keep_delta) W_dyp[i] = dy;
       }
       SCO_PH(3)
       checked = false;

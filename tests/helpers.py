@@ -86,21 +86,58 @@ def split_J(st, Jflat):
     return out
 
 
+def split_b(st, bflat):
+    """stored (m_nl,) offsets -> per block (m,)."""
+    out, r0 = [], 0
+    for blk in st.blocks:
+        out.append(np.asarray(bflat[r0:r0 + blk.m]))
+        r0 += blk.m
+    return out
+
+
+def masks_from_bits(st, bits):
+    """Frozen-sparsity mask words of one problem -> per block dense (m, n) bool masks.  `bits`: (m_nl,) or
+    (m_nl, words) 32-bit words, bit s of word s // 32 of row r <=> stored slot s of that row participates;
+    None switches every slot on."""
+    out, r0 = [], 0
+    for bi, blk in enumerate(st.blocks):
+        M = np.zeros((blk.m, st.n), dtype=bool)
+        cols = st.jac_cols(bi)
+        for r in range(blk.m):
+            for s in range(blk.jw):
+                if bits is None:
+                    M[r, cols[r, s]] = True
+                else:
+                    w = np.atleast_1d(np.asarray(bits[r0 + r]).astype(np.uint32))
+                    if (int(w[s // 32]) >> (s % 32)) & 1:
+                        M[r, cols[r, s]] = True
+        out.append(M)
+        r0 += blk.m
+    return out
+
+
+def stage_qp(st, row, Jflat, bflat, lbx, ubx, pi, kdup, bits=None):
+    """The penalty QP the device stage (Engine.qp_solve) solves for one problem, from the stored J / b and mask words
+    it is given, expanded to the (P, q, A, l, u) the reference hands to OSQP."""
+    return expand_qp(st, row, split_J(st, Jflat), split_b(st, bflat), masks_from_bits(st, bits), lbx, ubx, pi, kdup)
+
+
 def _port_job(job):
-    name, index, solver, quirks = job
+    name, index, solver, quirks, gen_kw, osqp_kw = job
     from sco_py_b200 import workloads as W
-    st, params, x0 = W.GENERATORS[name](1, first=index)
-    r = sqp_port.solve(st, params[0], x0[0], solver=solver, quirks=quirks)
+    st, params, x0 = W.GENERATORS[name](1, first=index, **gen_kw)
+    r = sqp_port.solve(st, params[0], x0[0], solver=solver, quirks=quirks, osqp_kw=osqp_kw)
     r.pop("trace", None)
     return index, r
 
 
-def port_solve_many(name, indices, solver, quirks=None, workers=None):
-    """The oracle port on problems `indices` of config `name`, one process per core (the port is single-threaded and
-    a heavy-tailed problem can take a minute).  -> {index: result}"""
+def port_solve_many(name, indices, solver, quirks=None, workers=None, gen_kw=None, osqp_kw=None):
+    """The oracle port on problems `indices` of config `name` (generator keywords `gen_kw`, e.g. a QCQP's n and m;
+    OSQP settings `osqp_kw`), one process per core (the port is single-threaded and a heavy-tailed problem can take
+    a minute).  -> {index: result}"""
     import multiprocessing as mp
     import os
-    jobs = [(name, int(i), solver, quirks) for i in indices]
+    jobs = [(name, int(i), solver, quirks, dict(gen_kw or {}), osqp_kw) for i in indices]
     workers = workers or min(len(jobs), os.cpu_count() or 1)
     if workers <= 1:
         return dict(_port_job(j) for j in jobs)

@@ -113,9 +113,8 @@ def test_wide_rows_convexify_and_masked_qp_stage(wide):
                                          mask=None if mask is None else mask.view(np.int32))
         xq, status, iters = xq.cpu().numpy(), status.cpu().numpy(), iters.cpu().numpy()
         for i in range(B):
-            Jd = helpers.split_J(st, Jn[i])
-            M = np.ones_like(Jd[0], dtype=bool) if mask is None else keep[i][:, :WIDE_N]
-            P, q, A, l, u = helpers.expand_qp(st, params[i], Jd, [bn[i]], [M], lbx[i], ubx[i], 10.0, 2)
+            P, q, A, l, u = helpers.stage_qp(st, params[i], Jn[i], bn[i], lbx[i], ubx[i], 10.0, 2,
+                                             bits=None if mask is None else mask[i])
             res = helpers.oracle_qp(P, q, A, l, u)
             assert status[i] == res.info.status_val and iters[i] == res.info.iter, (i, status[i], iters[i], res.info.iter)
             assert np.abs(xq[i] - res.x).max() <= 1e-7 * max(1.0, np.abs(res.x).max())
@@ -197,13 +196,7 @@ def test_large_structure_keeps_S_in_global_memory_qp_stage(big):
                                      kdup=np.full(B, 1, np.int32))
     xq, status, iters = xq.cpu().numpy(), status.cpu().numpy(), iters.cpu().numpy()
     for i in range(B):
-        Jd = helpers.split_J(st, Jn[i])
-        bl, r0 = [], 0
-        for blk in st.blocks:
-            bl.append(bn[i, r0:r0 + blk.m])
-            r0 += blk.m
-        masks = [np.ones_like(Jb, dtype=bool) for Jb in Jd]
-        P, q, A, l, u = helpers.expand_qp(st, params[i], Jd, bl, masks, lbx[i], ubx[i], 10.0, 1)
+        P, q, A, l, u = helpers.stage_qp(st, params[i], Jn[i], bn[i], lbx[i], ubx[i], 10.0, 1)
         res = helpers.oracle_qp(P, q, A, l, u)
         assert status[i] == res.info.status_val and iters[i] == res.info.iter, (i, status[i], iters[i], res.info.iter)
         assert np.abs(xq[i] - res.x).max() <= 1e-7 * max(1.0, np.abs(res.x).max())

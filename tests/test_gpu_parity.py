@@ -89,24 +89,9 @@ def test_qp_stage_matches_oracle(engines, name, kdup, pi, delta, masked):
                                      mask=None if bits is None else bits.view(np.int32))
     xq, status, iters = xq.cpu().numpy(), status.cpu().numpy(), iters.cpu().numpy()
     for i in range(B):
-        Jd = helpers.split_J(st, Jn[i])
-        bl, r0 = [], 0
-        for blk in st.blocks:
-            bl.append(bn[i, r0:r0 + blk.m])
-            r0 += blk.m
-        masks = [np.ones_like(Jb, dtype=bool) for Jb in Jd]
-        if masked:  # bit s of row r <=> stored slot s of that row participates
-            r0 = 0
-            for bi, blk in enumerate(st.blocks):
-                cols = st.jac_cols(bi)
-                M = np.zeros_like(masks[bi])
-                for r in range(blk.m):
-                    for s_ in range(blk.jw):
-                        if (int(bits[i, r0 + r]) >> s_) & 1:
-                            M[r, cols[r, s_]] = True
-                masks[bi] = M
-                r0 += blk.m
-        P, q, A, l, u = helpers.expand_qp(st, params[i], Jd, bl, masks, lbx[i], ubx[i], pi, kdup)
+        # bit s of row r <=> stored slot s of that row participates
+        P, q, A, l, u = helpers.stage_qp(st, params[i], Jn[i], bn[i], lbx[i], ubx[i], pi, kdup,
+                                         bits=None if bits is None else bits[i])
         res = helpers.oracle_qp(P, q, A, l, u)
         assert status[i] == res.info.status_val, (i, status[i], res.info.status_val, iters[i], res.info.iter)
         assert iters[i] == res.info.iter, (i, iters[i], res.info.iter)
@@ -251,13 +236,7 @@ def test_adaptive_rho_reaches_the_same_qp_optimum(engines):
                                          kdup=np.full(B, 2, np.int32))
         xq, status = xq.cpu().numpy(), status.cpu().numpy()
         for i in range(min(B, 3)):
-            Jd = helpers.split_J(st, Jn[i])
-            bl, r0 = [], 0
-            for blk in st.blocks:
-                bl.append(bn[i, r0:r0 + blk.m])
-                r0 += blk.m
-            masks = [np.ones_like(Jb, dtype=bool) for Jb in Jd]
-            P, q, A, l, u = helpers.expand_qp(st, params[i], Jd, bl, masks, lbx[i], ubx[i], 10.0, 2)
+            P, q, A, l, u = helpers.stage_qp(st, params[i], Jn[i], bn[i], lbx[i], ubx[i], 10.0, 2)
             res = helpers.oracle_qp(P, q, A, l, u, adaptive_rho=True)
             assert status[i] in (1, 2) and res.info.status_val in (1, 2), (name, i, status[i], res.info.status_val)
             assert np.abs(xq[i] - res.x).max() <= 1e-5 * max(1.0, np.abs(res.x).max()), (name, i)
