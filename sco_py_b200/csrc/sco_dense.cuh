@@ -63,11 +63,13 @@ __device__ __forceinline__ double dense_sc(const uint32_t sb, const int k) {
   return lds_f64(sb + 8u * (DenseL<NP, MP>::Sc + k));
 }
 
-// ---- termination test (OSQP check_termination on the unscaled residuals), both warps.
+// ---- termination test (OSQP check_termination on the unscaled residuals), both warps: the dense
+// layout's norms and certificate first stages, decided by qp_termination (sco_qp.cuh).
 // Expects Xs / Ys published and a barrier passed.  The lane passes the five constants its ADMM loop
 // keeps in registers; the rest comes from DL::LA / DL::Sc.  Returns 1 / 2 (solved / solved
 // inaccurate), -7, or 0; `want_cert` tells the caller which infeasibility certificates passed their
-// first stage (bit 0 primal, bit 1 dual) and have to be evaluated in full.
+// first stage (bit 0 primal, bit 1 dual) and have to be evaluated in full by dense_certificates, which
+// reads the reduced first stage from the per-warp slots of DL::Red this function leaves.
 template <int NP, int MP>
 __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp, const int lane,
                                           const double u0, const double u1, const double u2, const double lo,
@@ -177,23 +179,17 @@ __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp,
   const uint32_t r0a = sb + 8u * DL::Red;
   s0 = lds_f64(r0a + 48u) + lds_f64(r0a + 128u + 48u);
   s1 = lds_f64(r0a + 56u) + lds_f64(r0a + 128u + 56u);
-  const double f = approximate ? 10.0 : 1.0;
-  const double eps_abs = dense_sc<NP, MP>(sb, 0), eps_rel = dense_sc<NP, MP>(sb, 1);
-  const double c = dense_sc<NP, MP>(sb, 4), cinv = dense_sc<NP, MP>(sb, 5);
-  const double pri_res = v0, dua_res = cinv * v3;
-  pri_out = pri_res;
-  dua_out = dua_res;
-  want_cert = 0;
-  if (pri_res > OSQP_INFTY || dua_res > OSQP_INFTY) return -7;
-  const double eps_p = f * eps_abs + f * eps_rel * v12;
-  const double eps_d = f * eps_abs + f * eps_rel * cinv * v456;
-  const bool prim_ok = pri_res < eps_p, dual_ok = dua_res < eps_d;
-  if (prim_ok && dual_ok) return approximate ? 2 : 1;
-  const double epi = f * dense_sc<NP, MP>(sb, 2), edi = f * dense_sc<NP, MP>(sb, 3);
-  // first stage holds -- and, in tail mode, the lane-local part of the second stage does not refute it
-  if (!prim_ok && nvp > epi && s0 < -epi * nvp && !(tail && mvs >= epi * nvp)) want_cert |= 1;
-  if (!dual_ok && nvd > edi && s1 < -c * edi * nvd && !(tail && rej > edi * nvd)) want_cert |= 2;
-  return 0;
+  const double eps_pinf = dense_sc<NP, MP>(sb, 2), eps_dinf = dense_sc<NP, MP>(sb, 3);
+  const int status = qp_termination(v0, v12, v3, v456, nvp, s0, nvd, s1, dense_sc<NP, MP>(sb, 4), dense_sc<NP, MP>(sb, 5),
+                                    dense_sc<NP, MP>(sb, 0), dense_sc<NP, MP>(sb, 1), eps_pinf, eps_dinf, approximate,
+                                    pri_out, dua_out, want_cert);
+  // in tail mode, drop a certificate whose second stage the lane-local part already refutes
+  if (tail) {
+    const double f = approximate ? 10.0 : 1.0;
+    if (mvs >= f * eps_pinf * nvp) want_cert &= ~1;
+    if (rej > f * eps_dinf * nvd) want_cert &= ~2;
+  }
+  return status;
 }
 
 // ---- rare paths.  Both work on the iterates spilled to DL::Sp and rebuild the lane constants from
@@ -246,9 +242,10 @@ __device__ __forceinline__ void dense_team2(const uint32_t sb, const bool rowwar
   sm = lds_f64(r + 8u) + lds_f64(r + 136u);
 }
 
-// OSQP is_primal_infeasible / is_dual_infeasible on delta_y / delta_x of the last iteration.
-// Returns bit 0 = primal infeasible, bit 1 = dual infeasible.  Restates QPSolver::primal_infeasible /
-// dual_infeasible (sco_qp.cuh) for the dense layout.
+// Second stage of OSQP is_primal_infeasible / is_dual_infeasible on delta_y / delta_x of the last
+// iteration, for the certificates whose first stage dense_test found to hold (the dense layout's
+// QPSolver::primal_infeasible / dual_infeasible).  Returns bit 0 = primal infeasible, bit 1 = dual
+// infeasible.
 template <int NP, int MP>
 __device__ __noinline__ int dense_certificates(const uint32_t sb, const int n, const int m, const bool approximate,
                                                const bool need_p, const bool need_d) {
@@ -257,6 +254,11 @@ __device__ __noinline__ int dense_certificates(const uint32_t sb, const int n, c
   const int tid = threadIdx.x, lane = tid & 31;
   const bool rowwarp = tid < 32;
   const bool act = rowwarp ? lane < m : lane < n;
+  // |E dy|_inf and |D dx|_inf as dense_test reduced them (rows, then variables: dense_team2's order),
+  // read before dense_team2 reuses the slots
+  const uint32_t red = sb + 8u * DL::Red;
+  const double nvp = max_nn(lds_f64(red + 32u), lds_f64(red + 128u + 32u));
+  const double nvd = max_nn(lds_f64(red + 40u), lds_f64(red + 128u + 40u));
   DenseLane L;
   DenseState X;
   dense_reload<NP, MP>(sb, rowwarp, lane, L, X);
@@ -265,75 +267,62 @@ __device__ __noinline__ int dense_certificates(const uint32_t sb, const int n, c
   int res = 0;
   if (need_p) {
     const double eps = f * dense_sc<NP, MP>(sb, 2);
-    double nv, lhs, d1 = 0.0, d2 = 0.0, d3 = 0.0;
+    double d1 = 0.0, d2 = 0.0, d3 = 0.0;
     if (rowwarp) {
-      const double lpl = -OSQP_INFTY * L.e0, usmax = OSQP_INFTY * L.e1;
-      d1 = proj_dy(X.y0 - X.py0, lpl, L.hi); d2 = proj_dy(X.ys - X.pys, 0.0, usmax);
-      nv = max_nn(fabs(L.e0 * d1), fabs(L.e1 * d2));
-      lhs = kd * (L.hi * fmax(d1, 0.0) + lpl * fmin(d1, 0.0)) + usmax * fmax(d2, 0.0);
+      d1 = proj_dy(X.y0 - X.py0, -OSQP_INFTY * L.e0, L.hi); d2 = proj_dy(X.ys - X.pys, 0.0, OSQP_INFTY * L.e1);
       sts_f64(sb + 8u * (DL::Ys + lane), kd * d1);
     } else {
       d3 = proj_dy(X.y0 - X.py0, L.lo, L.hi);
-      nv = fabs(L.e0 * d3);
-      lhs = L.hi * fmax(d3, 0.0) + L.lo * fmin(d3, 0.0);
     }
-    dense_team2<NP, MP>(sb, rowwarp, lane, nv, lhs);  // its barriers also publish Ys
-    if (nv > eps && lhs < -eps * nv) {
-      double mv, dummy = 0.0;
-      if (rowwarp) {
-        mv = fabs((L.u1 * (kd * d1) + L.u2 * d2) * L.r2);
-      } else {
-        double t = 0.0;
-        for (int i = 0; i < MP; i++) t = fma(lds_f64(sb + 8u * (DL::Js + i * LDJ + (lane < NP ? lane : 0))), lds_f64(sb + 8u * (DL::Ys + i)), t);
-        mv = fabs((t + L.u1 * d3) * L.r1);
-      }
-      dense_team2<NP, MP>(sb, rowwarp, lane, mv, dummy);
-      if (mv < eps * nv) res |= 1;
+    __syncthreads();  // publishes Ys
+    double mv, dummy = 0.0;
+    if (rowwarp) {
+      mv = fabs((L.u1 * (kd * d1) + L.u2 * d2) * L.r2);
+    } else {
+      double t = 0.0;
+      for (int i = 0; i < MP; i++) t = fma(lds_f64(sb + 8u * (DL::Js + i * LDJ + (lane < NP ? lane : 0))), lds_f64(sb + 8u * (DL::Ys + i)), t);
+      mv = fabs((t + L.u1 * d3) * L.r1);
     }
+    dense_team2<NP, MP>(sb, rowwarp, lane, mv, dummy);
+    if (mv < eps * nvp) res |= 1;
   }
   if (need_d) {
     const double eps = f * dense_sc<NP, MP>(sb, 3);
-    double nv, qd, dx = 0.0, dss = 0.0;
+    double dx = 0.0, dss = 0.0;
     if (rowwarp) {
       dss = X.s - X.ps;
-      nv = fabs(L.e2 * dss);
-      qd = L.u0 * dss;
     } else {
       dx = X.p0 - X.pp0;
-      nv = fabs(L.e1 * dx);
-      qd = L.u0 * dx;
       sts_f64(sb + 8u * (DL::Xs + lane), dx);
     }
-    dense_team2<NP, MP>(sb, rowwarp, lane, nv, qd);  // publishes Xs = delta_x
-    const double thr = c * eps * nv;
-    if (nv > eps && qd < -thr) {
-      double pv = 0.0, dummy = 0.0;
-      if (!rowwarp) {  // |c Psym (D dx)|_j = |(Ph dx)_j / D_j|
+    __syncthreads();  // publishes Xs = delta_x
+    const double thr = c * eps * nvd;
+    double pv = 0.0, dummy = 0.0;
+    if (!rowwarp) {  // |c Psym (D dx)|_j = |(Ph dx)_j / D_j|
+      double t = 0.0;
+      for (int k = 0; k < NP; k++) t = fma(lds_f64(sb + 8u * (DL::Ph + k * NP + (lane < NP ? lane : 0))), lds_f64(sb + 8u * (DL::Xs + k)), t);
+      pv = fabs(t * L.r1);
+    }
+    dense_team2<NP, MP>(sb, rowwarp, lane, pv, dummy);
+    if (pv < thr) {
+      const double lim = eps * nvd;
+      double bad = 0.0;
+      if (rowwarp) {
         double t = 0.0;
-        for (int k = 0; k < NP; k++) t = fma(lds_f64(sb + 8u * (DL::Ph + k * NP + (lane < NP ? lane : 0))), lds_f64(sb + 8u * (DL::Xs + k)), t);
-        pv = fabs(t * L.r1);
+        for (int k = 0; k < NP; k++) t = fma(lds_f64(sb + 8u * (DL::Js + (lane < MP ? lane : 0) * LDJ + k)), lds_f64(sb + 8u * (DL::Xs + k)), t);
+        const double adx = (t + L.u1 * dss) * L.r0;
+        const double lpl = -OSQP_INFTY * L.e0, usmax = OSQP_INFTY * L.e1;
+        if (act && ((L.hi < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
+                    (lpl > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim))) bad = 1.0;
+        const double ads = L.u2 * dss * L.r1;  // slack row [0, +inf)
+        if (act && ((usmax < OSQP_INFTY * OSQP_MIN_SCALING && ads > lim) || ads < -lim)) bad = 1.0;
+      } else {
+        const double adx = L.u1 * dx * L.r0;
+        if (act && ((L.hi < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
+                    (L.lo > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim))) bad = 1.0;
       }
-      dense_team2<NP, MP>(sb, rowwarp, lane, pv, dummy);
-      if (pv < thr) {
-        const double lim = eps * nv;
-        double bad = 0.0;
-        if (rowwarp) {
-          double t = 0.0;
-          for (int k = 0; k < NP; k++) t = fma(lds_f64(sb + 8u * (DL::Js + (lane < MP ? lane : 0) * LDJ + k)), lds_f64(sb + 8u * (DL::Xs + k)), t);
-          const double adx = (t + L.u1 * dss) * L.r0;
-          const double lpl = -OSQP_INFTY * L.e0, usmax = OSQP_INFTY * L.e1;
-          if (act && ((L.hi < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
-                      (lpl > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim))) bad = 1.0;
-          const double ads = L.u2 * dss * L.r1;  // slack row [0, +inf)
-          if (act && ((usmax < OSQP_INFTY * OSQP_MIN_SCALING && ads > lim) || ads < -lim)) bad = 1.0;
-        } else {
-          const double adx = L.u1 * dx * L.r0;
-          if (act && ((L.hi < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
-                      (L.lo > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim))) bad = 1.0;
-        }
-        dense_team2<NP, MP>(sb, rowwarp, lane, bad, dummy);
-        if (bad == 0.0) res |= 2;
-      }
+      dense_team2<NP, MP>(sb, rowwarp, lane, bad, dummy);
+      if (bad == 0.0) res |= 2;
     }
   }
   __syncthreads();
@@ -785,32 +774,6 @@ __device__ __noinline__ QPResult dense_qp_solve(const DevStruct &S_, const DevSe
     __syncthreads();
     int cert;
     status = dense_test<NP, MP>(sb, rowwarp, lane, u0, u1, u2, lo, hi, X, false, tail, res.pri_res, res.dua_res, cert);
-#ifdef SCO_SKIP_PROBE
-    {  // experiment: how often would a lane-local lower bound of the primal residual already decide "not converged"?
-      const double r0p = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 5)), r1p = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 6));
-      double plb, vloc, dummy = 0.0;
-      if (rowwarp) {
-        const double axs = u2 * X.s;
-        plb = fabs((axs - X.zs) * r1p);
-        vloc = max_nn(fabs(X.z0 * r0p), max_nn(fabs(X.zs * r1p), fabs(axs * r1p)));
-      } else {
-        const double ax = u1 * X.p0;
-        plb = fabs((ax - X.z0) * r0p);
-        vloc = max_nn(fabs(X.z0 * r0p), fabs(ax * r0p));
-      }
-      double dlb = 0.0;
-      if (rowwarp) dlb = fabs((u0 + (lo * X.y0 + u2 * X.ys)) * lds_f64(dense_la<NP, MP>(sb, true, lane, 7))) * dense_sc<NP, MP>(sb, 5);
-      dense_team2<NP, MP>(sb, rowwarp, lane, dlb, dummy);
-      dense_team2<NP, MP>(sb, rowwarp, lane, plb, dummy);
-      dense_team2<NP, MP>(sb, rowwarp, lane, vloc, dummy);
-      if (status == 0 && (dlb >= 2.0 * dense_sc<NP, MP>(sb, 0))) res.cyc_c[4] += 1;  // slack-column dual bound alone
-      const double ep = (dense_sc<NP, MP>(sb, 0) + dense_sc<NP, MP>(sb, 1) * vloc) / (1.0 - dense_sc<NP, MP>(sb, 1)) * (1.0 + 1e-12);
-      res.cyc_c[0] += 1;                       // tests
-      if (status == 0) res.cyc_c[1] += 1;      // failing tests
-      if (status == 0 && (plb >= ep || dlb >= 2.0 * dense_sc<NP, MP>(sb, 0))) res.cyc_c[2] += 1;  // ... that the bounds decide
-      if (status != 0 && plb >= ep) res.cyc_c[3] += 1;  // must stay 0 (the bound is rigorous)
-    }
-#endif
     if (status != 0) break;
     if (cert) {
       dense_spill<NP, MP>(sb, rowwarp, lane, X);

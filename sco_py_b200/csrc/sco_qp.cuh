@@ -69,7 +69,76 @@ __device__ __forceinline__ double proj_dy(double dy, double l, double u) {
   return dy;
 }
 
+// OSQP check_termination on the team-reduced, unscaled norms, for every ADMM loop: pri_res, max(|z|, |Ax|), the dual
+// residual times c, max(|q|, |A'y|, |Px|), and the first stage of the primal (|E dy|_inf, u'dy+ + l'dy-) and of the dual
+// (|D dx|_inf, q'dx) infeasibility certificates.  Returns 1 / 2 (solved / solved inaccurate), -7 or 0; `cert` gets
+// bit 0 / bit 1 when the test failed on the primal / dual side and that certificate's first stage holds, so that
+// its second stage has to run.  `approximate`: all tolerances x10 (the last test at max_iter).
+__device__ __forceinline__ int qp_termination(double pri_res, double pri_scale, double dua_c, double dua_scale, double nvp,
+                                              double lhs, double nvd, double qd, double c, double cinv, double eps_abs,
+                                              double eps_rel, double eps_pinf, double eps_dinf, bool approximate,
+                                              double &pri_out, double &dua_out, int &cert) {
+  const double f = approximate ? 10.0 : 1.0;
+  const double ea = f * eps_abs, er = f * eps_rel, epi = f * eps_pinf, edi = f * eps_dinf;
+  const double dua_res = cinv * dua_c;
+  pri_out = pri_res;
+  dua_out = dua_res;
+  cert = 0;
+  if (pri_res > OSQP_INFTY || dua_res > OSQP_INFTY) return -7;
+  const double eps_p = ea + er * pri_scale;
+  const double eps_d = ea + er * cinv * dua_scale;
+  const bool prim_ok = pri_res < eps_p, dual_ok = dua_res < eps_d;
+  if (prim_ok && dual_ok) return approximate ? 2 : 1;
+  if (!prim_ok && nvp > epi && lhs < -epi * nvp) cert |= 1;
+  if (!dual_ok && nvd > edi && qd < -(c * edi * nvd)) cert |= 2;
+  return 0;
+}
+
 #include "sco_dense.cuh"
+
+// Per-entity terms of the termination test in the QPSolver mapping, accumulated into the caller's v[6] / sums[2]
+// as maxima of absolute values (exact in any order): v[0] pri_res, v[1] max(|z|, |Ax|), v[2] the dual residual,
+// v[3] max(|q|, |A'y|, |Px|) (each scaled back by E or D), v[4] / sums[0] the primal and v[5] / sums[1] the dual
+// certificate's first stage -- the arguments of qp_termination once the team has reduced them.
+// Unscaled primal residual terms of one row of A with scale E
+__device__ __forceinline__ void qp_term_pri(double *v, double ax, double z, double E) {
+  const double ei = 1.0 / E;
+  v[0] = fmax(v[0], fabs((ax - z) * ei)); v[1] = fmax(v[1], fmax(fabs(z * ei), fabs(ax * ei)));
+}
+// First stage of the dual certificate for one variable (scale D, linear cost q^) with step dx
+__device__ __forceinline__ void qp_term_dx(double *v, double *sums, double D, double dx, double q) {
+  v[5] = fmax(v[5], fabs(D * dx));
+  sums[1] += q * dx;
+}
+// A linear row (wt = 1) or a penalty row (wt = kd copies) [l, u] with its dual step dy
+__device__ __forceinline__ void qp_term_row(double *v, double *sums, double ax, double z, double E, double dy, double l,
+                                            double u, double wt) {
+  qp_term_pri(v, ax, z, E);
+  dy = proj_dy(dy, l, u);
+  v[4] = fmax(v[4], fabs(E * dy));
+  sums[0] += wt * (u * fmax(dy, 0.0) + l * fmin(dy, 0.0));
+}
+// A slack with its bound row [0, +inf): residuals and the primal certificate (qp_term_dx adds its dual one).
+// qs = c pi Ds, aty = kd sl yp + bs ys
+__device__ __forceinline__ void qp_term_slack(double *v, double *sums, double axs, double zs, double Es, double Ds,
+                                              double qs, double aty, double dys) {
+  qp_term_pri(v, axs, zs, Es);
+  const double di = 1.0 / Ds;
+  v[2] = fmax(v[2], fabs((qs + aty) * di)); v[3] = fmax(v[3], fmax(fabs(qs * di), fabs(aty * di)));
+  const double us = OSQP_INFTY * Es;
+  dys = proj_dy(dys, 0.0, us);
+  v[4] = fmax(v[4], fabs(Es * dys));
+  sums[0] += us * fmax(dys, 0.0);
+}
+// A variable with its box row [lb, ub]: ax = bx x, px = (P^ x)_j, aty = (A'y)_j including the box row
+__device__ __forceinline__ void qp_term_var(double *v, double *sums, double ax, double zb, double Eb, double D, double q,
+                                            double px, double aty, double dyb, double lb, double ub, double dx) {
+  qp_term_row(v, sums, ax, zb, Eb, dyb, lb, ub, 1.0);
+  const double di = 1.0 / D;
+  v[2] = fmax(v[2], fabs((q + px + aty) * di));
+  v[3] = fmax(v[3], fmax(fabs(q * di), fmax(fabs(aty * di), fabs(px * di))));
+  qp_term_dx(v, sums, D, dx, q);
+}
 
 template <int TEAM, int DK>
 struct QPSolver {
@@ -424,61 +493,38 @@ struct QPSolver {
 #define SM_GLOBAL (w.Sg != nullptr)
 
   // ================================================================== termination
-  // Returns a terminal status or 0.  Scratch: xt (D.*x), wp (kd*yp).  sc[] receives the scaled
-  // norms needed by the rho estimate: {|Ax-z|, |z|, |Ax|, |Px+q+A'y|, |q|, |A'y|, |Px|}.
+  // Returns a terminal status or 0.  Scratch: xt (D.*x), wp (kd*yp).  sc[], when given, receives the scaled
+  // norms needed by the rho estimate: {|Ax-z|, max(|z|, |Ax|), |Px+q+A'y|, max(|q|, |A'y|, |Px|)}.
   __device__ __noinline__ int check(int approximate, double &pri_res_out, double &dua_res_out, double *sc) {
     SCO_QP_LOCALS
-    double ea = st.eps_abs, er = st.eps_rel, epi = st.eps_prim_inf, edi = st.eps_dual_inf;
-    if (approximate) { ea *= 10; er *= 10; epi *= 10; edi *= 10; }
-    const double cinv = 1.0 / c;
-    // unscaled: v[0]=pri_res v[1]=|z/E| v[2]=|Ax/E| v[3]=dua_res*c v[4]=|q/D| v[5]=|A'y/D| v[6]=|Px/D|
-    // v[7], lhs: first stage of the primal-infeasibility certificate (|E dy|_inf, u'dy+ + l'dy-), v[8], qd: of the
-    // dual one (|D dx|_inf, q'dx) -- the quantities primal_infeasible / dual_infeasible start with, gathered in the
-    // same pass and the same reduction, so that those functions (loops + reductions of their own) only run when
-    // their first stage holds.  Same values, same order of accumulation, same decisions as calling them outright.
-    double v[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-    double u[7] = {0, 0, 0, 0, 0, 0, 0};
-    double sums[2] = {0.0, 0.0};  // lhs, qd
-    const bool cert = !sc;        // the rho update (sc) keeps the plain flow
+    // v[6], sums[2]: see qp_term_pri.  The per-thread order of the sums is the one the certificates' first stage is
+    // defined with: linear rows, penalty rows with their slacks, variables, then the slacks' dual-certificate terms.
+    double v[6] = {0, 0, 0, 0, 0, 0};
+    double u[4] = {0, 0, 0, 0};  // v[0..3] in the scaled problem, for the rho estimate
+    const bool rho_est = sc != nullptr;  // u only then: the loops get a version with fewer live values for the tests
+    double sums[2] = {0.0, 0.0};
     for (int r = tid; r < m_lin; r += TEAM) {
-      const double ax = lin_row_dot(r, W_x), ei = 1.0 / W_El[r], z = W_zl[r];
-      v[0] = fmax(v[0], fabs((ax - z) * ei)); v[1] = fmax(v[1], fabs(z * ei)); v[2] = fmax(v[2], fabs(ax * ei));
-      u[0] = fmax(u[0], fabs(ax - z)); u[1] = fmax(u[1], fabs(z)); u[2] = fmax(u[2], fabs(ax));
-      if (cert) {
-        const double dy = proj_dy(W_dyl[r], W_ll[r], W_ul[r]);
-        v[7] = fmax(v[7], fabs(W_El[r] * dy));
-        sums[0] += W_ul[r] * fmax(dy, 0.0) + W_ll[r] * fmin(dy, 0.0);
-      }
+      const double ax = lin_row_dot(r, W_x), z = W_zl[r];
+      qp_term_row(v, sums, ax, z, W_El[r], W_dyl[r], W_ll[r], W_ul[r], 1.0);
+      if (rho_est) { u[0] = fmax(u[0], fabs(ax - z)); u[1] = fmax(u[1], fmax(fabs(z), fabs(ax))); }
     }
     for (int i = tid; i < m_nl; i += TEAM) {
       const int eq = __ldg(S.row_eq + (i));
       double ax = pen_row_dot(i, W_x) + W_sl[i] * W_s[i];
       if (eq) ax += W_sl[ms + i] * W_s[ms + i];
-      double ei = 1.0 / W_Ep[i], z = W_zp[i];
-      v[0] = fmax(v[0], fabs((ax - z) * ei)); v[1] = fmax(v[1], fabs(z * ei)); v[2] = fmax(v[2], fabs(ax * ei));
-      u[0] = fmax(u[0], fabs(ax - z)); u[1] = fmax(u[1], fabs(z)); u[2] = fmax(u[2], fabs(ax));
-      if (cert) {
-        const double dy = proj_dy(W_dyp[i], W_lp[i], W_up[i]);
-        v[7] = fmax(v[7], fabs(W_Ep[i] * dy));
-        sums[0] += a.kd * (W_up[i] * fmax(dy, 0.0) + W_lp[i] * fmin(dy, 0.0));
-      }
+      const double z = W_zp[i];
+      qp_term_row(v, sums, ax, z, W_Ep[i], W_dyp[i], W_lp[i], W_up[i], a.kd);
+      if (rho_est) { u[0] = fmax(u[0], fabs(ax - z)); u[1] = fmax(u[1], fmax(fabs(z), fabs(ax))); }
       for (int k2 = 0; k2 <= eq; k2++) {
         const int si = k2 * ms + i;
-        const double axs = W_bs[si] * W_s[si];
-        ei = 1.0 / W_Es[si]; z = W_zs[si];
-        v[0] = fmax(v[0], fabs((axs - z) * ei)); v[1] = fmax(v[1], fabs(z * ei)); v[2] = fmax(v[2], fabs(axs * ei));
-        u[0] = fmax(u[0], fabs(axs - z)); u[1] = fmax(u[1], fabs(z)); u[2] = fmax(u[2], fabs(axs));
+        const double axs = W_bs[si] * W_s[si], zs = W_zs[si];
         // slack variable: q^ + A'y (its P block is zero)
-        const double di = 1.0 / W_Ds[si];
         const double qs = c * a.pi * W_Ds[si];
         const double aty = a.kd * W_sl[si] * W_yp[i] + W_bs[si] * W_ys[si];
-        v[3] = fmax(v[3], fabs((qs + aty) * di)); v[4] = fmax(v[4], fabs(qs * di)); v[5] = fmax(v[5], fabs(aty * di));
-        u[3] = fmax(u[3], fabs(qs + aty)); u[4] = fmax(u[4], fabs(qs)); u[5] = fmax(u[5], fabs(aty));
-        if (cert) {
-          const double us = OSQP_INFTY * W_Es[si];
-          const double dys = proj_dy(W_dys[si], 0.0, us);
-          v[7] = fmax(v[7], fabs(W_Es[si] * dys));
-          sums[0] += us * fmax(dys, 0.0);
+        qp_term_slack(v, sums, axs, zs, W_Es[si], W_Ds[si], qs, aty, W_dys[si]);
+        if (rho_est) {
+          u[0] = fmax(u[0], fabs(axs - zs)); u[1] = fmax(u[1], fmax(fabs(zs), fabs(axs)));
+          u[2] = fmax(u[2], fabs(qs + aty)); u[3] = fmax(u[3], fmax(fabs(qs), fabs(aty)));
         }
       }
     }
@@ -486,170 +532,114 @@ struct QPSolver {
     for (int j = tid; j < n; j += TEAM) W_xt[j] = W_D[j] * W_x[j];
     sync();
     for (int j = tid; j < n; j += TEAM) {
-      const double ax = W_bx[j] * W_x[j], ei = 1.0 / W_Eb[j], z = W_zb[j];
-      v[0] = fmax(v[0], fabs((ax - z) * ei)); v[1] = fmax(v[1], fabs(z * ei)); v[2] = fmax(v[2], fabs(ax * ei));
-      u[0] = fmax(u[0], fabs(ax - z)); u[1] = fmax(u[1], fabs(z)); u[2] = fmax(u[2], fabs(ax));
+      const double ax = W_bx[j] * W_x[j], z = W_zb[j];
       double px = psym_dot(j, W_xt);
       px *= c * W_D[j];
       const double aty = gatherAT(j, W_yl, W_wp) + W_bx[j] * W_yb[j];
-      const double di = 1.0 / W_D[j], q = W_qh[j];
-      v[3] = fmax(v[3], fabs((q + px + aty) * di)); v[4] = fmax(v[4], fabs(q * di));
-      v[5] = fmax(v[5], fabs(aty * di)); v[6] = fmax(v[6], fabs(px * di));
-      u[3] = fmax(u[3], fabs(q + px + aty)); u[4] = fmax(u[4], fabs(q)); u[5] = fmax(u[5], fabs(aty));
-      u[6] = fmax(u[6], fabs(px));
-      if (cert) {
-        const double dy = proj_dy(W_dyb[j], W_lb[j], W_ub[j]);
-        v[7] = fmax(v[7], fabs(W_Eb[j] * dy));
-        sums[0] += W_ub[j] * fmax(dy, 0.0) + W_lb[j] * fmin(dy, 0.0);
-        v[8] = fmax(v[8], fabs(W_D[j] * W_dxv[j]));
-        sums[1] += W_qh[j] * W_dxv[j];
+      const double q = W_qh[j];
+      qp_term_var(v, sums, ax, z, W_Eb[j], W_D[j], q, px, aty, W_dyb[j], W_lb[j], W_ub[j], W_dxv[j]);
+      if (rho_est) {
+        u[0] = fmax(u[0], fabs(ax - z)); u[1] = fmax(u[1], fmax(fabs(z), fabs(ax)));
+        u[2] = fmax(u[2], fabs(q + px + aty)); u[3] = fmax(u[3], fmax(fabs(q), fmax(fabs(aty), fabs(px))));
       }
     }
-    if (cert)
-      for (int i = tid; i < m_nl; i += TEAM)  // after the variables: the order dual_infeasible accumulates in
-        for (int k2 = 0; k2 <= __ldg(S.row_eq + (i)); k2++) {
-          const int si = k2 * ms + i;
-          v[8] = fmax(v[8], fabs(W_Ds[si] * W_dss[si]));
-          sums[1] += c * a.pi * W_Ds[si] * W_dss[si];
-        }
-    if (cert) {
-      Team<TEAM>::template reduce_mixed<9, 2>(v, sums, W_red);
-    } else {
-      double v7[7];
-      for (int k = 0; k < 7; k++) v7[k] = v[k];
-      Team<TEAM>::reduce_max(v7, W_red);
-      for (int k = 0; k < 7; k++) v[k] = v7[k];
+    for (int i = tid; i < m_nl; i += TEAM)
+      for (int k2 = 0; k2 <= __ldg(S.row_eq + (i)); k2++) {
+        const int si = k2 * ms + i;
+        qp_term_dx(v, sums, W_Ds[si], W_dss[si], c * a.pi * W_Ds[si]);
+      }
+    Team<TEAM>::template reduce_mixed<6, 2>(v, sums, W_red);
+    if (rho_est) {
       Team<TEAM>::reduce_max(u, W_red);
-      for (int k = 0; k < 7; k++) sc[k] = u[k];
+      for (int k = 0; k < 4; k++) sc[k] = u[k];
     }
-    const double pri_res = v[0], dua_res = cinv * v[3];
-    pri_res_out = pri_res;
-    dua_res_out = dua_res;
-    if (pri_res > OSQP_INFTY || dua_res > OSQP_INFTY) return -7;
-    const double eps_p = ea + er * fmax(v[1], v[2]);
-    const double eps_d = ea + er * cinv * fmax(v[4], fmax(v[5], v[6]));
-    const bool prim_ok = pri_res < eps_p, dual_ok = dua_res < eps_d;
-    if (prim_ok && dual_ok) return approximate ? 2 : 1;
-    bool pinf = false, dinf = false;
-    // the certificate functions re-derive their first stage; they are only entered when it holds (always, on the
-    // rho-update path, where it was not gathered)
-    if (!prim_ok && (!cert || (v[7] > epi && sums[0] < -epi * v[7]))) pinf = primal_infeasible(epi);
-    if (!dual_ok && (!cert || (v[8] > edi && sums[1] < -(c * edi * v[8])))) dinf = dual_infeasible(edi);
+    int cert;
+    const int status = qp_termination(v[0], v[1], v[2], v[3], v[4], sums[0], v[5], sums[1], c, 1.0 / c, st.eps_abs,
+                                      st.eps_rel, st.eps_prim_inf, st.eps_dual_inf, approximate != 0, pri_res_out,
+                                      dua_res_out, cert);
+    if (status != 0) return status;
+    const double f = approximate ? 10.0 : 1.0;
+    const bool pinf = (cert & 1) && primal_infeasible(f * st.eps_prim_inf, v[4]);
+    const bool dinf = (cert & 2) && dual_infeasible(f * st.eps_dual_inf, v[5]);
     if (pinf) return approximate ? 3 : -3;
     if (dinf) return approximate ? 4 : -4;
     return 0;
   }
 
-  // delta_y of the last iteration: dyl (lin), dyp (pen), dyb (x bounds), dys (slack bounds)
-  __device__ __noinline__ bool primal_infeasible(double eps) {
+  // Second stage of OSQP is_primal_infeasible on delta_y of the last iteration: dyl (lin), dyp (pen), dyb (x bounds),
+  // dys (slack bounds).  Entered when the first stage holds: nv = |E dy|_inf, reduced by check().
+  __device__ __noinline__ bool primal_infeasible(double eps, double nv) {
     SCO_QP_LOCALS
-    double nv[1] = {0.0}, lhs[1] = {0.0};
-    for (int r = tid; r < m_lin; r += TEAM) {
-      const double dy = proj_dy(W_dyl[r], W_ll[r], W_ul[r]);
-      W_dyl[r] = dy;
-      nv[0] = fmax(nv[0], fabs(W_El[r] * dy));
-      lhs[0] += W_ul[r] * fmax(dy, 0.0) + W_ll[r] * fmin(dy, 0.0);
-    }
+    for (int r = tid; r < m_lin; r += TEAM) W_dyl[r] = proj_dy(W_dyl[r], W_ll[r], W_ul[r]);
     for (int i = tid; i < m_nl; i += TEAM) {
       const double dy = proj_dy(W_dyp[i], W_lp[i], W_up[i]);
       W_dyp[i] = dy;
       W_wp[i] = a.kd * dy;
-      nv[0] = fmax(nv[0], fabs(W_Ep[i] * dy));
-      lhs[0] += a.kd * (W_up[i] * fmax(dy, 0.0) + W_lp[i] * fmin(dy, 0.0));
       for (int k2 = 0; k2 <= __ldg(S.row_eq + (i)); k2++) {
         const int si = k2 * ms + i;
-        const double us = OSQP_INFTY * W_Es[si];
-        const double dys = proj_dy(W_dys[si], 0.0, us);
-        W_dys[si] = dys;
-        nv[0] = fmax(nv[0], fabs(W_Es[si] * dys));
-        lhs[0] += us * fmax(dys, 0.0);
+        W_dys[si] = proj_dy(W_dys[si], 0.0, OSQP_INFTY * W_Es[si]);
       }
     }
-    for (int j = tid; j < n; j += TEAM) {
-      const double dy = proj_dy(W_dyb[j], W_lb[j], W_ub[j]);
-      W_dyb[j] = dy;
-      nv[0] = fmax(nv[0], fabs(W_Eb[j] * dy));
-      lhs[0] += W_ub[j] * fmax(dy, 0.0) + W_lb[j] * fmin(dy, 0.0);
-    }
-    Team<TEAM>::reduce_max(nv, W_red);
-    Team<TEAM>::reduce_sum(lhs, W_red);
+    for (int j = tid; j < n; j += TEAM) W_dyb[j] = proj_dy(W_dyb[j], W_lb[j], W_ub[j]);
     sync();
-    bool res = false;
-    if (nv[0] > eps && lhs[0] < -eps * nv[0]) {
-      double mv[1] = {0.0};
-      for (int j = tid; j < n; j += TEAM) {
-        const double aty = gatherAT(j, W_dyl, W_wp) + W_bx[j] * W_dyb[j];
-        mv[0] = fmax(mv[0], fabs(aty / W_D[j]));
-      }
-      for (int i = tid; i < m_nl; i += TEAM)
-        for (int k2 = 0; k2 <= __ldg(S.row_eq + (i)); k2++) {
-          const int si = k2 * ms + i;
-          const double aty = W_sl[si] * W_wp[i] + W_bs[si] * W_dys[si];
-          mv[0] = fmax(mv[0], fabs(aty / W_Ds[si]));
-        }
-      Team<TEAM>::reduce_max(mv, W_red);
-      res = mv[0] < eps * nv[0];
-    }
-    sync();
-    return res;
-  }
-
-  // delta_x of the last iteration: dxv (user variables), dss (slacks)
-  __device__ __noinline__ bool dual_infeasible(double eps) {
-    SCO_QP_LOCALS
-    double nv[1] = {0.0}, qd[1] = {0.0};
+    double mv[1] = {0.0};
     for (int j = tid; j < n; j += TEAM) {
-      nv[0] = fmax(nv[0], fabs(W_D[j] * W_dxv[j]));
-      qd[0] += W_qh[j] * W_dxv[j];
-      W_xt[j] = W_D[j] * W_dxv[j];
+      const double aty = gatherAT(j, W_dyl, W_wp) + W_bx[j] * W_dyb[j];
+      mv[0] = fmax(mv[0], fabs(aty / W_D[j]));
     }
     for (int i = tid; i < m_nl; i += TEAM)
       for (int k2 = 0; k2 <= __ldg(S.row_eq + (i)); k2++) {
         const int si = k2 * ms + i;
-        nv[0] = fmax(nv[0], fabs(W_Ds[si] * W_dss[si]));
-        qd[0] += c * a.pi * W_Ds[si] * W_dss[si];
+        const double aty = W_sl[si] * W_wp[i] + W_bs[si] * W_dys[si];
+        mv[0] = fmax(mv[0], fabs(aty / W_Ds[si]));
       }
-    Team<TEAM>::reduce_max(nv, W_red);
-    Team<TEAM>::reduce_sum(qd, W_red);
+    Team<TEAM>::reduce_max(mv, W_red);
+    sync();
+    return mv[0] < eps * nv;
+  }
+
+  // Second stage of OSQP is_dual_infeasible on delta_x of the last iteration: dxv (user variables), dss (slacks).
+  // Entered when the first stage holds: nv = |D dx|_inf, reduced by check().
+  __device__ __noinline__ bool dual_infeasible(double eps, double nv) {
+    SCO_QP_LOCALS
+    for (int j = tid; j < n; j += TEAM) W_xt[j] = W_D[j] * W_dxv[j];
     sync();
     bool res = false;
-    const double thr = c * eps * nv[0];
-    if (nv[0] > eps && qd[0] < -thr) {
-      double pv[1] = {0.0};
+    const double thr = c * eps * nv;
+    double pv[1] = {0.0};
+    for (int j = tid; j < n; j += TEAM) {
+      const double px = psym_dot(j, W_xt);
+      pv[0] = fmax(pv[0], fabs(c * px));  // Dinv .* (c D Psym D dx) = c * Psym (D dx)
+    }
+    Team<TEAM>::reduce_max(pv, W_red);
+    if (pv[0] < thr) {
+      const double lim = eps * nv;
+      double bad[1] = {0.0};
+      for (int r = tid; r < m_lin; r += TEAM) {
+        const double adx = lin_row_dot(r, W_dxv) / W_El[r];
+        if ((W_ul[r] < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
+            (W_ll[r] > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim)) bad[0] = 1.0;
+      }
+      for (int i = tid; i < m_nl; i += TEAM) {
+        double adx = pen_row_dot(i, W_dxv) + W_sl[i] * W_dss[i];
+        if (__ldg(S.row_eq + (i))) adx += W_sl[ms + i] * W_dss[ms + i];
+        adx /= W_Ep[i];
+        if ((W_up[i] < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
+            (W_lp[i] > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim)) bad[0] = 1.0;
+        for (int k2 = 0; k2 <= __ldg(S.row_eq + (i)); k2++) {
+          const int si = k2 * ms + i;
+          const double ads = W_bs[si] * W_dss[si] / W_Es[si];
+          if ((OSQP_INFTY * W_Es[si] < OSQP_INFTY * OSQP_MIN_SCALING && ads > lim) || ads < -lim)
+            bad[0] = 1.0;
+        }
+      }
       for (int j = tid; j < n; j += TEAM) {
-        const double px = psym_dot(j, W_xt);
-        pv[0] = fmax(pv[0], fabs(c * px));  // Dinv .* (c D Psym D dx) = c * Psym (D dx)
+        const double adx = W_bx[j] * W_dxv[j] / W_Eb[j];
+        if ((W_ub[j] < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
+            (W_lb[j] > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim)) bad[0] = 1.0;
       }
-      Team<TEAM>::reduce_max(pv, W_red);
-      if (pv[0] < thr) {
-        const double lim = eps * nv[0];
-        double bad[1] = {0.0};
-        for (int r = tid; r < m_lin; r += TEAM) {
-          const double adx = lin_row_dot(r, W_dxv) / W_El[r];
-          if ((W_ul[r] < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
-              (W_ll[r] > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim)) bad[0] = 1.0;
-        }
-        for (int i = tid; i < m_nl; i += TEAM) {
-          double adx = pen_row_dot(i, W_dxv) + W_sl[i] * W_dss[i];
-          if (__ldg(S.row_eq + (i))) adx += W_sl[ms + i] * W_dss[ms + i];
-          adx /= W_Ep[i];
-          if ((W_up[i] < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
-              (W_lp[i] > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim)) bad[0] = 1.0;
-          for (int k2 = 0; k2 <= __ldg(S.row_eq + (i)); k2++) {
-            const int si = k2 * ms + i;
-            const double ads = W_bs[si] * W_dss[si] / W_Es[si];
-            if ((OSQP_INFTY * W_Es[si] < OSQP_INFTY * OSQP_MIN_SCALING && ads > lim) || ads < -lim)
-              bad[0] = 1.0;
-          }
-        }
-        for (int j = tid; j < n; j += TEAM) {
-          const double adx = W_bx[j] * W_dxv[j] / W_Eb[j];
-          if ((W_ub[j] < OSQP_INFTY * OSQP_MIN_SCALING && adx > lim) ||
-              (W_lb[j] > -OSQP_INFTY * OSQP_MIN_SCALING && adx < -lim)) bad[0] = 1.0;
-        }
-        Team<TEAM>::reduce_max(bad, W_red);
-        res = bad[0] == 0.0;
-      }
+      Team<TEAM>::reduce_max(bad, W_red);
+      res = bad[0] == 0.0;
     }
     sync();
     return res;
@@ -1033,60 +1023,27 @@ struct QPSolver {
               else if (PEN) sco_smem[o_wp + id] = kd * y;
             }
             sync();
-            double v[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+            double v[6] = {0, 0, 0, 0, 0, 0};
             double sums[2] = {0.0, 0.0};
             if (act) {
-              if (ROLE == 1) {
+              if (ROLE == 1 || PEN) {
                 double ax = 0.0;
 #pragma unroll
                 for (int k = 0; k < SCO_EN; k++) ax = fma(ec[k], sco_smem[ea[k]], ax);
-                const double ei = 1.0 / k0;
-                v[0] = fabs((ax - z) * ei); v[1] = fabs(z * ei); v[2] = fabs(ax * ei);
-                const double dy = proj_dy(d0, lo, hi);
-                v[7] = fabs(k0 * dy);
-                sums[0] += hi * fmax(dy, 0.0) + lo * fmin(dy, 0.0);
-              } else if (PEN) {
-                double ax = 0.0;
-#pragma unroll
-                for (int k = 0; k < SCO_EN; k++) ax = fma(ec[k], sco_smem[ea[k]], ax);
-                ax = ax + sl1 * s1;
-                if (EQS && eq) ax += sl2 * s2;
-                double ei = 1.0 / k0;
-                v[0] = fabs((ax - z) * ei); v[1] = fabs(z * ei); v[2] = fabs(ax * ei);
-                {
-                  const double dy = proj_dy(d0, lo, hi);
-                  v[7] = fabs(k0 * dy);
-                  sums[0] += kd * (hi * fmax(dy, 0.0) + lo * fmin(dy, 0.0));
-                }
-                {
-                  const double axs = bs1 * s1;
-                  ei = 1.0 / k1;
-                  v[0] = fmax(v[0], fabs((axs - zs1) * ei)); v[1] = fmax(v[1], fabs(zs1 * ei)); v[2] = fmax(v[2], fabs(axs * ei));
-                  const double di = 1.0 / k2s;
-                  const double aty = kd * sl1 * y + bs1 * ys1;
-                  v[3] = fabs((cd1 + aty) * di); v[4] = fabs(cd1 * di); v[5] = fabs(aty * di);
-                  const double dys = proj_dy(d2, 0.0, us1);
-                  v[7] = fmax(v[7], fabs(k1 * dys));
-                  sums[0] += us1 * fmax(dys, 0.0);
-                  v[8] = fabs(k2s * d1);
-                  sums[1] += cd1 * d1;
-                }
-                if (EQS && eq) {
-                  const double axs = bs2 * s2;
-                  ei = 1.0 / k3;
-                  v[0] = fmax(v[0], fabs((axs - zs2) * ei)); v[1] = fmax(v[1], fabs(zs2 * ei)); v[2] = fmax(v[2], fabs(axs * ei));
-                  const double di = 1.0 / k4;
-                  const double aty = kd * sl2 * y + bs2 * ys2;
-                  v[3] = fmax(v[3], fabs((cd2 + aty) * di)); v[4] = fmax(v[4], fabs(cd2 * di)); v[5] = fmax(v[5], fabs(aty * di));
-                  const double dys = proj_dy(d4, 0.0, us2);
-                  v[7] = fmax(v[7], fabs(k3 * dys));
-                  sums[0] += us2 * fmax(dys, 0.0);
-                  v[8] = fmax(v[8], fabs(k4 * d3));
-                  sums[1] += cd2 * d3;
+                if (ROLE == 1) {
+                  qp_term_row(v, sums, ax, z, k0, d0, lo, hi, 1.0);
+                } else {
+                  ax = ax + sl1 * s1;
+                  if (EQS && eq) ax += sl2 * s2;
+                  qp_term_row(v, sums, ax, z, k0, d0, lo, hi, kd);
+                  qp_term_slack(v, sums, bs1 * s1, zs1, k1, k2s, cd1, kd * sl1 * y + bs1 * ys1, d2);
+                  qp_term_dx(v, sums, k2s, d1, cd1);
+                  if (EQS && eq) {
+                    qp_term_slack(v, sums, bs2 * s2, zs2, k3, k4, cd2, kd * sl2 * y + bs2 * ys2, d4);
+                    qp_term_dx(v, sums, k4, d3, cd2);
+                  }
                 }
               } else if (ROLE == 0) {
-                const double ax = bx * x, ei = 1.0 / k0;
-                v[0] = fabs((ax - zb) * ei); v[1] = fabs(zb * ei); v[2] = fabs(ax * ei);
                 double px = 0.0;
 #pragma unroll
                 for (int k = 0; k < 4; k++) px = fma(pq[k], sco_smem[pa[k]], px);
@@ -1098,27 +1055,17 @@ struct QPSolver {
                   accp = fma(ec[SCO_EH + k], sco_smem[ea[SCO_EH + k]], accp);
                 }
                 if (has_pen) acc += accp;
-                const double aty = acc + bx * yb;
-                const double di = 1.0 / k1;
-                v[3] = fabs((qh + px + aty) * di); v[4] = fabs(qh * di); v[5] = fabs(aty * di); v[6] = fabs(px * di);
-                const double dy = proj_dy(d1, lb, ub);
-                v[7] = fabs(k0 * dy);
-                sums[0] += ub * fmax(dy, 0.0) + lb * fmin(dy, 0.0);
-                v[8] = fabs(k1 * d0);
-                sums[1] += qh * d0;
+                qp_term_var(v, sums, bx * x, zb, k0, k1, qh, px, acc + bx * yb, d1, lb, ub, d0);
               }
             }
-            Team<TEAM>::template reduce_mixed<9, 2>(v, sums, Sh{f.o_red});
-            const double cinv = 1.0 / f.c;
-            const double pri_res = v[0], dua_res = cinv * v[3];
-            bool go_on = !(pri_res > OSQP_INFTY || dua_res > OSQP_INFTY);
-            const double eps_p = f.eps_abs + f.eps_rel * fmax(v[1], v[2]);
-            const double eps_d = f.eps_abs + f.eps_rel * cinv * fmax(v[4], fmax(v[5], v[6]));
-            const bool prim_ok = pri_res < eps_p, dual_ok = dua_res < eps_d;
-            if (prim_ok && dual_ok) go_on = false;
-            if (!prim_ok && v[7] > f.eps_pinf && sums[0] < -f.eps_pinf * v[7]) go_on = false;
-            if (!dual_ok && v[8] > f.eps_dinf && sums[1] < -(f.c * f.eps_dinf * v[8])) go_on = false;
-            if (go_on) { leave = false; tested = false; }
+            Team<TEAM>::template reduce_mixed<6, 2>(v, sums, Sh{f.o_red});
+            double pri_res, dua_res;
+            int cert;
+            if (qp_termination(v[0], v[1], v[2], v[3], v[4], sums[0], v[5], sums[1], f.c, 1.0 / f.c, f.eps_abs, f.eps_rel,
+                               f.eps_pinf, f.eps_dinf, false, pri_res, dua_res, cert) == 0 && cert == 0) {
+              leave = false;
+              tested = false;
+            }
             SCO_PH(4)
           }
         } else if (iter >= max_iter) {
@@ -1383,14 +1330,14 @@ struct QPSolver {
       checked = false;
       if (want_delta) {
         sync();
-        double sc[7];
+        double sc[4];
         status = check(0, res.pri_res, res.dua_res, do_rho ? sc : nullptr);
         checked = can_check;
         if (can_check && status != 0) break;
         status = 0;
         if (do_rho) {
-          double pri = sc[0] / (fmax(sc[1], sc[2]) + 1e-10);
-          double dua = sc[3] / (fmax(sc[4], fmax(sc[5], sc[6])) + 1e-10);
+          double pri = sc[0] / (sc[1] + 1e-10);
+          double dua = sc[2] / (sc[3] + 1e-10);
           double rn = rho * sqrt(pri / (dua + 1e-10));
           rn = fmin(fmax(rn, OSQP_RHO_MIN), OSQP_RHO_MAX);
           if (rn > rho * 5.0 || rn < rho / 5.0) {
