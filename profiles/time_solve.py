@@ -4,6 +4,12 @@ merit / objective / max_vio / x[:, 0:2] outputs carry cycle totals per problem:
 total, QP setup (scaling + factorisation), ADMM loop (incl. termination tests), termination tests,
 convexification.
     python profiles/time_solve.py [config] [batch]
+
+"Termination tests" counts what a test still exposes.  The dense loop (sco_dense.cuh) runs the first half of the
+test of iteration k beside iteration k+1; their shared barrier ends the ADMM-loop share.  The test's count runs
+from there to the decision, plus the certificates and the restore of iteration k, the test that ends the solve
+included.  Where the dense loop tests unpipelined (check_termination 1, or k+1 = max_iter), and in the other
+loops, it runs from the end of the tested iteration to the decision, the ending test excluded.
 """
 import os
 import sys

@@ -48,6 +48,15 @@ struct DenseLane {
   // variable lane: u0=q^ u1=bx u2=rho_j lo/hi=box   r0=1/Eb r1=1/D        e0=Eb e1=D
   // row lane     : u0=c pi Ds u1=sl u2=bs lo=kd sl hi=up r0=1/Ep r1=1/Es r2=1/Ds e0=Ep e1=Es e2=Ds
 };
+// proj_dy (sco_qp.cuh) with selects instead of branches, the same value in every case: l and u differ
+// from lane to lane, and a branch would split the basic block the dense loop overlaps with an ADMM
+// iteration (the generic loops keep the branches, which cost them fewer registers)
+__device__ __forceinline__ double proj_dy_sel(double dy, double l, double u) {
+  const bool u_inf = u > OSQP_INFTY * OSQP_MIN_SCALING, l_inf = l < -OSQP_INFTY * OSQP_MIN_SCALING;
+  const double upper_only = l_inf ? 0.0 : fmin(dy, 0.0), lower_only = l_inf ? fmax(dy, 0.0) : dy;
+  return u_inf ? upper_only : lower_only;
+}
+template <bool B> struct BoolC { static constexpr bool value = B; };  // a compile-time flag passed to a generic lambda
 struct DenseState {
   double p0, z0, y0, s, zs, ys;   // (x, zb, yb) or (-, zp, yp, s, zs, ys)
   double pp0, py0, ps, pys;       // the same before the last iteration
@@ -65,20 +74,24 @@ __device__ __forceinline__ double dense_sc(const uint32_t sb, const int k) {
 
 // ---- termination test (OSQP check_termination on the unscaled residuals), both warps: the dense
 // layout's norms and certificate first stages, decided by qp_termination (sco_qp.cuh).
-// Expects Xs / Ys published and a barrier passed.  The lane passes the five constants its ADMM loop
-// keeps in registers; the rest comes from DL::LA / DL::Sc.  Returns 1 / 2 (solved / solved
-// inaccurate), -7, or 0; `want_cert` tells the caller which infeasibility certificates passed their
-// first stage (bit 0 primal, bit 1 dual) and have to be evaluated in full by dense_certificates, which
-// reads the reduced first stage from the per-warp slots of DL::Red this function leaves.
-template <int NP, int MP>
-__device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp, const int lane,
-                                          const double u0, const double u1, const double u2, const double lo,
-                                          const double hi, const DenseState &X, const bool approximate,
-                                          const bool tail, double &pri_out, double &dua_out, int &want_cert) {
+//
+// First half, one warp (ROW: the penalty-row warp): this lane's terms of state X (dense_test_terms),
+// then their reduction over the warp, which lane 0 stores into the warp's slots of DL::Red
+// (dense_test_publish).  Expects Xs / Ys of state X published and a barrier passed.  The lane passes
+// the five constants its ADMM loop keeps in registers; the rest comes from DL::LA / DL::Sc.  Nothing in
+// it depends on the ADMM iterates in registers, so the dense loop runs it beside the next iteration
+// (dense_qp_solve) and one barrier publishes both.
+struct DenseTestTerms {
+  double v0, v12, v3, v456, nvp, nvd, s0, s1, mvs, rej;
+};
+template <int NP, int MP, bool ROW>
+__device__ __forceinline__ DenseTestTerms dense_test_terms(const uint32_t sb, const int lane, const double u0,
+                                                           const double u1, const double u2, const double lo,
+                                                           const double hi, const DenseState &X, const bool tail) {
   using DL = DenseL<NP, MP>;
   constexpr int LDJ = DL::LDJ;
-  const double r0 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 5)), r1 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 6));
-  const double e0 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 8)), e1 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 9));
+  const double r0 = lds_f64(dense_la<NP, MP>(sb, ROW, lane, 5)), r1 = lds_f64(dense_la<NP, MP>(sb, ROW, lane, 6));
+  const double e0 = lds_f64(dense_la<NP, MP>(sb, ROW, lane, 8)), e1 = lds_f64(dense_la<NP, MP>(sb, ROW, lane, 9));
   const double kd = dense_sc<NP, MP>(sb, 8);
   double v0, v12, v3, v456, nvp, nvd, s0, s1;
   // Tail mode (the launch's queue is drained, this problem is on the critical path): lane-local parts of
@@ -88,13 +101,13 @@ __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp,
   // almost none of them needs dense_certificates (a lone problem runs 7 % faster; on a full machine the
   // extra instructions cost 4 %, hence only in tail mode -- profiles/README.md).
   double mvs = 0.0, rej = 0.0;
-  if (rowwarp) {
+  if (ROW) {
     const double r2 = lds_f64(dense_la<NP, MP>(sb, true, lane, 7)), e2 = lds_f64(dense_la<NP, MP>(sb, true, lane, 10));
     // lanes beyond the padded row / column count read row / column 0: what lies behind the matrices may
     // be stale shared memory (a NaN pattern times their zero scale factor would still be NaN)
     const uint32_t jr = sb + 8u * (DL::Js + (lane < MP ? lane : 0) * LDJ), xs = sb + 8u * DL::Xs;
     double a0 = 0.0, a1 = 0.0;
-#pragma unroll 2
+#pragma unroll
     for (int k = 0; k < NP; k += 2) {
       const double2 xk = lds_v2(xs + 8u * k);
       a0 = fma(lds_f64(jr + 8u * k), xk.x, a0);
@@ -104,14 +117,14 @@ __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp,
     v0 = fabs((ax - X.z0) * r0);
     v12 = max_nn(fabs(X.z0 * r0), fabs(ax * r0));
     const double axs = u2 * X.s;
-    v0 = max_nn(v0, fabs((axs - X.zs) * r1));
+    v0 = max_nn(v0, fabs(__dsub_rn(axs, X.zs) * r1));
     v12 = max_nn(v12, max_nn(fabs(X.zs * r1), fabs(axs * r1)));
     const double aty = lo * X.y0 + u2 * X.ys;
     v3 = fabs((u0 + aty) * r2);
     v456 = max_nn(fabs(u0 * r2), fabs(aty * r2));
     // first stage of the certificates, lane-local part
     const double lpl = -OSQP_INFTY * e0, usmax = OSQP_INFTY * e1;
-    const double d1 = proj_dy(X.y0 - X.py0, lpl, hi), d2 = proj_dy(X.ys - X.pys, 0.0, usmax);
+    const double d1 = proj_dy_sel(X.y0 - X.py0, lpl, hi), d2 = proj_dy_sel(X.ys - X.pys, 0.0, usmax);
     nvp = max_nn(fabs(e0 * d1), fabs(e1 * d2));
     s0 = kd * (hi * fmax(d1, 0.0) + lpl * fmin(d1, 0.0)) + usmax * fmax(d2, 0.0);
     const double dss = X.s - X.ps;
@@ -127,16 +140,16 @@ __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp,
     const uint32_t pc = sb + 8u * (DL::Ph + col), jc = sb + 8u * (DL::Js + col);
     const uint32_t xs = sb + 8u * DL::Xs, ys = sb + 8u * DL::Ys;
     const double ax = u1 * X.p0;
-    v0 = fabs((ax - X.z0) * r0);
+    v0 = fabs(__dsub_rn(ax, X.z0) * r0);
     v12 = max_nn(fabs(X.z0 * r0), fabs(ax * r0));
     double p0 = 0.0, p1 = 0.0, t0 = 0.0, t1 = 0.0;
-#pragma unroll 2
+#pragma unroll
     for (int k = 0; k < NP; k += 2) {
       const double2 xk = lds_v2(xs + 8u * k);
       p0 = fma(lds_f64(pc + 8u * (k * NP)), xk.x, p0);
       if (k + 1 < NP) p1 = fma(lds_f64(pc + 8u * ((k + 1) * NP)), xk.y, p1);
     }
-#pragma unroll 2
+#pragma unroll
     for (int i = 0; i < MP; i += 2) {
       const double2 yi = lds_v2(ys + 8u * i);
       t0 = fma(lds_f64(jc + 8u * (i * LDJ)), yi.x, t0);
@@ -145,7 +158,7 @@ __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp,
     const double px = p0 + p1, aty = (t0 + t1) + u1 * X.y0;
     v3 = fabs((u0 + px + aty) * r1);
     v456 = max_nn(fabs(u0 * r1), max_nn(fabs(aty * r1), fabs(px * r1)));
-    const double d3 = proj_dy(X.y0 - X.py0, lo, hi);
+    const double d3 = proj_dy_sel(X.y0 - X.py0, lo, hi);
     nvp = fabs(e0 * d3);
     s0 = hi * fmax(d3, 0.0) + lo * fmin(d3, 0.0);
     const double dx = X.p0 - X.pp0;
@@ -156,29 +169,47 @@ __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp,
       rej = max_nn(hi < OSQP_INFTY * OSQP_MIN_SCALING ? adx : 0.0, max_nn(lo > -OSQP_INFTY * OSQP_MIN_SCALING ? -adx : 0.0, 0.0));
     }
   }
-  // one combined team reduction
-  v0 = warp_max_nonneg(v0); v12 = warp_max_nonneg(v12); v3 = warp_max_nonneg(v3);
-  v456 = warp_max_nonneg(v456); nvp = warp_max_nonneg(nvp); nvd = warp_max_nonneg(nvd);
-  if (tail) { mvs = warp_max_nonneg(mvs); rej = warp_max_nonneg(rej); }
+  return DenseTestTerms{v0, v12, v3, v456, nvp, nvd, s0, s1, mvs, rej};
+}
+template <int NP, int MP, bool ROW>
+__device__ __forceinline__ void dense_test_publish(const uint32_t sb, const int lane, DenseTestTerms t, const bool tail) {
+  using DL = DenseL<NP, MP>;
+  // one combined warp reduction
+  t.v0 = warp_max_nonneg(t.v0); t.v12 = warp_max_nonneg(t.v12); t.v3 = warp_max_nonneg(t.v3);
+  t.v456 = warp_max_nonneg(t.v456); t.nvp = warp_max_nonneg(t.nvp); t.nvd = warp_max_nonneg(t.nvd);
+  if (tail) { t.mvs = warp_max_nonneg(t.mvs); t.rej = warp_max_nonneg(t.rej); }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
-    s0 += __shfl_xor_sync(0xffffffffu, s0, o);
-    s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+    t.s0 += __shfl_xor_sync(0xffffffffu, t.s0, o);
+    t.s1 += __shfl_xor_sync(0xffffffffu, t.s1, o);
   }
-  const uint32_t mine = sb + 8u * (DL::Red + (rowwarp ? 0 : 16)), other = sb + 8u * (DL::Red + (rowwarp ? 16 : 0));
+  const uint32_t mine = sb + 8u * (DL::Red + (ROW ? 0 : 16));
   if (lane == 0) {
-    sts_f64(mine, v0); sts_f64(mine + 8u, v12); sts_f64(mine + 16u, v3); sts_f64(mine + 24u, v456);
-    sts_f64(mine + 32u, nvp); sts_f64(mine + 40u, nvd); sts_f64(mine + 48u, s0); sts_f64(mine + 56u, s1);
-    if (tail) { sts_f64(mine + 64u, mvs); sts_f64(mine + 72u, rej); }
+    sts_f64(mine, t.v0); sts_f64(mine + 8u, t.v12); sts_f64(mine + 16u, t.v3); sts_f64(mine + 24u, t.v456);
+    sts_f64(mine + 32u, t.nvp); sts_f64(mine + 40u, t.nvd); sts_f64(mine + 48u, t.s0); sts_f64(mine + 56u, t.s1);
+    if (tail) { sts_f64(mine + 64u, t.mvs); sts_f64(mine + 72u, t.rej); }
   }
-  __syncthreads();
-  if (tail) { mvs = max_nn(mvs, lds_f64(other + 64u)); rej = max_nn(rej, lds_f64(other + 72u)); }
-  v0 = max_nn(v0, lds_f64(other)); v12 = max_nn(v12, lds_f64(other + 8u)); v3 = max_nn(v3, lds_f64(other + 16u));
-  v456 = max_nn(v456, lds_f64(other + 24u)); nvp = max_nn(nvp, lds_f64(other + 32u)); nvd = max_nn(nvd, lds_f64(other + 40u));
+}
+
+// Second half, both warps, after a barrier that published both warps' slots: the team's norms (this
+// warp's value first, as max_nn is not symmetric in a NaN), decided by qp_termination.  Returns 1 / 2
+// (solved / solved inaccurate), -7, or 0; `want_cert` tells the caller which infeasibility certificates
+// passed their first stage (bit 0 primal, bit 1 dual) and have to be evaluated in full by
+// dense_certificates, which reads the reduced first stage from the per-warp slots of DL::Red.
+template <int NP, int MP>
+__device__ __forceinline__ int dense_test_decide(const uint32_t sb, const bool rowwarp, const bool approximate,
+                                                 const bool tail, double &pri_out, double &dua_out, int &want_cert) {
+  using DL = DenseL<NP, MP>;
+  const uint32_t mine = sb + 8u * (DL::Red + (rowwarp ? 0 : 16)), other = sb + 8u * (DL::Red + (rowwarp ? 16 : 0));
+  double mvs = 0.0, rej = 0.0;
+  if (tail) { mvs = max_nn(lds_f64(mine + 64u), lds_f64(other + 64u)); rej = max_nn(lds_f64(mine + 72u), lds_f64(other + 72u)); }
+  const double v0 = max_nn(lds_f64(mine), lds_f64(other)), v12 = max_nn(lds_f64(mine + 8u), lds_f64(other + 8u));
+  const double v3 = max_nn(lds_f64(mine + 16u), lds_f64(other + 16u)), v456 = max_nn(lds_f64(mine + 24u), lds_f64(other + 24u));
+  const double nvp = max_nn(lds_f64(mine + 32u), lds_f64(other + 32u)), nvd = max_nn(lds_f64(mine + 40u), lds_f64(other + 40u));
   // fixed order (rows + variables) so that both warps take the same decision
   const uint32_t r0a = sb + 8u * DL::Red;
-  s0 = lds_f64(r0a + 48u) + lds_f64(r0a + 128u + 48u);
-  s1 = lds_f64(r0a + 56u) + lds_f64(r0a + 128u + 56u);
+  const double s0 = lds_f64(r0a + 48u) + lds_f64(r0a + 128u + 48u);
+  const double s1 = lds_f64(r0a + 56u) + lds_f64(r0a + 128u + 56u);
   const double eps_pinf = dense_sc<NP, MP>(sb, 2), eps_dinf = dense_sc<NP, MP>(sb, 3);
   const int status = qp_termination(v0, v12, v3, v456, nvp, s0, nvd, s1, dense_sc<NP, MP>(sb, 4), dense_sc<NP, MP>(sb, 5),
                                     dense_sc<NP, MP>(sb, 0), dense_sc<NP, MP>(sb, 1), eps_pinf, eps_dinf, approximate,
@@ -190,6 +221,18 @@ __device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp,
     if (rej > f * eps_dinf * nvd) want_cert &= ~2;
   }
   return status;
+}
+
+// the whole test on state X, both warps (expects Xs / Ys of X published and a barrier passed)
+template <int NP, int MP>
+__device__ __forceinline__ int dense_test(const uint32_t sb, const bool rowwarp, const int lane,
+                                          const double u0, const double u1, const double u2, const double lo,
+                                          const double hi, const DenseState &X, const bool approximate,
+                                          const bool tail, double &pri_out, double &dua_out, int &want_cert) {
+  if (rowwarp) dense_test_publish<NP, MP, true>(sb, lane, dense_test_terms<NP, MP, true>(sb, lane, u0, u1, u2, lo, hi, X, tail), tail);
+  else dense_test_publish<NP, MP, false>(sb, lane, dense_test_terms<NP, MP, false>(sb, lane, u0, u1, u2, lo, hi, X, tail), tail);
+  __syncthreads();
+  return dense_test_decide<NP, MP>(sb, rowwarp, approximate, tail, pri_out, dua_out, want_cert);
 }
 
 // ---- rare paths.  Both work on the iterates spilled to DL::Sp and rebuild the lane constants from
@@ -207,8 +250,7 @@ __device__ __forceinline__ void dense_spill(const uint32_t sb, const bool rowwar
   }
 }
 template <int NP, int MP>
-__device__ __forceinline__ void dense_reload(const uint32_t sb, const bool rowwarp, const int lane, DenseLane &L,
-                                             DenseState &X) {
+__device__ __forceinline__ void dense_unspill(const uint32_t sb, const bool rowwarp, const int lane, DenseState &X) {
   using DL = DenseL<NP, MP>;
   const uint32_t a = sb + 8u * (DL::Sp + lane);
   X.p0 = X.z0 = X.y0 = X.s = X.zs = X.ys = X.pp0 = X.py0 = X.ps = X.pys = 0.0;
@@ -219,6 +261,11 @@ __device__ __forceinline__ void dense_reload(const uint32_t sb, const bool rowwa
     X.p0 = lds_f64(a); X.z0 = lds_f64(a + 8u * 32); X.y0 = lds_f64(a + 8u * 64); X.pp0 = lds_f64(a + 8u * 96);
     X.py0 = lds_f64(a + 8u * 128);
   }
+}
+template <int NP, int MP>
+__device__ __forceinline__ void dense_reload(const uint32_t sb, const bool rowwarp, const int lane, DenseLane &L,
+                                             DenseState &X) {
+  dense_unspill<NP, MP>(sb, rowwarp, lane, X);
   L.u0 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 0)); L.u1 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 1));
   L.u2 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 2)); L.lo = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 3));
   L.hi = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 4)); L.r0 = lds_f64(dense_la<NP, MP>(sb, rowwarp, lane, 5));
@@ -697,8 +744,8 @@ __device__ __noinline__ QPResult dense_qp_solve(const DevStruct &S_, const DevSe
   int next_check = chk ? chk : max_iter + 1;
   __syncthreads();
 
-  // one ADMM iteration: reads (c, wp) at `vcur`, publishes this lane's new entry at `vnext`
-  auto iterate = [&](const uint32_t vcur, const uint32_t vnext) {
+  // one ADMM iteration: the dot product of this lane's row with (c, wp) at `vcur` ...
+  auto lane_dot = [&](const uint32_t vcur) {
     double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
 #pragma unroll
     for (int k = 0; k < NV / 4; k++) {
@@ -713,42 +760,64 @@ __device__ __noinline__ QPResult dense_qp_solve(const DevStruct &S_, const DevSe
       a0 = fma(Mr[NV - 2], va.x, a0);
       a1 = fma(Mr[NV - 1], va.y, a1);
     }
-    const double acc = (a0 + a1) + (a2 + a3);
-    double out;
-    // The updates are those of the generic loop (sco_qp.cuh generic_loop P1..P4) with the exact
-    // identities  y+ = y + rho (v - z+) = rho (t - z+),  rho z+ - y+ = rho (2 z+ - t),  t = v + y / rho,
-    // which shorten the dependent chain behind the dot product from 16 to 10 FP64 operations.
-    if (rowwarp) {
-      // t = acc ; slack and penalty-row updates, then wp for the next iteration
-      const double stil = g - u3 * acc;
-      const double sn = alpha * stil + oma * X.s;
-      const double ts = (alpha * u2) * stil + (oma * X.zs + X.ys * rhoi);
-      const double zns = relu_bits(ts);
-      X.ys = rho * (ts - zns);
-      const double zt = acc + u1 * stil;
-      const double tz = alpha * zt + (oma * X.z0 + X.y0 * rhoi);
-      const double zn = tz < hi ? tz : hi;
-      X.y0 = rho * (tz - zn);
-      X.s = sn;
-      X.zs = zns;
-      X.z0 = zn;
-      const double wpen = rho * (2.0 * zn - tz);
-      const double rr = (sigma * sn - u0) + u2 * (rho * (2.0 * zns - ts)) + lo * wpen;
-      g = Mi * rr;
-      out = kd * wpen - (rho * lo) * g;
-    } else {
-      // x~ = acc ; x and box-row updates, then c for the next iteration
-      const double xn = alpha * acc + oma * X.p0;
-      const double tz = (alpha * u1) * acc + (oma * X.z0 + X.y0 * u3);
-      const double zn = clampd(tz, lo, hi);
-      X.y0 = u2 * (tz - zn);
-      X.p0 = xn;
-      X.z0 = zn;
-      out = (sigma * xn - u0) + (u1 * u2) * (2.0 * zn - tz);
-    }
+    return (a0 + a1) + (a2 + a3);
+  };
+  // ... then the lane-local update, which returns this lane's entry of (c, wp) for the next iteration.
+  // The updates are those of the generic loop (sco_qp.cuh generic_loop P1..P4) with the exact
+  // identities  y+ = y + rho (v - z+) = rho (t - z+),  rho z+ - y+ = rho (2 z+ - t),  t = v + y / rho,
+  // which shorten the dependent chain behind the dot product from 16 to 10 FP64 operations.  A product
+  // feeding a subtraction is written as an explicit fma: left to ptxas, which multiply it fuses depends
+  // on the surrounding code, and the plain and the tested iterations would round differently.
+  auto row_update = [&](const double acc) {
+    // t = acc ; slack and penalty-row updates, then wp for the next iteration
+    const double stil = fma(acc, -u3, g);
+    const double sn = alpha * stil + oma * X.s;
+    const double ts = (alpha * u2) * stil + (oma * X.zs + X.ys * rhoi);
+    const double zns = relu_bits(ts);
+    X.ys = rho * (ts - zns);
+    const double zt = acc + u1 * stil;
+    const double tz = alpha * zt + (oma * X.z0 + X.y0 * rhoi);
+    const double zn = tz < hi ? tz : hi;
+    X.y0 = rho * (tz - zn);
+    X.s = sn;
+    X.zs = zns;
+    X.z0 = zn;
+    const double wpen = rho * (2.0 * zn - tz);
+    const double rr = fma(lo, wpen, fma(u2, rho * (2.0 * zns - ts), fma(sigma, sn, -u0)));
+    g = Mi * rr;
+    return fma(kd, wpen, -((rho * lo) * g));
+  };
+  auto var_update = [&](const double acc) {
+    // x~ = acc ; x and box-row updates, then c for the next iteration
+    const double xn = alpha * acc + oma * X.p0;
+    const double tz = (alpha * u1) * acc + (oma * X.z0 + X.y0 * u3);
+    const double zn = clampd(tz, lo, hi);
+    X.y0 = u2 * (tz - zn);
+    X.p0 = xn;
+    X.z0 = zn;
+    return fma(u1 * u2, 2.0 * zn - tz, fma(sigma, xn, -u0));
+  };
+  // reads (c, wp) at `vcur`, publishes this lane's new entry at `vnext`
+  auto iterate = [&](const uint32_t vcur, const uint32_t vnext) {
+    const double acc = lane_dot(vcur);
+    const double out = rowwarp ? row_update(acc) : var_update(acc);
     sts_f64(vnext + my_out, out);
   };
-
+  // iteration k+1 with the first half of the termination test of iteration k (Xs / Ys published, its
+  // iterates spilled to DL::Sp) in its shadow: neither depends on the other, and with the warp's role and
+  // the tail mode fixed at compile time each warp runs both in one basic block, so the test's loads, dot
+  // products and lane-local terms fill the latency of the iteration's dependent chain.  The barrier after
+  // it publishes the test's partials with (c, wp).
+  auto iterate_and_test = [&](const uint32_t vcur, const uint32_t vnext, auto row, auto tl) {
+    constexpr bool ROW = decltype(row)::value, TAIL = decltype(tl)::value;
+    DenseState Xk;
+    dense_unspill<NP, MP>(sb, ROW, lane, Xk);
+    const double acc = lane_dot(vcur);
+    const DenseTestTerms t = dense_test_terms<NP, MP, ROW>(sb, lane, u0, u1, u2, lo, hi, Xk, TAIL);
+    const double out = ROW ? row_update(acc) : var_update(acc);
+    dense_test_publish<NP, MP, ROW>(sb, lane, t, TAIL);  // after the update: a warp collective is a scheduling fence
+    sts_f64(vnext + my_out, out);
+  };
   int p = 0;
   while (iter < max_iter) {
     // ---- plain iterations up to (not including) the next tested / last one
@@ -765,12 +834,47 @@ __device__ __noinline__ QPResult dense_qp_solve(const DevStruct &S_, const DevSe
     iter = seg_end;
     checked = false;
     if (iter != next_check) { __syncthreads(); break; }
-#ifdef SCO_TIMING
-    const long long tc0 = clock64();
-#endif
     next_check += chk;
     checked = true;
     sts_f64(my_chk, rowwarp ? kd * X.y0 : X.p0);
+    if (chk >= 2 && iter + 1 < max_iter) {
+      // ---- pipelined test of iteration k = iter, decided after iteration k+1.  Iteration k+1 is never
+      // tested itself (chk >= 2) nor the last one, so the max_iter epilogue never sees this path.  State k
+      // goes to DL::Sp: the test reads it from there, and a verdict on k restores it.
+      dense_spill<NP, MP>(sb, rowwarp, lane, X);
+      __syncthreads();
+      const uint32_t vcur = p ? vb1 : vb0, vnext = p ? vb0 : vb1;
+      if (rowwarp) {
+        if (tail) iterate_and_test(vcur, vnext, BoolC<true>(), BoolC<true>());
+        else iterate_and_test(vcur, vnext, BoolC<true>(), BoolC<false>());
+      } else {
+        if (tail) iterate_and_test(vcur, vnext, BoolC<false>(), BoolC<true>());
+        else iterate_and_test(vcur, vnext, BoolC<false>(), BoolC<false>());
+      }
+      p ^= 1;
+      __syncthreads();
+#ifdef SCO_TIMING
+      const long long tc0 = clock64();
+#endif
+      int cert;
+      status = dense_test_decide<NP, MP>(sb, rowwarp, false, tail, res.pri_res, res.dua_res, cert);
+      if (status == 0 && cert) {  // Xs / Ys / Red are free again: the decision has been read
+        const int r = dense_certificates<NP, MP>(sb, n, m, false, (cert & 1) != 0, (cert & 2) != 0);
+        if (r & 1) status = -3;
+        else if (r & 2) status = -4;
+      }
+      if (status != 0) dense_unspill<NP, MP>(sb, rowwarp, lane, X);  // the result is iteration k's
+      else iter++;
+#ifdef SCO_TIMING
+      res.cyc_check += clock64() - tc0;
+#endif
+      if (status != 0) break;
+      continue;
+    }
+    // ---- unpipelined test (check_termination 1, or k+1 = max_iter)
+#ifdef SCO_TIMING
+    const long long tc0 = clock64();
+#endif
     __syncthreads();
     int cert;
     status = dense_test<NP, MP>(sb, rowwarp, lane, u0, u1, u2, lo, hi, X, false, tail, res.pri_res, res.dua_res, cert);
