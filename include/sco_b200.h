@@ -47,6 +47,16 @@ extern "C" {
                               (opcode, operand) pairs; ipar = {n, m, instructions, analytic}; analytic = 0:
                               finite-difference Jacobian, like a black-box Expr without grad (expr.py:61-69);
                               analytic = 1: the program differentiated in forward mode, like Expr(f, grad) (:86-88) */
+/* Column maps (sco_block_desc.cols, the Variable a BoundExpr is bound to, expr.py:413-437).  cols = NULL: the
+ * columns above, every row over all n variables (CIRCLE2D: x[2t], x[2t+1]; FK7: x[n-7:n]).  Otherwise row r
+ * reads x[cols[r*n_in + i]] as its local input i, and the formulas above hold with n replaced by n_in:
+ *   QUADFORM, VM: row r is a function of its n_in local inputs; P_r is packed over n_in, a_r has n_in entries,
+ *                 PUSH_X operands are local indices, ipar[0] = n_in.  Rows of different maps may share a block.
+ *   CIRCLE2D:     n_in = 2; row r reads the point (x[cols[2r]], x[cols[2r+1]]) against circle r % K; T = m / K.
+ *   FK7:          n_in = 7; m is a multiple of 3, rows 3i..3i+2 are instance i (one flange position), have the
+ *                 same map, and every instance uses the block's one DH table.
+ * Indices lie in [0, n) and do not repeat within a row.  A block with a map never takes the dense QP kernels
+ * (sco_dense.cuh), which assume rows over all n variables. */
 
 #define SCO_CNT_LEQ 0 /* LEqExpr -> hinge penalty, one slack per row  (expr.py:353-371) */
 #define SCO_CNT_EQ 1  /* EqExpr  -> abs penalty, two slacks per row   (expr.py:314-332) */
@@ -86,10 +96,11 @@ typedef struct {
   int32_t m;          /* rows */
   int32_t group_mask; /* bit g set <=> member of constraint group g (prob.py:135-142) */
   int32_t jw;         /* Jacobian entries stored per row */
-  int32_t pad_;
+  int32_t n_in;       /* inputs per row when cols != NULL (see the column maps above); ignored otherwise */
   int32_t ipar[8];
   sco_field par; /* family parameters */
   sco_field val; /* CompExpr.val, m doubles */
+  const int32_t *cols; /* host, m * n_in column indices, row-major, or NULL (implied columns) */
 } sco_block_desc;
 
 typedef struct {

@@ -21,7 +21,8 @@ class CField(ctypes.Structure):
 
 class CBlock(ctypes.Structure):
     _fields_ = [("family", c_i32), ("cnt_type", c_i32), ("m", c_i32), ("group_mask", c_i32),
-                ("jw", c_i32), ("pad_", c_i32), ("ipar", c_i32 * 8), ("par", CField), ("val", CField)]
+                ("jw", c_i32), ("n_in", c_i32), ("ipar", c_i32 * 8), ("par", CField), ("val", CField),
+                ("cols", c_vp)]
 
 
 class CStructure(ctypes.Structure):

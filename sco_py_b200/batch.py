@@ -29,7 +29,7 @@ class Compiled(object):
         self.lb0 = self.ub0 = None  # user bounds of the scalar variables
         self.c = 0.0
         self.lin_A = self.lin_l = self.lin_u = None
-        self.blocks = []         # (family expr, cnt_type, val[m], group ids)
+        self.blocks = []         # device blocks: (family expr, cnt_type, val[m], group ids, column map [m, n_in] or None)
         self.obj_prog = None     # SymExpr of a non-quadratic objective
         self.gids = []
 
@@ -42,6 +42,56 @@ def _columns(var, col_of):
                                      "Prob.add_osqp_var" % (ov.var_name,))
         cols.append(col_of[id(ov)])
     return np.asarray(cols, dtype=np.int64)
+
+
+class PackedRows(object):
+    """Bound QUADFORM or VM constraints of one kind (family, Eq / LEq, groups, inputs per row; for VM also the
+    derivative mode) packed into one device block, rows in add order: per-row P and a concatenated (QUADFORM), or
+    programs concatenated with re-offset row tables (VM).  Has the attributes of a family expression that
+    compile_batch reads."""
+
+    shared_params = False
+
+    def __init__(self, parts):
+        f0 = parts[0]
+        self.parts = parts
+        self.family = f0.family
+        self.n = self.jw = f0.n
+        self.m = sum(p.m for p in parts)
+        if self.family == E.FAM_VM:
+            self.n_instr = sum(p.n_instr for p in parts)
+            self.ipar = [self.n, self.m, self.n_instr, int(f0.analytic), 0, 0, 0, 0]
+        else:
+            self.ipar = [self.n, self.m, 0, 0, 0, 0, 0, 0]
+
+    def params(self):
+        if self.family == E.FAM_QUADFORM:
+            ntri = self.n * (self.n + 1) // 2
+            ps = [p.params() for p in self.parts]
+            return np.concatenate([q[:p.m * ntri] for p, q in zip(self.parts, ps)] +
+                                  [q[p.m * ntri:] for p, q in zip(self.parts, ps)])
+        offsets, code, base = [], [], 0
+        for p in self.parts:
+            offsets.append(p.program[:p.m] + base)
+            code.append(p.program[p.m:])
+            base += p.n_instr
+        return np.concatenate(offsets + code)
+
+
+def _row_map(fam, cols, n):
+    """Column map [m, n_in] of a family constraint bound to the Variable whose columns (in the Variable's own
+    order, the order expr.py evaluates it in) are `cols`."""
+    name = type(fam).__name__
+    if isinstance(fam, E.CircleDistExpr):
+        if 2 * fam.T > cols.size:
+            raise UnsupportedProblem("CircleDistExpr: %d way-points need %d variables, its Variable has %d"
+                                     % (fam.T, 2 * fam.T, cols.size))
+        return np.repeat(cols[:2 * fam.T].reshape(fam.T, 2), fam.K, axis=0)
+    if fam.n != cols.size:
+        raise UnsupportedProblem("a %s over %d variables is bound to a Variable of %d" % (name, fam.n, cols.size))
+    if isinstance(fam, E.FK7Expr):
+        return np.tile(cols[-7:], (3, 1))
+    return np.tile(cols, (fam.m, 1))
 
 
 def compile_problem(prob):
@@ -119,6 +169,7 @@ def compile_problem(prob):
         cp.lin_u = np.concatenate(rows_u)
     # ---- nonlinear constraints -> family blocks
     cp.gids = sorted(prob._cnt_groups.keys())
+    packs = {}  # bound QUADFORM / VM constraints of one kind -> index of their device block
     for b in prob._nonlin_cnt_exprs:
         comp = b.expr
         fam = comp.expr
@@ -127,22 +178,43 @@ def compile_problem(prob):
                 "constraint on a black-box Expr: the device engine evaluates closed families only "
                 "(QuadFormExpr, CircleDistExpr, FK7Expr in sco_py_b200.expr); there is no CPU fallback")
         cols = _columns(b.var, col_of)
-        if cols.size != n or not np.array_equal(cols, np.arange(n)):
-            raise UnsupportedProblem("family constraints must be bound to a Variable that holds ALL scalar "
-                                     "variables of the problem in QP order")
-        if getattr(fam, "n", n) != n:
-            raise UnsupportedProblem("a %s over %d variables is bound to a problem of %d variables"
-                                     % (type(fam).__name__, fam.n, n))
-        if isinstance(fam, E.CircleDistExpr) and 2 * fam.T > n:
-            raise UnsupportedProblem("CircleDistExpr: %d way-points need %d variables, the problem has %d" % (fam.T, 2 * fam.T, n))
+        uniq, counts = np.unique(cols, return_counts=True)
+        if (counts > 1).any():
+            raise UnsupportedProblem("a constraint's Variable lists scalar variable %r more than once"
+                                     % (cp.ovars[int(uniq[counts > 1][0])].var_name,))
         ctype = CNT_EQ if isinstance(comp, E.EqExpr) else CNT_LEQ
         val = np.asarray(comp.val, dtype=float).ravel()
         if val.size != fam.m:
             raise UnsupportedProblem("comparison value has %d entries, the expression %d rows" % (val.size, fam.m))
         gids = [g for g in cp.gids if b in prob._cnt_groups[g]]
-        cp.blocks.append((fam, ctype, val, gids))
+        if cols.size == n and np.array_equal(cols, np.arange(n)):
+            # bound to every variable in QP order: the implied columns, no map (the structure of earlier versions)
+            if getattr(fam, "n", n) != n:
+                raise UnsupportedProblem("a %s over %d variables is bound to a problem of %d variables"
+                                         % (type(fam).__name__, fam.n, n))
+            if isinstance(fam, E.CircleDistExpr) and 2 * fam.T > n:
+                raise UnsupportedProblem("CircleDistExpr: %d way-points need %d variables, the problem has %d" % (fam.T, 2 * fam.T, n))
+            cp.blocks.append((fam, ctype, val, gids, None))
+            continue
+        rows = _row_map(fam, cols, n)
+        if fam.family not in (E.FAM_QUADFORM, E.FAM_VM):
+            cp.blocks.append((fam, ctype, val, gids, rows))
+            continue
+        key = (fam.family, ctype, tuple(gids), fam.n, getattr(fam, "analytic", None))
+        if key not in packs:
+            packs[key] = len(cp.blocks)
+            cp.blocks.append(([], ctype, [], gids, []))
+        parts, _, vals, _, maps = cp.blocks[packs[key]]
+        parts.append(fam)
+        vals.append(val)
+        maps.append(rows)
+    for k in packs.values():
+        parts, ctype, vals, gids, maps = cp.blocks[k]
+        cp.blocks[k] = (PackedRows(parts), ctype, np.concatenate(vals), gids, np.vstack(maps))
     if len(cp.blocks) > MAX_BLOCKS or len(cp.gids) > MAX_GROUPS:
-        raise UnsupportedProblem("more than %d constraint blocks / %d groups" % (MAX_BLOCKS, MAX_GROUPS))
+        raise UnsupportedProblem("%d device constraint blocks (bound QUADFORM / VM constraints of one family, Eq / "
+                                 "LEq kind, group set and input count share one) and %d groups: the limits are %d "
+                                 "and %d" % (len(cp.blocks), len(cp.gids), MAX_BLOCKS, MAX_GROUPS))
     return cp
 
 
@@ -160,7 +232,8 @@ def group_key(cp):
     """What two compiled problems must have in common to go into one launch."""
     return (cp.x0.size, cp.qa is not None, cp.lb0 is not None,
             None if cp.lin_A is None else (cp.lin_A.shape, cp.lin_A.tobytes()), tuple(cp.gids),
-            tuple((b[0].family, b[0].m, b[1], tuple(b[0].ipar), tuple(b[3])) for b in cp.blocks),
+            tuple((b[0].family, b[0].m, b[1], tuple(b[0].ipar), tuple(b[3])) +
+                  (() if b[4] is None else (b[4].shape, b[4].tobytes())) for b in cp.blocks),
             None if cp.obj_prog is None else (cp.obj_prog.n_instr, cp.obj_prog.analytic))
 
 
@@ -176,7 +249,8 @@ def compile_batch(probs, compiled=None):
                 (c.lin_A is None) == (c0.lin_A is None) and
                 (c.lin_A is None or (c.lin_A.shape == c0.lin_A.shape and np.array_equal(c.lin_A, c0.lin_A))) and
                 all(a[0].family == b[0].family and a[0].m == b[0].m and a[1] == b[1] and a[3] == b[3] and
-                    list(a[0].ipar) == list(b[0].ipar) for a, b in zip(c.blocks, c0.blocks)) and
+                    list(a[0].ipar) == list(b[0].ipar) and (a[4] is None) == (b[4] is None) and
+                    (a[4] is None or np.array_equal(a[4], b[4])) for a, b in zip(c.blocks, c0.blocks)) and
                 (c.obj_prog is None) == (c0.obj_prog is None) and (c.qa is None) == (c0.qa is None) and
                 (c.lb0 is None) == (c0.lb0 is None) and
                 (c.obj_prog is None or (c.obj_prog.n_instr == c0.obj_prog.n_instr and c.obj_prog.analytic == c0.obj_prog.analytic)))
@@ -238,7 +312,7 @@ def compile_batch(probs, compiled=None):
             fills.append((of, lambda c: c.obj_prog.params()))
         kw.update(obj_prog=of, obj_prog_len=c0.obj_prog.n_instr, obj_prog_flags=int(c0.obj_prog.analytic))
     blocks = []
-    for bi, (fam, ctype, val, gids) in enumerate(c0.blocks):
+    for bi, (fam, ctype, val, gids, cols) in enumerate(c0.blocks):
         p0 = fam.params()
         if fam.shared_params or (B > 1 and all(np.array_equal(c.blocks[bi][0].params(), p0) for c in cps[1:])):
             pf = shared_field(p0)
@@ -252,7 +326,8 @@ def compile_batch(probs, compiled=None):
             mask |= 1 << c0.gids.index(g)
         # group_ids=[] puts a constraint in NO group (prob.py:135-142): mask 0, and a problem without any group
         # has n_groups = 0 -- the reference then skips the per-group test (solver.py:209)
-        blocks.append(Block(fam.family, ctype, fam.m, pf, vf, ipar=list(fam.ipar), group_mask=mask, jw=fam.jw))
+        blocks.append(Block(fam.family, ctype, fam.m, pf, vf, ipar=list(fam.ipar), group_mask=mask, jw=fam.jw,
+                            cols=None if cols is None else np.ascontiguousarray(cols, dtype=np.int32)))
     ng = len(c0.gids)
     overlap = np.zeros((ng, ng), dtype=np.int32)
     ov = getattr(probs[0], "_cnt_groups_overlap", {}) if probs else {}
@@ -284,7 +359,8 @@ def signature(st):
             st.obj_prog_len, st.obj_prog_flags, st.m_lin, lin, st.n_groups,
             None if st.group_overlap is None else st.group_overlap.tobytes(),
             None if st.shared is None else st.shared.tobytes(),
-            tuple((b.family, b.cnt_type, b.m, fld(b.par), fld(b.val), tuple(b.ipar), b.group_mask, b.jw)
+            tuple((b.family, b.cnt_type, b.m, fld(b.par), fld(b.val), tuple(b.ipar), b.group_mask, b.jw) +
+                  (() if b.cols is None else (b.cols.shape, np.ascontiguousarray(b.cols, dtype=np.int32).tobytes()))
                   for b in st.blocks))
 
 

@@ -5,7 +5,8 @@ results somebody obtained for it, so that benchmarks are reproducible and regres
 
     format            "sco_b200.batch"          version  1
     structure         JSON (n, stride, every Field as [off, shared], blocks, groups)  + the structure's arrays
-                      (lin_rowptr / lin_col / lin_val, shared, group_overlap)
+                      (lin_rowptr / lin_col / lin_val, shared, group_overlap; st_cols<i>: column map of block i,
+                      only for blocks that have one)
     params [B, stride] float64      x0 [B, n] float64
     settings          JSON of the solver / OSQP settings the results belong to (optional)
     expected_*        verdict [B] int32, x [B, n], max_vio [B], objective [B], nonconverged [B] (optional)
@@ -44,10 +45,17 @@ def structure_to_json(st):
     return d
 
 
+def _maps(st):
+    """{array name: column map} of the blocks that have one."""
+    return {"cols%d" % i: np.ascontiguousarray(b.cols, dtype=np.int32) for i, b in enumerate(st.blocks)
+            if b.cols is not None}
+
+
 def structure_from_json(d, arrays):
     kw = {name: Field(int(d[name][0]), bool(d[name][1])) for name in _FIELDS if name in d}
     blocks = [Block(b["family"], b["cnt_type"], b["m"], Field(*b["par"]), Field(*b["val"]), ipar=list(b["ipar"]),
-                    group_mask=b["group_mask"], jw=b["jw"]) for b in d["blocks"]]
+                    group_mask=b["group_mask"], jw=b["jw"], cols=arrays.get("cols%d" % i))
+              for i, b in enumerate(d["blocks"])]
     for name in _ARRAYS:
         if name in arrays:
             kw[name] = arrays[name]
@@ -62,6 +70,10 @@ def structure_signature(st):
         if a is not None:
             h.update(name.encode())
             h.update(np.ascontiguousarray(a).tobytes())
+    for name, a in _maps(st).items():  # nothing for a structure without maps: its signature is unchanged
+        h.update(name.encode())
+        h.update(np.asarray(a.shape, dtype=np.int64).tobytes())
+        h.update(a.tobytes())
     return h.hexdigest()
 
 
@@ -76,6 +88,8 @@ def save_batch(path, st, params, x0, settings=None, expected=None):
         a = getattr(st, name)
         if a is not None:
             out["st_" + name] = np.asarray(a)
+    for name, a in _maps(st).items():
+        out["st_" + name] = a
     if settings is not None:
         out["settings"] = np.array(json.dumps(settings))
     for k, v in (expected or {}).items():
@@ -87,7 +101,7 @@ def load_batch(path):
     with np.load(path, allow_pickle=False) as z:
         if str(z["format"]) != FORMAT or int(z["version"]) > VERSION:
             raise ValueError("%s is not a %s file of version <= %d" % (path, FORMAT, VERSION))
-        arrays = {name: z["st_" + name] for name in _ARRAYS if "st_" + name in z.files}
+        arrays = {k[3:]: z[k] for k in z.files if k.startswith("st_")}
         st = structure_from_json(json.loads(str(z["structure"])), arrays)
         if structure_signature(st) != str(z["signature"]):
             raise ValueError("%s: structure signature mismatch (file damaged or written by another version)" % path)

@@ -213,8 +213,26 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
       if (b.m <= 0) return fail(SCO_ERR_ARG, "block %d: m must be positive", bi);
       if (desc->n_groups < 32 && (b.group_mask >> desc->n_groups) != 0)
         return fail(SCO_ERR_ARG, "block %d: group_mask names a group >= n_groups", bi);
+      if (b.cols) {
+        const int want = b.family == SCO_FAM_CIRCLE2D ? 2 : b.family == SCO_FAM_FK7 ? 7 : b.n_in;
+        if (b.n_in <= 0 || b.n_in > n_ || b.n_in != want)
+          return fail(SCO_ERR_ARG, "block %d: n_in = %d is wrong for family %d (CIRCLE2D 2, FK7 7, else 1..n)", bi, b.n_in,
+                      b.family);
+        if (b.family == SCO_FAM_FK7 && b.m % 3 != 0) return fail(SCO_ERR_ARG, "block %d: FK7 with a map needs m %% 3 == 0", bi);
+        for (int r = 0; r < b.m; r++) {
+          const int32_t *c = b.cols + (size_t)r * b.n_in;
+          for (int i = 0; i < b.n_in; i++) {
+            if (c[i] < 0 || c[i] >= n_) return fail(SCO_ERR_ARG, "block %d row %d: column %d outside [0, %d)", bi, r, c[i], (int)n_);
+            for (int k = 0; k < i; k++)
+              if (c[k] == c[i]) return fail(SCO_ERR_ARG, "block %d row %d: column %d repeats", bi, r, c[i]);
+            if (b.family == SCO_FAM_FK7 && r % 3 != 0 && c[i] != c[i - (r % 3) * 7])
+              return fail(SCO_ERR_ARG, "block %d: rows of FK7 instance %d have different maps", bi, r / 3);
+          }
+        }
+      }
+      const long long nb = b.cols ? b.n_in : n_;  // inputs of a row
       long long plen = 0;
-      if (b.family == SCO_FAM_QUADFORM) plen = (long long)b.m * (n_ * (n_ + 1) / 2 + n_);
+      if (b.family == SCO_FAM_QUADFORM) plen = (long long)b.m * (nb * (nb + 1) / 2 + nb);
       else if (b.family == SCO_FAM_CIRCLE2D) plen = 3LL * b.ipar[1];
       else if (b.family == SCO_FAM_FK7) plen = 30;
       else if (b.family == SCO_FAM_VM) plen = b.m + 2LL * b.ipar[2];
@@ -257,6 +275,7 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
   std::vector<int> row_goff, row_soff, row_w, row_eq, row_gmask, jcol;
   int m_nl = 0, jnnz = 0, sj = 0, n_slack = 0, any_eq = 0, max_stage = 0;
   int max_jw = 1;
+  bool any_map = false;
   for (int bi = 0; bi < desc->n_blocks; bi++) {
     const sco_block_desc &b = desc->blocks[bi];
     DevBlock &d = S.blocks[bi];
@@ -264,18 +283,26 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
     d.row0 = m_nl; d.joff = jnnz;
     memcpy(d.ipar, b.ipar, sizeof(d.ipar));
     d.par = cvt(b.par); d.val = cvt(b.val);
+    const bool mapped = b.cols != nullptr;
+    const int nb = mapped ? b.n_in : n;  // inputs of a row
+    any_map = any_map || mapped;
+    d.n_in = mapped ? b.n_in : 0;
     int jw = 0;
-    if (b.family == SCO_FAM_QUADFORM) { jw = n; max_stage = std::max(max_stage, n * (n + 1) / 2); }
-    else if (b.family == SCO_FAM_CIRCLE2D) {
+    if (b.family == SCO_FAM_QUADFORM) {
+      jw = nb;
+      // a map's inputs are gathered into the staging buffer behind P_r
+      max_stage = std::max(max_stage, nb * (nb + 1) / 2 + (mapped ? nb : 0));
+    } else if (b.family == SCO_FAM_CIRCLE2D) {
       jw = 2;
-      if (b.ipar[0] * b.ipar[1] != b.m || 2 * b.ipar[0] > n) { delete h; return fail(SCO_ERR_ARG, "CIRCLE2D: m != T*K or 2T > n"); }
+      if (b.ipar[1] <= 0 || b.ipar[0] * b.ipar[1] != b.m || (!mapped && 2 * b.ipar[0] > n)) { sco_destroy(h); return fail(SCO_ERR_ARG, "CIRCLE2D: m != T*K or 2T > n"); }
     } else if (b.family == SCO_FAM_FK7) {
       jw = 7;
-      if (b.m != 3 || n < 7) { delete h; return fail(SCO_ERR_ARG, "FK7: m must be 3 and n >= 7"); }
+      if (mapped) max_stage = std::max(max_stage, 106);  // 98 doubles of finite differences + the gathered joints
+      if ((!mapped && b.m != 3) || n < 7) { sco_destroy(h); return fail(SCO_ERR_ARG, "FK7: m must be 3 (without a map) and n >= 7"); }
     } else if (b.family == SCO_FAM_VM) {
-      jw = n;
-      if (b.ipar[0] != n || b.ipar[1] != b.m || b.ipar[2] <= 0) { delete h; return fail(SCO_ERR_ARG, "VM: ipar must be {n, m, instructions}"); }
-    } else { delete h; return fail(SCO_ERR_UNSUPPORTED, "unknown constraint family %d", b.family); }
+      jw = nb;
+      if (b.ipar[0] != nb || b.ipar[1] != b.m || b.ipar[2] <= 0) { sco_destroy(h); return fail(SCO_ERR_ARG, "VM: ipar must be {n (n_in with a map), m, instructions}"); }
+    } else { sco_destroy(h); return fail(SCO_ERR_UNSUPPORTED, "unknown constraint family %d", b.family); }
     max_jw = std::max(max_jw, jw);
     d.jw = jw;
     const int ldj = (jw % 2 == 0) ? jw + 1 : jw;
@@ -287,7 +314,8 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
       row_gmask.push_back(b.group_mask);
       for (int k = 0; k < jw; k++) {
         int col = 0;
-        if (b.family == SCO_FAM_QUADFORM || b.family == SCO_FAM_VM) col = k;
+        if (mapped) col = b.cols[(size_t)r * b.n_in + k];
+        else if (b.family == SCO_FAM_QUADFORM || b.family == SCO_FAM_VM) col = k;
         else if (b.family == SCO_FAM_CIRCLE2D) col = 2 * (r / b.ipar[1]) + k;
         else col = n - 7 + k;
         jcol.push_back(col);
@@ -318,7 +346,7 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
   std::vector<int> lrp(desc->m_lin + 1, 0), lcol, lcptr(n + 1, 0), lcentry, lcrow;
   std::vector<double> lval;
   if (desc->m_lin > 0) {
-    if (!desc->lin_rowptr || !desc->lin_col || !desc->lin_val) { delete h; return fail(SCO_ERR_ARG, "m_lin > 0 but CSR arrays are null"); }
+    if (!desc->lin_rowptr || !desc->lin_col || !desc->lin_val) { sco_destroy(h); return fail(SCO_ERR_ARG, "m_lin > 0 but CSR arrays are null"); }
     lrp.assign(desc->lin_rowptr, desc->lin_rowptr + desc->m_lin + 1);
     const int nnz = lrp[desc->m_lin];
     lcol.assign(desc->lin_col, desc->lin_col + nnz);
@@ -326,7 +354,7 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
     std::vector<std::vector<std::pair<int, int>>> cols(n);
     for (int r = 0; r < desc->m_lin; r++)
       for (int p = lrp[r]; p < lrp[r + 1]; p++) {
-        if (lcol[p] < 0 || lcol[p] >= n) { delete h; return fail(SCO_ERR_ARG, "linear row column out of range"); }
+        if (lcol[p] < 0 || lcol[p] >= n) { sco_destroy(h); return fail(SCO_ERR_ARG, "linear row column out of range"); }
         cols[lcol[p]].push_back({p, r});
       }
     for (int j = 0; j < n; j++) {
@@ -388,13 +416,14 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
     S.p_narrow = narrow ? 1 : 0;
     bool dense = desc->m_lin == 0 && n <= 32 && m_nl > 0 && m_nl <= 48;
     for (int i = 0; i < m_nl; i++) dense = dense && row_w[i] == n;
+    dense = dense && !any_map;  // its kernels assume rows over all n variables in column order
     S.fast_dense = dense && !ok ? 1 : 0;
   }
   if (rc) { sco_destroy(h); return SCO_ERR_CUDA; }
-  // ---- dense fast path: one dense hinge block, no linear rows, sizes within the instantiated table
+  // ---- dense fast path: one dense hinge block over all variables, no linear rows, sizes within the instantiated table
   S.dense_kind = 0;
   if (desc->m_lin == 0 && S.obj_len == 0 && desc->n_blocks == 1 && desc->blocks[0].family == SCO_FAM_QUADFORM &&
-      desc->blocks[0].cnt_type == SCO_CNT_LEQ) {
+      desc->blocks[0].cnt_type == SCO_CNT_LEQ && !any_map) {
     static const int table[][2] = {{8, 6}, {12, 16}, {20, 30}, {32, 32}};  // keep in sync with QPSolver::solve in sco_qp.cuh
     for (int k = 0; k < 4; k++)
       if (n <= table[k][0] && m_nl <= table[k][1]) { S.dense_kind = k + 1; break; }

@@ -32,7 +32,8 @@ struct DevBlock {
   int jw;    // stored Jacobian entries per row
   int row0;  // first penalty row of the block
   int joff;  // offset of the block inside the per-problem J array (global layout, unpadded)
-  int pad_;
+  int n_in;  // != 0: the block has a column map (include/sco_b200.h) with n_in inputs per row; row r reads
+             // x[jcol_g[joff + r * n_in + i]] as its input i (the map is the block's stored-entry columns)
   int ipar[8];
   DevField par, val;
 };
@@ -96,7 +97,8 @@ struct DevStruct {
   int dense_kind;      // != 0: two-warp dense solve (sco_dense.cuh), index into its size table
   int fast_ok;         // rows of A with <= 8 entries, columns with <= 4 + 4: the thread-per-entity loop applies
   int p_narrow;        // every column of the objective matrix's pattern has <= 4 entries (in-loop termination test)
-  int fast_dense;      // dense penalty rows over n <= 32 variables, m_nl <= 48, no linear rows: its dense variant applies
+  int fast_dense;      // dense penalty rows over n <= 32 variables (no column map), m_nl <= 48, no linear rows: its
+                       // dense variant applies
   int s_bw;            // structural half-bandwidth of S = P + A'RA (max |i - j| over its pattern): the Gauss-Jordan
                        // sweep of pivot k only touches the leading (k + s_bw + 1)^2 block
   int stage_per_warp;  // doubles

@@ -21,16 +21,21 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // ---- QUADFORM: f_j = 0.5 x'P_j x + a_j'x, P_j packed upper row-major, one warp per row ----
+// With a column map x is the row's n_in inputs, gathered into the staging buffer behind P_j.
 template <int TEAM>
 __device__ void eval_quadform(const DevStruct &S, const DevBlock &B, const double *par,
-                              Sh x, Sh f, double *Jout, Sh stage) {
-  const int n = S.n, ntri = n * (n + 1) / 2, m = B.m;
+                              Sh xg, Sh f, double *Jout, Sh stage) {
+  const int *cm = B.n_in ? S.jcol_g + B.joff : nullptr;  // column map
+  const int n = cm ? B.n_in : S.n, ntri = n * (n + 1) / 2, m = B.m;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const Sh buf = stage + warp * S.stage_per_warp;
+  const Sh x = cm ? buf + ntri : xg;
   const double *A = par + (size_t)m * ntri;
   for (int j = warp; j < m; j += TEAM / 32) {
     const double *Pj = par + (size_t)j * ntri;
     for (int e = lane; e < ntri; e += 32) buf[e] = __ldg(Pj + e);
+    if (cm)
+      for (int i = lane; i < n; i += 32) x[i] = xg[__ldg(cm + j * n + i)];
     __syncwarp();
     double fj = 0.0;
     for (int r = lane; r < n; r += 32) {
@@ -49,13 +54,16 @@ __device__ void eval_quadform(const DevStruct &S, const DevBlock &B, const doubl
 }
 
 // ---- CIRCLE2D: row t*K+k: R_k - |p_t - c_k| ----
+// With a column map row r reads the point (x[cols[2r]], x[cols[2r+1]]).
 template <int TEAM>
 __device__ void eval_circle2d(const DevStruct &S, const DevBlock &B, const double *par,
                               Sh x, Sh f, double *Jout) {
   const int K = B.ipar[1], m = B.m;
+  const int *cm = B.n_in ? S.jcol_g + B.joff : nullptr;  // column map
   for (int r = threadIdx.x; r < m; r += TEAM) {
     const int t = r / K, k = r % K;
-    const double dx = x[2 * t] - par[2 * k], dy = x[2 * t + 1] - par[2 * k + 1];
+    const int i0 = cm ? __ldg(cm + 2 * r) : 2 * t, i1 = cm ? __ldg(cm + 2 * r + 1) : 2 * t + 1;
+    const double dx = x[i0] - par[2 * k], dy = x[i1] - par[2 * k + 1];
     const double dist = sqrt(dx * dx + dy * dy);
     f[r] = par[2 * K + k] - dist;
     if (Jout) {
@@ -97,38 +105,50 @@ __device__ __forceinline__ void fk7_pos(const double *q, const double *tab, doub
 
 // Central differences at steps h and 2h, Richardson-combined -- the scheme of
 // oracle/shims/numdifftools (restating numdifftools.Jacobian as called at expr.py:67).
+// Without a column map one instance on x[n-7:n]; with one, instance i (rows 3i..3i+2) on x[cols[21i + k]], its joints
+// gathered into stage[98..104] (sco_create gives a structure with a mapped FK7 block a stage of >= 106 doubles).
 template <int TEAM>
 __device__ void eval_fk7(const DevStruct &S, const DevBlock &B, const double *tab, Sh x, Sh f,
                          double *Jout, Sh stage) {
   const int n = S.n, t = threadIdx.x;
-  const Sh q = x + (n - 7);
-  if (t == 0) {
-    double o[3], q0[7];
-    for (int k = 0; k < 7; k++) q0[k] = q[k];
-    fk7_pos(q0, tab, o);
-    f[0] = o[0]; f[1] = o[1]; f[2] = o[2];
-  }
-  if (Jout) {
-    // thread e = col*4 + (mult_idx*2 + sign): 28 evaluations -> stage[e*3 .. e*3+2]; stage[84+..] = hh
-    for (int e = t; e < 28; e += TEAM) {
-      const int col = e >> 2, mi = (e >> 1) & 1, sg = e & 1;
-      double qq[7];
-      for (int k = 0; k < 7; k++) qq[k] = q[k];
-      const double h0 = tab[29] * fmax(log1p(fabs(q[col])), 1.0);
-      const double h = h0 * (mi ? 2.0 : 1.0);
-      const double xp = q[col] + h, xm = q[col] - h;
-      qq[col] = sg ? xm : xp;
-      double o[3];
-      fk7_pos(qq, tab, o);
-      stage[e * 3] = o[0]; stage[e * 3 + 1] = o[1]; stage[e * 3 + 2] = o[2];
-      if (sg == 0) stage[84 + col * 2 + mi] = xp - xm;
+  const int ninst = B.n_in ? B.m / 3 : 1;
+  for (int inst = 0; inst < ninst; inst++) {
+    const int *cm = B.n_in ? S.jcol_g + B.joff + inst * 21 : nullptr;  // column map of the instance's first row
+    const Sh q = cm ? stage + 98 : x + (n - 7);                           // its joints
+    if (cm) {
+      Team<TEAM>::sync();  // the stage may still be read (previous instance or block)
+      for (int k = t; k < 7; k += TEAM) q[k] = x[__ldg(cm + k)];
+      Team<TEAM>::sync();
     }
-    Team<TEAM>::sync();
-    for (int e = t; e < 21; e += TEAM) {
-      const int r = e / 7, col = e % 7;
-      const double d1 = (stage[(col * 4 + 0) * 3 + r] - stage[(col * 4 + 1) * 3 + r]) / stage[84 + col * 2];
-      const double d2 = (stage[(col * 4 + 2) * 3 + r] - stage[(col * 4 + 3) * 3 + r]) / stage[84 + col * 2 + 1];
-      Jout[r * 7 + col] = (4.0 * d1 - d2) / 3.0;
+    if (t == 0) {
+      double o[3], q0[7];
+      for (int k = 0; k < 7; k++) q0[k] = q[k];
+      fk7_pos(q0, tab, o);
+      f[3 * inst] = o[0]; f[3 * inst + 1] = o[1]; f[3 * inst + 2] = o[2];
+    }
+    if (Jout) {
+      // thread e = col*4 + (mult_idx*2 + sign): 28 evaluations -> stage[e*3 .. e*3+2]; stage[84+..] = hh
+      for (int e = t; e < 28; e += TEAM) {
+        const int col = e >> 2, mi = (e >> 1) & 1, sg = e & 1;
+        double qq[7];
+        for (int k = 0; k < 7; k++) qq[k] = q[k];
+        const double h0 = tab[29] * fmax(log1p(fabs(q[col])), 1.0);
+        const double h = h0 * (mi ? 2.0 : 1.0);
+        const double xp = q[col] + h, xm = q[col] - h;
+        qq[col] = sg ? xm : xp;
+        double o[3];
+        fk7_pos(qq, tab, o);
+        stage[e * 3] = o[0]; stage[e * 3 + 1] = o[1]; stage[e * 3 + 2] = o[2];
+        if (sg == 0) stage[84 + col * 2 + mi] = xp - xm;
+      }
+      Team<TEAM>::sync();
+      double *J = Jout + inst * 21;
+      for (int e = t; e < 21; e += TEAM) {
+        const int r = e / 7, col = e % 7;
+        const double d1 = (stage[(col * 4 + 0) * 3 + r] - stage[(col * 4 + 1) * 3 + r]) / stage[84 + col * 2];
+        const double d2 = (stage[(col * 4 + 2) * 3 + r] - stage[(col * 4 + 3) * 3 + r]) / stage[84 + col * 2 + 1];
+        J[r * 7 + col] = (4.0 * d1 - d2) / 3.0;
+      }
     }
   }
 }
@@ -138,13 +158,15 @@ __device__ void eval_fk7(const DevStruct &S, const DevBlock &B, const double *ta
 // (opcode, operand) pairs of doubles; opcodes END 0, PUSH_X 1, PUSH_C 2, ADD 3, SUB 4, MUL 5, DIV 6,
 // NEG 7, POWI 8, SQRT 9, LOG 10, EXP 11, SIN 12, COS 13, ABS 14, MIN 15, MAX 16, TEE 17 (copy the top of the stack
 // into temporary k), LOAD 18 (push temporary k).  Up to two variables may be replaced by
-// given values (the perturbed points of the finite differences) without copying x.
+// given values (the perturbed points of the finite differences) without copying x.  `cols` is the row's column map
+// (PUSH_X k reads x[cols[k]]) or null (PUSH_X k reads x[k]); pi / pj / wrt name local inputs.
 #define SCO_VM_STACK 16
 #define SCO_VM_SLOTS 128  // a seven-link kinematic chain keeps ~100 rotation entries alive
 #define SCO_FD_JAC_STEP 5.477420592293901e-07    // eps^(1/2.5): numdifftools base step, first derivatives
 #define SCO_FD_HESS_STEP 9.843133202303692e-03  // eps^(1/7.8): second derivatives (oracle/shims/numdifftools)
 
-static __device__ __noinline__ double vm_eval(const double *prog, int m, int row, Sh x, int pi, double vi, int pj, double vj) {
+static __device__ __noinline__ double vm_eval(const double *prog, int m, int row, Sh x, const int *cols, int pi, double vi,
+                                              int pj, double vj) {
   const double *ins = prog + m;
   int pc = (int)prog[row];
   double stk[SCO_VM_STACK], slot[SCO_VM_SLOTS];
@@ -156,7 +178,7 @@ static __device__ __noinline__ double vm_eval(const double *prog, int m, int row
     if (op == 0) break;
     if (op == 1) {
       const int i = (int)arg;
-      stk[sp++] = i == pi ? vi : (i == pj ? vj : x[i]);
+      stk[sp++] = i == pi ? vi : (i == pj ? vj : x[cols ? __ldg(cols + i) : i]);
     } else if (op == 2) {
       stk[sp++] = arg;
     } else if (op <= 6) {
@@ -188,7 +210,8 @@ static __device__ __noinline__ double vm_eval(const double *prog, int m, int row
 
 // The same program in forward mode: value and d/dx_wrt, the exact counterpart of a user-supplied gradient
 // (Expr(f, grad), expr.py:86-88); SymExpr(..., analytic=True).  Rules as in sym.eval_program_dual.
-static __device__ __noinline__ double vm_eval_dual(const double *prog, int m, int row, Sh x, int wrt, double *dout) {
+static __device__ __noinline__ double vm_eval_dual(const double *prog, int m, int row, Sh x, const int *cols, int wrt,
+                                                   double *dout) {
   const double *ins = prog + m;
   int pc = (int)prog[row];
   double stk[SCO_VM_STACK], dsk[SCO_VM_STACK], slot[SCO_VM_SLOTS], dslot[SCO_VM_SLOTS];
@@ -200,7 +223,7 @@ static __device__ __noinline__ double vm_eval_dual(const double *prog, int m, in
     if (op == 0) break;
     if (op == 1) {
       const int i = (int)arg;
-      stk[sp] = x[i];
+      stk[sp] = x[cols ? __ldg(cols + i) : i];
       dsk[sp++] = i == wrt ? 1.0 : 0.0;
     } else if (op == 2) {
       stk[sp] = arg;
@@ -252,14 +275,14 @@ static __device__ __noinline__ double vm_eval_dual(const double *prog, int m, in
 
 // d f_row / d x_j by two central differences, Richardson-combined (numdifftools.Jacobian as called at
 // expr.py:67; the scheme of oracle/shims/numdifftools.jacobian_fd)
-static __device__ double vm_fd1(const double *prog, int m, int row, Sh x, int j) {
-  const double xj = x[j];
+static __device__ double vm_fd1(const double *prog, int m, int row, Sh x, const int *cols, int j) {
+  const double xj = x[cols ? __ldg(cols + j) : j];
   const double h0 = SCO_FD_JAC_STEP * fmax(log1p(fabs(xj)), 1.0);
   double est[2];
   for (int k = 0; k < 2; k++) {
     const double h = h0 * (k ? 2.0 : 1.0);
     const double xp = xj + h, xm = xj - h;
-    est[k] = (vm_eval(prog, m, row, x, j, xp, -1, 0.0) - vm_eval(prog, m, row, x, j, xm, -1, 0.0)) / (xp - xm);
+    est[k] = (vm_eval(prog, m, row, x, cols, j, xp, -1, 0.0) - vm_eval(prog, m, row, x, cols, j, xm, -1, 0.0)) / (xp - xm);
   }
   return (4.0 * est[0] - est[1]) / 3.0;
 }
@@ -273,30 +296,32 @@ static __device__ double vm_fd2(const double *prog, Sh x, int i, int j, double f
   for (int k = 0; k < 2; k++) {
     const double hi = hi0 * (k ? 2.0 : 1.0), hj = hj0 * (k ? 2.0 : 1.0);
     if (i == j) {
-      est[k] = (vm_eval(prog, 1, 0, x, i, xi + 2.0 * hi, -1, 0.0) - 2.0 * f0 + vm_eval(prog, 1, 0, x, i, xi - 2.0 * hi, -1, 0.0)) /
+      est[k] = (vm_eval(prog, 1, 0, x, nullptr, i, xi + 2.0 * hi, -1, 0.0) - 2.0 * f0 + vm_eval(prog, 1, 0, x, nullptr, i, xi - 2.0 * hi, -1, 0.0)) /
                (4.0 * hi * hi);
     } else {
-      est[k] = (vm_eval(prog, 1, 0, x, i, xi + hi, j, xj + hj) - vm_eval(prog, 1, 0, x, i, xi + hi, j, xj - hj) -
-                vm_eval(prog, 1, 0, x, i, xi - hi, j, xj + hj) + vm_eval(prog, 1, 0, x, i, xi - hi, j, xj - hj)) /
+      est[k] = (vm_eval(prog, 1, 0, x, nullptr, i, xi + hi, j, xj + hj) - vm_eval(prog, 1, 0, x, nullptr, i, xi + hi, j, xj - hj) -
+                vm_eval(prog, 1, 0, x, nullptr, i, xi - hi, j, xj + hj) + vm_eval(prog, 1, 0, x, nullptr, i, xi - hi, j, xj - hj)) /
                (4.0 * hi * hj);
     }
   }
   return (4.0 * est[0] - est[1]) / 3.0;
 }
 
+// With a column map row r is a function of its n_in inputs: n_in Jacobian entries per row instead of n.
 template <int TEAM>
 __device__ void eval_vm(const DevStruct &S, const DevBlock &B, const double *prog, Sh x, Sh f, double *Jout) {
-  const int n = S.n, m = B.m;
-  for (int r = threadIdx.x; r < m; r += TEAM) f[r] = vm_eval(prog, m, r, x, -1, 0.0, -1, 0.0);
+  const int *cm = B.n_in ? S.jcol_g + B.joff : nullptr;  // column map
+  const int n = cm ? B.n_in : S.n, m = B.m;
+  for (int r = threadIdx.x; r < m; r += TEAM) f[r] = vm_eval(prog, m, r, x, cm ? cm + r * n : nullptr, -1, 0.0, -1, 0.0);
   if (Jout) {
     if (B.ipar[3]) {  // analytic: the program differentiated in forward mode (one pass per entry)
       for (int e = threadIdx.x; e < m * n; e += TEAM) {
         double d;
-        vm_eval_dual(prog, m, e / n, x, e % n, &d);
+        vm_eval_dual(prog, m, e / n, x, cm ? cm + (e / n) * n : nullptr, e % n, &d);
         Jout[e] = d;
       }
     } else {
-      for (int e = threadIdx.x; e < m * n; e += TEAM) Jout[e] = vm_fd1(prog, m, e / n, x, e % n);
+      for (int e = threadIdx.x; e < m * n; e += TEAM) Jout[e] = vm_fd1(prog, m, e / n, x, cm ? cm + (e / n) * n : nullptr, e % n);
     }
   }
 }

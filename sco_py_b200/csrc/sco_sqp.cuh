@@ -60,7 +60,7 @@ struct SqpSolver {
   // exact objective: quadratic terms + the non-quadratic term (prob.py:573-574)
   __device__ double objective() {
     double v = objective_quad();
-    if (S.obj_len) v += vm_eval(field_ptr(S, S.objp, prm), 1, 0, xc, -1, 0.0, -1, 0.0);
+    if (S.obj_len) v += vm_eval(field_ptr(S, S.objp, prm), 1, 0, xc, nullptr, -1, 0.0, -1, 0.0);
     return v;
   }
 
@@ -86,7 +86,7 @@ struct SqpSolver {
   // Leaves H in w.Hq (n x n), b in w.Hq[n*n], A in w.gq.  Uses w.Sm as scratch.
   __device__ void convexify_objective() {
     const double *prog = field_ptr(S, S.objp, prm);
-    const double f0 = vm_eval(prog, 1, 0, xc, -1, 0.0, -1, 0.0);
+    const double f0 = vm_eval(prog, 1, 0, xc, nullptr, -1, 0.0, -1, 0.0);
     for (int e = tid; e < n * n; e += TEAM) {
       const int i = e / n, j = e % n;
       if (i <= j) {
@@ -96,8 +96,8 @@ struct SqpSolver {
       }
     }
     for (int j = tid; j < n; j += TEAM) {  // gradient: finite differences, or the program's own derivative
-      if (S.obj_flags & 1) { double d; vm_eval_dual(prog, 1, 0, xc, j, &d); w.xt[j] = d; }
-      else w.xt[j] = vm_fd1(prog, 1, 0, xc, j);
+      if (S.obj_flags & 1) { double d; vm_eval_dual(prog, 1, 0, xc, nullptr, j, &d); w.xt[j] = d; }
+      else w.xt[j] = vm_fd1(prog, 1, 0, xc, nullptr, j);
     }
     sync();
     if (tid < 32) {

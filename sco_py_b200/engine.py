@@ -81,6 +81,9 @@ class Engine(object):
             for k in range(8):
                 cb.ipar[k] = int(b.ipar[k])
             cb.par, cb.val = _field(b.par), _field(b.val)
+            if b.cols is not None:
+                cb.n_in = int(np.shape(b.cols)[1])
+                cb.cols = hold(b.cols, np.int32)
         h = ctypes.c_void_p()
         _lib.check(self.lib.sco_create(ctypes.byref(cs), device, ctypes.byref(h)))
         self.h = h

@@ -20,6 +20,9 @@ FAM_QUADFORM = 1   # f_j = 0.5 x'P_j x + a_j'x        (packed-upper P_j, then a_
 FAM_CIRCLE2D = 2   # f_{t,k} = R_k - ||p_t - c_k||    (centres K x 2, radii K)
 FAM_FK7 = 3        # flange position of a 7-link DH chain on x[-7:], FD Jacobian
 FAM_VM = 4         # stack program of sco_py_b200.sym, finite-difference Jacobian (dense rows)
+# A block with a column map (Block.cols, include/sco_b200.h) reads the inputs of row r from x[cols[r]] instead:
+# QUADFORM / VM rows are functions of their cols.shape[1] inputs, CIRCLE2D reads one point per row, FK7 one
+# seven-joint instance per three rows.
 
 CNT_LEQ = 0        # LEqExpr  -> hinge penalty, 1 slack per row   (expr.py:353-371)
 CNT_EQ = 1         # EqExpr   -> abs penalty,   2 slacks per row  (expr.py:314-332)
@@ -44,6 +47,12 @@ class Block:
     ipar: List[int] = field(default_factory=lambda: [0] * 8)
     group_mask: int = 1              # bit g <=> member of constraint group g
     jw: int = 0                      # Jacobian entries stored per row (ELL width)
+    cols: Optional[np.ndarray] = None  # (m, n_in) int32 column map, or None: the family's implied columns
+
+    @property
+    def n_in(self):
+        """Inputs per row of a block with a column map (None without one)."""
+        return None if self.cols is None else int(self.cols.shape[1])
 
 
 @dataclass
@@ -82,6 +91,8 @@ class Structure:
         """Column index of every stored Jacobian slot of block bi: (m, jw) int32."""
         b = self.blocks[bi]
         n = self.n
+        if b.cols is not None:
+            return np.asarray(b.cols, dtype=np.int32)
         if b.family == FAM_QUADFORM:
             return np.tile(np.arange(n, dtype=np.int32), (b.m, 1))
         if b.family == FAM_CIRCLE2D:
