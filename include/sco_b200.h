@@ -37,6 +37,7 @@ extern "C" {
 
 #define SCO_MAX_BLOCKS 16
 #define SCO_MAX_GROUPS 8
+#define SCO_MAX_OBJ_BLOCKS 4
 
 /* nonlinear constraint families evaluated on device (closed set; the reference takes
  * black-box Python callables, sco_py/expr.py:22-25) */
@@ -104,6 +105,15 @@ typedef struct {
 } sco_block_desc;
 
 typedef struct {
+  int32_t m;           /* terms, one scalar program row each */
+  int32_t n_in;        /* inputs per term, 1..64 */
+  int32_t n_instr;     /* instructions of the packed program */
+  int32_t flags;       /* bit 0: forward-mode gradient (SymExpr analytic=True) */
+  sco_field prog;      /* m row offsets, then 2*n_instr */
+  const int32_t *cols; /* host, m*n_in column indices (the Variable's order) */
+} sco_obj_block_desc;
+
+typedef struct {
   int32_t n;        /* user variables (sorted-name order, osqp_utils.py:136-143) */
   int32_t m_lin;    /* linear Eq/LEq rows added at add_cnt_expr time (prob.py:317-346) */
   int32_t n_blocks; /* nonlinear constraint blocks */
@@ -137,6 +147,18 @@ typedef struct {
    * (prob.py:369-412) -- the first trust region overwrites them (variable.py:37-45).  -1 = (-inf, +inf). */
   sco_field lb0;
   sco_field ub0;
+  /* Non-quadratic objective terms, each bound to its own Variable (prob.py:97-103; BoundExpr, expr.py:413-437).
+   * Terms with the same input count and derivative mode share a block: one scalar program row per term, and a
+   * column map like that of a constraint block -- term r of a block reads x[cols[r*n_in + i]] as its local input i.
+   * Every term is convexified on its own, as Expr.convexify(degree=2) does per term (expr.py:143-153): H_t = the
+   * numerical Hessian over its n_in inputs, H_t+ = H_t - min(lambda_min(H_t), 0) I, A_t = g_t - x_t'H_t+,
+   * b_t = 0.5 x_t'H_t+ x_t - g_t.x_t + f_t; the QP adds sum_t scatter(H_t+) to P and sum_t scatter(A_t) to q
+   * (prob.py:348-367), the merits sum_t f_t (prob.py:573-574) and sum_t of the models (prob.py:624-626).
+   * Indices lie in [0, n) and do not repeat within a term, 1 <= n_in <= 64.  obj_prog above is the same thing for
+   * one term over all n variables in QP order (n <= 64); a structure has one or the other, not both.  Hosts that
+   * memset this struct get n_obj_blocks = 0. */
+  int32_t n_obj_blocks;
+  sco_obj_block_desc obj_blocks[SCO_MAX_OBJ_BLOCKS];
 } sco_structure_desc;
 
 typedef struct {
@@ -253,9 +275,11 @@ int sco_solve_batch_host(sco_handle *h, int64_t B, const double *params, const d
  * obj[B] = 0.5x'Qx + q'x + c.  Any output may be NULL. */
 int sco_convexify(sco_handle *h, int64_t B, const double *d_params, const double *d_x, double *d_f,
                   double *d_J, double *d_b, double *d_obj, void *stream);
-/* Same, plus the convex degree-2 model of the non-quadratic objective term (Expr.hess / _num_hess and
- * Expr.convexify degree 2, expr.py:102-128,143-153): H+ = H - min(lambda_min, 0) I [B,n,n], A = grad - x'H+ [B,n],
- * b = 0.5 x'H+x - grad.x + f [B].  Any output may be NULL; an error if the structure has no such term. */
+/* Same, plus the convex degree-2 model of the non-quadratic objective terms (Expr.hess / _num_hess and
+ * Expr.convexify degree 2, expr.py:102-128,143-153), each term convexified on its own and the models summed:
+ * H+ = sum_t scatter(H_t - min(lambda_min(H_t), 0) I) [B,n,n], A = sum_t scatter(grad_t - x_t'H_t+) [B,n],
+ * b = sum_t (0.5 x_t'H_t+ x_t - grad_t.x_t + f_t) [B].  Any output may be NULL; an error if the structure has no such
+ * term. */
 int sco_convexify_model(sco_handle *h, int64_t B, const double *d_params, const double *d_x, double *d_f,
                         double *d_J, double *d_b, double *d_obj, double *d_H, double *d_g, double *d_c,
                         void *stream);

@@ -11,6 +11,7 @@ LIB_PATH = os.environ.get("SCO_B200_LIB", os.path.join(PKG, "libsco_b200.so"))  
 
 MAX_BLOCKS = 16
 MAX_GROUPS = 8
+MAX_OBJ_BLOCKS = 4
 
 c_i32, c_i64, c_dbl, c_vp = ctypes.c_int32, ctypes.c_int64, ctypes.c_double, ctypes.c_void_p
 
@@ -25,6 +26,11 @@ class CBlock(ctypes.Structure):
                 ("cols", c_vp)]
 
 
+class CObjBlock(ctypes.Structure):
+    _fields_ = [("m", c_i32), ("n_in", c_i32), ("n_instr", c_i32), ("flags", c_i32), ("prog", CField),
+                ("cols", c_vp)]
+
+
 class CStructure(ctypes.Structure):
     _fields_ = [("n", c_i32), ("m_lin", c_i32), ("n_blocks", c_i32), ("n_groups", c_i32),
                 ("stride", c_i64), ("shared_len", c_i64),
@@ -32,7 +38,8 @@ class CStructure(ctypes.Structure):
                 ("lin_rowptr", c_vp), ("lin_col", c_vp), ("lin_val", c_vp), ("shared", c_vp),
                 ("group_overlap", c_vp), ("blocks", CBlock * MAX_BLOCKS),
                 ("obj_prog", CField), ("obj_prog_len", c_i32), ("obj_prog_flags", c_i32),
-                ("qa", CField), ("lb0", CField), ("ub0", CField)]
+                ("qa", CField), ("lb0", CField), ("ub0", CField),
+                ("n_obj_blocks", c_i32), ("obj_blocks", CObjBlock * MAX_OBJ_BLOCKS)]
 
 
 class CBatchIO(ctypes.Structure):

@@ -10,7 +10,8 @@ kernels run on (structure.py / include/sco_b200.h) plus one parameter row per pr
 import numpy as np
 
 from . import expr as E
-from .structure import CNT_EQ, CNT_LEQ, MAX_BLOCKS, MAX_GROUPS, Block, Field, Structure
+from .structure import (CNT_EQ, CNT_LEQ, MAX_BLOCKS, MAX_GROUPS, MAX_OBJ_BLOCKS, MAX_OBJ_INPUTS, Block, Field,
+                        ObjBlock, Structure)
 
 
 class UnsupportedProblem(Exception):
@@ -30,7 +31,8 @@ class Compiled(object):
         self.c = 0.0
         self.lin_A = self.lin_l = self.lin_u = None
         self.blocks = []         # device blocks: (family expr, cnt_type, val[m], group ids, column map [m, n_in] or None)
-        self.obj_prog = None     # SymExpr of a non-quadratic objective
+        self.obj_prog = None     # SymExpr of a non-quadratic objective over all variables in QP order (one term)
+        self.obj_blocks = []     # every other case: (PackedRows of scalar SymExpr terms, column map [m, n_in])
         self.gids = []
 
 
@@ -136,22 +138,43 @@ def compile_problem(prob):
                 cp.qa = np.zeros(n)
             np.add.at(cp.qa, cols, A.sum(axis=0))  # eval() sums the rows (prob.py:573-574)
             cp.c += float(np.asarray(e.b, dtype=float).sum())
-    if prob._nonquad_obj_exprs:  # convexified to degree 2 on the device (expr.py:143-153)
-        if len(prob._nonquad_obj_exprs) > 1:
-            raise UnsupportedProblem("more than one non-quadratic objective term: add them up in one SymExpr")
-        b = prob._nonquad_obj_exprs[0]
-        cols = _columns(b.var, col_of)
-        if not (isinstance(b.expr, E.SymExpr) and b.expr.m == 1 and cols.size == n and
-                np.array_equal(cols, np.arange(n))):
-            raise UnsupportedProblem("a non-quadratic objective must be a scalar SymExpr (sco_py_b200.sym) bound to "
-                                     "a Variable that holds all scalar variables in QP order; black-box callables "
-                                     "cannot run on the device and there is no CPU fallback")
-        if n > 64:
-            raise UnsupportedProblem("non-quadratic objectives are limited to 64 variables (n x n Hessian model per "
-                                     "problem in shared memory, n^2 / 2 program evaluations per convexification)")
-        if b.expr.n != n:
-            raise UnsupportedProblem("the objective SymExpr is over %d variables, the problem has %d" % (b.expr.n, n))
-        cp.obj_prog = b.expr
+    if prob._nonquad_obj_exprs:  # each term convexified to degree 2 on its own, on the device (expr.py:143-153)
+        terms = []
+        for b in prob._nonquad_obj_exprs:
+            cols = _columns(b.var, col_of)
+            e = b.expr
+            if not (isinstance(e, E.SymExpr) and e.m == 1):
+                raise UnsupportedProblem("a non-quadratic objective term must be a scalar SymExpr (sco_py_b200.sym) "
+                                         "bound to a Variable; black-box callables cannot run on the device and there "
+                                         "is no CPU fallback")
+            if e.n != cols.size:
+                raise UnsupportedProblem("an objective SymExpr over %d variables is bound to a Variable of %d"
+                                         % (e.n, cols.size))
+            uniq, counts = np.unique(cols, return_counts=True)
+            if (counts > 1).any():
+                raise UnsupportedProblem("an objective term's Variable lists scalar variable %r more than once"
+                                         % (cp.ovars[int(uniq[counts > 1][0])].var_name,))
+            if cols.size > MAX_OBJ_INPUTS:
+                raise UnsupportedProblem("an objective term over %d variables: the limit is %d inputs per term "
+                                         "(n_in x n_in Hessian model per term in shared memory, n_in^2 / 2 program "
+                                         "evaluations per convexification)" % (cols.size, MAX_OBJ_INPUTS))
+            terms.append((e, cols))
+        e, cols = terms[0]
+        if len(terms) == 1 and cols.size == n and np.array_equal(cols, np.arange(n)):
+            cp.obj_prog = e  # one term over every variable in QP order: the structure of earlier versions
+        else:
+            packs = {}  # terms of one input count and derivative mode -> index into cp.obj_blocks
+            for e, cols in terms:
+                key = (e.n, bool(e.analytic))
+                if key not in packs:
+                    packs[key] = len(cp.obj_blocks)
+                    cp.obj_blocks.append(([], []))
+                cp.obj_blocks[packs[key]][0].append(e)
+                cp.obj_blocks[packs[key]][1].append(cols)
+            if len(cp.obj_blocks) > MAX_OBJ_BLOCKS:
+                raise UnsupportedProblem("%d objective blocks (scalar SymExpr terms of one input count and derivative "
+                                         "mode share one): the limit is %d" % (len(cp.obj_blocks), MAX_OBJ_BLOCKS))
+            cp.obj_blocks = [(PackedRows(parts), np.vstack(maps)) for parts, maps in cp.obj_blocks]
     # ---- linear constraints
     rows_A, rows_l, rows_u = [], [], []
     for b, kind in prob._lin_cnt_exprs:
@@ -234,7 +257,14 @@ def group_key(cp):
             None if cp.lin_A is None else (cp.lin_A.shape, cp.lin_A.tobytes()), tuple(cp.gids),
             tuple((b[0].family, b[0].m, b[1], tuple(b[0].ipar), tuple(b[3])) +
                   (() if b[4] is None else (b[4].shape, b[4].tobytes())) for b in cp.blocks),
-            None if cp.obj_prog is None else (cp.obj_prog.n_instr, cp.obj_prog.analytic))
+            None if cp.obj_prog is None else (cp.obj_prog.n_instr, cp.obj_prog.analytic)) + _obj_key(cp)
+
+
+def _obj_key(cp):
+    """Identity of the objective blocks (empty without any, so that other keys stay as they were)."""
+    if not cp.obj_blocks:
+        return ()
+    return (tuple((pk.m, pk.n, pk.n_instr, int(pk.ipar[3]), cols.tobytes()) for pk, cols in cp.obj_blocks),)
 
 
 def compile_batch(probs, compiled=None):
@@ -253,7 +283,8 @@ def compile_batch(probs, compiled=None):
                     (a[4] is None or np.array_equal(a[4], b[4])) for a, b in zip(c.blocks, c0.blocks)) and
                 (c.obj_prog is None) == (c0.obj_prog is None) and (c.qa is None) == (c0.qa is None) and
                 (c.lb0 is None) == (c0.lb0 is None) and
-                (c.obj_prog is None or (c.obj_prog.n_instr == c0.obj_prog.n_instr and c.obj_prog.analytic == c0.obj_prog.analytic)))
+                (c.obj_prog is None or (c.obj_prog.n_instr == c0.obj_prog.n_instr and c.obj_prog.analytic == c0.obj_prog.analytic)) and
+                _obj_key(c) == _obj_key(c0))
         if not same:
             raise UnsupportedProblem("problem %d of the batch does not share the structure of problem 0" % i)
     shared_parts, shared_off = [], 0
@@ -311,6 +342,16 @@ def compile_batch(probs, compiled=None):
             of = own_field(p0.size)
             fills.append((of, lambda c: c.obj_prog.params()))
         kw.update(obj_prog=of, obj_prog_len=c0.obj_prog.n_instr, obj_prog_flags=int(c0.obj_prog.analytic))
+    obj_blocks = []
+    for oi, (pk, cols) in enumerate(c0.obj_blocks):
+        p0 = pk.params()
+        if B > 1 and all(np.array_equal(c.obj_blocks[oi][0].params(), p0) for c in cps[1:]):
+            of = shared_field(p0)
+        else:
+            of = own_field(p0.size)
+            fills.append((of, lambda c, oi=oi: c.obj_blocks[oi][0].params()))
+        obj_blocks.append(ObjBlock(of, pk.m, pk.n, pk.n_instr, int(pk.ipar[3]),
+                                   np.ascontiguousarray(cols, dtype=np.int32)))
     blocks = []
     for bi, (fam, ctype, val, gids, cols) in enumerate(c0.blocks):
         p0 = fam.params()
@@ -337,7 +378,7 @@ def compile_batch(probs, compiled=None):
                 overlap[c0.gids.index(g), c0.gids.index(o)] = 1
     st = Structure(n=n, stride=max(off, 1), Q=Qf, q=qf, c=cf, blocks=blocks, n_groups=ng,
                    group_overlap=overlap if ng > 1 else None,
-                   shared=np.concatenate(shared_parts) if shared_parts else None, **kw)
+                   shared=np.concatenate(shared_parts) if shared_parts else None, obj_blocks=obj_blocks, **kw)
     params = np.zeros((B, st.stride))
     x0 = np.empty((B, n))
     for i, c in enumerate(cps):
@@ -355,13 +396,17 @@ def signature(st):
     lin = None
     if st.m_lin:
         lin = (st.lin_rowptr.tobytes(), st.lin_col.tobytes(), st.lin_val.tobytes(), fld(st.lin_l), fld(st.lin_u))
-    return (st.n, st.stride, fld(st.Q), fld(st.q), fld(st.c), fld(st.qa), fld(st.lb0), fld(st.ub0), fld(st.obj_prog),
+    sig = (st.n, st.stride, fld(st.Q), fld(st.q), fld(st.c), fld(st.qa), fld(st.lb0), fld(st.ub0), fld(st.obj_prog),
             st.obj_prog_len, st.obj_prog_flags, st.m_lin, lin, st.n_groups,
             None if st.group_overlap is None else st.group_overlap.tobytes(),
             None if st.shared is None else st.shared.tobytes(),
             tuple((b.family, b.cnt_type, b.m, fld(b.par), fld(b.val), tuple(b.ipar), b.group_mask, b.jw) +
                   (() if b.cols is None else (b.cols.shape, np.ascontiguousarray(b.cols, dtype=np.int32).tobytes()))
                   for b in st.blocks))
+    if st.obj_blocks:  # appended only when present: the signatures of other structures stay as they were
+        sig += (tuple((fld(o.prog), o.m, o.n_in, o.n_instr, o.flags,
+                       np.ascontiguousarray(o.cols, dtype=np.int32).tobytes()) for o in st.obj_blocks),)
+    return sig
 
 
 def scatter_solution(cp, x):

@@ -6,7 +6,7 @@ results somebody obtained for it, so that benchmarks are reproducible and regres
     format            "sco_b200.batch"          version  1
     structure         JSON (n, stride, every Field as [off, shared], blocks, groups)  + the structure's arrays
                       (lin_rowptr / lin_col / lin_val, shared, group_overlap; st_cols<i>: column map of block i,
-                      only for blocks that have one)
+                      only for blocks that have one; st_ocols<i>: column map of objective block i)
     params [B, stride] float64      x0 [B, n] float64
     settings          JSON of the solver / OSQP settings the results belong to (optional)
     expected_*        verdict [B] int32, x [B, n], max_vio [B], objective [B], nonconverged [B] (optional)
@@ -23,7 +23,7 @@ import sys
 
 import numpy as np
 
-from .structure import Block, Field, Structure
+from .structure import Block, Field, ObjBlock, Structure
 
 FORMAT = "sco_b200.batch"
 VERSION = 1
@@ -42,13 +42,18 @@ def structure_to_json(st):
         d[name] = _fld(getattr(st, name))
     d["blocks"] = [dict(family=int(b.family), cnt_type=int(b.cnt_type), m=int(b.m), par=_fld(b.par), val=_fld(b.val),
                         ipar=[int(v) for v in b.ipar], group_mask=int(b.group_mask), jw=int(b.jw)) for b in st.blocks]
+    if st.obj_blocks:  # only when present: files and signatures of other structures stay as they were
+        d["obj_blocks"] = [dict(prog=_fld(o.prog), m=int(o.m), n_in=int(o.n_in), n_instr=int(o.n_instr),
+                                flags=int(o.flags)) for o in st.obj_blocks]
     return d
 
 
 def _maps(st):
     """{array name: column map} of the blocks that have one."""
-    return {"cols%d" % i: np.ascontiguousarray(b.cols, dtype=np.int32) for i, b in enumerate(st.blocks)
+    maps = {"cols%d" % i: np.ascontiguousarray(b.cols, dtype=np.int32) for i, b in enumerate(st.blocks)
             if b.cols is not None}
+    maps.update({"ocols%d" % i: np.ascontiguousarray(o.cols, dtype=np.int32) for i, o in enumerate(st.obj_blocks)})
+    return maps
 
 
 def structure_from_json(d, arrays):
@@ -59,6 +64,8 @@ def structure_from_json(d, arrays):
     for name in _ARRAYS:
         if name in arrays:
             kw[name] = arrays[name]
+    kw["obj_blocks"] = [ObjBlock(Field(*o["prog"]), o["m"], o["n_in"], o["n_instr"], o["flags"], arrays["ocols%d" % i])
+                        for i, o in enumerate(d.get("obj_blocks", []))]
     return Structure(n=d["n"], stride=d["stride"], m_lin=d["m_lin"], n_groups=d["n_groups"],
                      obj_prog_len=d.get("obj_prog_len", 0), obj_prog_flags=d.get("obj_prog_flags", 0), blocks=blocks, **kw)
 

@@ -111,7 +111,12 @@ static void build_layout(DevStruct &S, int team) {
   L.red = take((std::max(team / 32, 8) + 1) * 16);  // one 16-double slot per warp + one for the combined results
   L.msk = take((mp * S.mw + 1) / 2);
   L.stage = take(std::max((team / 32) * S.stage_per_warp, 100));
-  L.Hq = take(S.obj_len ? n * n + 2 : 0); L.gq = take(S.obj_len ? n : 0);
+  // objective terms: the eigenvalue shift runs one term per warp, on at most 4,096 doubles of scratch in all
+  S.nwj = S.n_ob ? std::max(1, std::min(std::min(S.n_terms, team / 32), 4096 / (S.n_in_max * S.n_in_max))) : 0;
+  int ot_len = 0;
+  for (int b = 0; b < S.n_ob; b++) ot_len += S.ob[b].m * (S.ob[b].n_in * (S.ob[b].n_in + 1) / 2 + S.ob[b].n_in + 1);
+  L.ot = take(ot_len); L.jac = take(S.nwj * S.n_in_max * S.n_in_max);
+  L.Hv = take(S.n_ob ? S.nnz_p : 0); L.gq = take(S.n_ob ? n : 0); L.oc = take(S.n_ob ? 1 : 0);
   L.ps = take(4 * n);
   L.total = off;
 }
@@ -208,6 +213,29 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
                field_ok(desc->lin_l, desc->m_lin) && field_ok(desc->lin_u, desc->m_lin) && field_ok(desc->qa, n_) &&
                field_ok(desc->lb0, n_) && field_ok(desc->ub0, n_) &&
                (desc->obj_prog_len <= 0 || field_ok(desc->obj_prog, 1 + 2LL * desc->obj_prog_len));
+    if (desc->n_obj_blocks < 0 || desc->n_obj_blocks > SCO_MAX_OBJ_BLOCKS)
+      return fail(SCO_ERR_ARG, "n_obj_blocks = %d outside [0, %d]", desc->n_obj_blocks, SCO_MAX_OBJ_BLOCKS);
+    if (desc->obj_prog_len > 0 && desc->n_obj_blocks > 0)
+      return fail(SCO_ERR_ARG, "obj_prog and objective blocks are both set: a structure has one or the other");
+    for (int oi = 0; oi < desc->n_obj_blocks && okf; oi++) {
+      const sco_obj_block_desc &o = desc->obj_blocks[oi];
+      if (o.m <= 0 || o.n_instr <= 0) return fail(SCO_ERR_ARG, "objective block %d: m and n_instr must be positive", oi);
+      if (o.n_in < 1 || o.n_in > 64)
+        return fail(SCO_ERR_ARG, "objective block %d: n_in = %d outside [1, 64] (inputs per term)", oi, o.n_in);
+      if (!o.cols) return fail(SCO_ERR_ARG, "objective block %d: cols is null", oi);
+      for (int r = 0; r < o.m; r++) {
+        const int32_t *c = o.cols + (size_t)r * o.n_in;
+        for (int i = 0; i < o.n_in; i++) {
+          if (c[i] < 0 || c[i] >= n_)
+            return fail(SCO_ERR_ARG, "objective block %d term %d: column %d outside [0, %d)", oi, r, c[i], (int)n_);
+          for (int k = 0; k < i; k++)
+            if (c[k] == c[i]) return fail(SCO_ERR_ARG, "objective block %d term %d: column %d repeats", oi, r, c[i]);
+        }
+      }
+      if (o.prog.off < 0) return fail(SCO_ERR_ARG, "objective block %d: the program is missing", oi);
+      if (!field_ok(o.prog, o.m + 2LL * o.n_instr))
+        return fail(SCO_ERR_ARG, "objective block %d: the program field lies outside its parameter block", oi);
+    }
     for (int bi = 0; bi < desc->n_blocks && okf; bi++) {
       const sco_block_desc &b = desc->blocks[bi];
       if (b.m <= 0) return fail(SCO_ERR_ARG, "block %d: m must be positive", bi);
@@ -261,9 +289,27 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
   S.Q = cvt(desc->Q); S.q = cvt(desc->q); S.c = cvt(desc->c);
   S.lin_l = cvt(desc->lin_l); S.lin_u = cvt(desc->lin_u);
   S.qa = cvt(desc->qa); S.lb0 = cvt(desc->lb0); S.ub0 = cvt(desc->ub0);
-  S.objp = cvt(desc->obj_prog); S.obj_len = desc->obj_prog_len > 0 && desc->obj_prog.off >= 0 ? desc->obj_prog_len : 0;
-  S.obj_flags = desc->obj_prog_flags;
-  if (S.obj_len && n > 64) { delete h; return fail(SCO_ERR_UNSUPPORTED, "non-quadratic objectives are limited to 64 variables"); }
+  // objective terms: the one-term obj_prog becomes a block of one term over all n variables in QP order
+  const bool legacy_obj = desc->obj_prog_len > 0 && desc->obj_prog.off >= 0;
+  if (legacy_obj && n > 64) { delete h; return fail(SCO_ERR_UNSUPPORTED, "non-quadratic objectives are limited to 64 variables"); }
+  std::vector<int> ob_cols;
+  S.n_ob = legacy_obj ? 1 : desc->n_obj_blocks;
+  for (int oi = 0, t0 = 0, toff = 0; oi < S.n_ob; oi++) {
+    DevObjBlock &d = S.ob[oi];
+    if (legacy_obj) {
+      d.m = 1; d.n_in = n; d.flags = desc->obj_prog_flags; d.prog = cvt(desc->obj_prog);
+      for (int j = 0; j < n; j++) ob_cols.push_back(j);
+    } else {
+      const sco_obj_block_desc &o = desc->obj_blocks[oi];
+      d.m = o.m; d.n_in = o.n_in; d.flags = o.flags; d.prog = cvt(o.prog);
+      ob_cols.insert(ob_cols.end(), o.cols, o.cols + (size_t)o.m * o.n_in);
+    }
+    d.t0 = t0; d.toff = toff; d.coff = (int)ob_cols.size() - d.m * d.n_in;
+    t0 += d.m;
+    toff += d.m * (d.n_in * (d.n_in + 1) / 2 + d.n_in + 1);
+    S.n_terms = t0;
+    S.n_in_max = std::max(S.n_in_max, d.n_in);
+  }
   for (int g = 0; g < desc->n_groups; g++) {
     int bits = 0;
     if (desc->group_overlap)
@@ -365,17 +411,62 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
   }
   std::vector<double> shared_v;
   if (desc->shared_len > 0 && desc->shared) shared_v.assign(desc->shared, desc->shared + desc->shared_len);
-  // pattern of Psym = (Q + Q') / 2 by column: exact for a shared Q, dense for a per-problem Q, empty without Q
+  // pattern of Psym = (Q + Q') / 2 by column: exact for a shared Q, dense for a per-problem Q, empty without Q; united
+  // with the n_in x n_in block of every objective term
   std::vector<int> P_cptr(n + 1, 0), P_row;
-  if (desc->Q.off >= 0) {
-    for (int j = 0; j < n; j++) {
-      for (int i = 0; i < n; i++) {
-        bool nz = true;
-        if (desc->Q.shared) nz = shared_v[desc->Q.off + (size_t)i * n + j] != 0.0 || shared_v[desc->Q.off + (size_t)j * n + i] != 0.0;
-        if (nz) P_row.push_back(i);
+  std::vector<int> hv_ptr, hv_src, gq_ptr(n + 1, 0), gq_src;
+  {
+    std::vector<int> pidx((size_t)n * n, -1);  // (i, j) -> pattern entry
+    if (desc->Q.off >= 0)
+      for (int j = 0; j < n; j++)
+        for (int i = 0; i < n; i++) {
+          bool nz = true;
+          if (desc->Q.shared) nz = shared_v[desc->Q.off + (size_t)i * n + j] != 0.0 || shared_v[desc->Q.off + (size_t)j * n + i] != 0.0;
+          if (nz) pidx[(size_t)i * n + j] = 0;
+        }
+    for (int oi = 0; oi < S.n_ob; oi++) {
+      const DevObjBlock &d = S.ob[oi];
+      for (int r = 0; r < d.m; r++) {
+        const int *c = ob_cols.data() + d.coff + (size_t)r * d.n_in;
+        for (int a = 0; a < d.n_in; a++)
+          for (int b = 0; b < d.n_in; b++) pidx[(size_t)c[a] * n + c[b]] = 0;
       }
+    }
+    for (int j = 0; j < n; j++) {
+      for (int i = 0; i < n; i++)
+        if (pidx[(size_t)i * n + j] >= 0) {
+          pidx[(size_t)i * n + j] = (int)P_row.size();
+          P_row.push_back(i);
+        }
       P_cptr[j + 1] = (int)P_row.size();
     }
+    // the term-model entries summed into each pattern entry of P and each entry of q, in term order
+    std::vector<std::vector<int>> hv(P_row.size()), gv(n);
+    for (int oi = 0; oi < S.n_ob; oi++) {
+      const DevObjBlock &d = S.ob[oi];
+      const int nn = d.n_in, ntri = nn * (nn + 1) / 2;
+      for (int r = 0; r < d.m; r++) {
+        const int *c = ob_cols.data() + d.coff + (size_t)r * nn;
+        const int base = d.toff + r * (ntri + nn + 1);
+        for (int a = 0; a < nn; a++) {
+          for (int b = 0; b < nn; b++) {
+            const int lo = std::min(a, b), hi = std::max(a, b);
+            hv[pidx[(size_t)c[a] * n + c[b]]].push_back(base + lo * nn - lo * (lo - 1) / 2 + (hi - lo));
+          }
+          gv[c[a]].push_back(base + ntri + a);
+        }
+      }
+    }
+    hv_ptr.assign(P_row.size() + 1, 0);
+    for (size_t p = 0; p < hv.size(); p++) {
+      hv_ptr[p + 1] = hv_ptr[p] + (int)hv[p].size();
+      hv_src.insert(hv_src.end(), hv[p].begin(), hv[p].end());
+    }
+    for (int j = 0; j < n; j++) {
+      gq_ptr[j + 1] = gq_ptr[j] + (int)gv[j].size();
+      gq_src.insert(gq_src.end(), gv[j].begin(), gv[j].end());
+    }
+    S.nnz_p = (int)P_row.size();
   }
   int rc = 0;
   rc |= upload(h, row_goff, &S.row_goff); rc |= upload(h, row_soff, &S.row_soff);
@@ -386,6 +477,8 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
   rc |= upload(h, lcptr, &S.lin_cptr); rc |= upload(h, lcentry, &S.lin_centry); rc |= upload(h, lcrow, &S.lin_crow);
   rc |= upload(h, shared_v, &S.shared);
   rc |= upload(h, P_cptr, &S.P_cptr); rc |= upload(h, P_row, &S.P_row);
+  rc |= upload(h, ob_cols, &S.ob_cols); rc |= upload(h, hv_ptr, &S.hv_ptr); rc |= upload(h, hv_src, &S.hv_src);
+  rc |= upload(h, gq_ptr, &S.gq_ptr); rc |= upload(h, gq_src, &S.gq_src);
   {
     int bw = 0;
     for (int j = 0; j < n; j++)
@@ -402,7 +495,6 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
         for (int k = 0; k < row_w[i]; k++) { lo = std::min(lo, jcol[row_goff[i] + k]); hi = std::max(hi, jcol[row_goff[i] + k]); }
         bw = std::max(bw, hi - lo);
       }
-    if (S.obj_len) bw = n - 1;  // the degree-2 model of a non-quadratic objective is dense
     S.s_bw = std::min(bw, n - 1);
     // thread-per-entity ADMM loop (sco_qp.cuh: fast_role keeps SCO_EN = 8 row entries / SCO_EH = 4 + 4 column entries
     // in registers and has no path for more)
@@ -422,7 +514,7 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
   if (rc) { sco_destroy(h); return SCO_ERR_CUDA; }
   // ---- dense fast path: one dense hinge block over all variables, no linear rows, sizes within the instantiated table
   S.dense_kind = 0;
-  if (desc->m_lin == 0 && S.obj_len == 0 && desc->n_blocks == 1 && desc->blocks[0].family == SCO_FAM_QUADFORM &&
+  if (desc->m_lin == 0 && S.n_ob == 0 && desc->n_blocks == 1 && desc->blocks[0].family == SCO_FAM_QUADFORM &&
       desc->blocks[0].cnt_type == SCO_CNT_LEQ && !any_map) {
     static const int table[][2] = {{8, 6}, {12, 16}, {20, 30}, {32, 32}};  // keep in sync with QPSolver::solve in sco_qp.cuh
     for (int k = 0; k < 4; k++)
@@ -443,7 +535,7 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
     build_layout(S, team);
     h->smem_bytes = (size_t)(S.L.total + ((n + 1) & ~1)) * sizeof(double);
     if (h->smem_bytes <= (size_t)prop.sharedMemPerBlockOptin) break;
-    if (!S.sws && !S.dense_kind && !S.obj_len) {
+    if (!S.sws && !S.dense_kind && !S.n_ob) {  // objective terms stay in the resident regime
       // the n x n matrix S (and its inverse) moves to a global workspace per resident team: the ADMM loop streams it
       // from L2 / HBM in every iteration (strided loop only); everything else stays in shared memory
       S.sws = n * n;
@@ -664,7 +756,7 @@ extern "C" int sco_convexify_model(sco_handle *h, int64_t B, const double *d_par
                                    double *d_f, double *d_J, double *d_b, double *d_obj, double *d_H, double *d_g,
                                    double *d_c, void *stream) {
   if (!h || !d_params || !d_x) return fail(SCO_ERR_ARG, "null argument");
-  if ((d_H || d_g || d_c) && !h->S.obj_len) return fail(SCO_ERR_ARG, "the structure has no non-quadratic objective term");
+  if ((d_H || d_g || d_c) && !h->S.n_ob) return fail(SCO_ERR_ARG, "the structure has no non-quadratic objective term");
   if (B <= 0) return SCO_OK;
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;

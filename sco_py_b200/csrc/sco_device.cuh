@@ -11,6 +11,7 @@
 
 #define SCO_DEV_MAX_BLOCKS 16
 #define SCO_DEV_MAX_GROUPS 8
+#define SCO_DEV_MAX_OBJ_BLOCKS 4
 
 #define OSQP_INFTY 1e30
 #define OSQP_MIN_SCALING 1e-4
@@ -38,6 +39,17 @@ struct DevBlock {
   DevField par, val;
 };
 
+// Non-quadratic objective terms of one input count and derivative mode (include/sco_b200.h sco_obj_block_desc; a
+// structure's obj_prog is turned into one such block over all n variables).  Term r of the block reads
+// x[ob_cols[coff + r * n_in + i]] as its input i; its convex model lives at toff + r * (n_in (n_in + 1) / 2 + n_in + 1)
+// in the term-model area (Layout::ot): the upper triangle of H_t+ (row-major), then A_t (n_in), then f_t.
+struct DevObjBlock {
+  int m, n_in, flags;  // flags bit 0: forward-mode gradient
+  int t0;              // index of its first term among all terms
+  int coff, toff;
+  DevField prog;       // m row offsets, then the code
+};
+
 // shared-memory carve-up, offsets in doubles
 struct Layout {
   int Js, S, Als;
@@ -53,7 +65,10 @@ struct Layout {
   int red;    // reduction scratch: 8 warps * 8 values
   int msk;    // m_nl * mw uint32 (counted in doubles, rounded up)
   int stage;  // per-warp staging buffers for family evaluation
-  int Hq, gq;  // degree-2 model of a non-quadratic objective: H+ (n*n, then b at [n*n]), linear term (n)
+  // convex model of the non-quadratic objective terms: per-term models (DevObjBlock), the Jacobi scratch of the
+  // eigenvalue shift (n_in_max^2 per warp), the assembled model on the pattern of P (nnz(P)), its linear term (n) and
+  // its constant (1)
+  int ot, jac, Hv, gq, oc;
   int ps;     // partial sums of S^-1 rhs: 4 column segments x n (fast_loop, sco_qp.cuh)
   int total;  // doubles
 };
@@ -109,8 +124,13 @@ struct DevStruct {
   DevField Q, q, c, lin_l, lin_u;
   DevField qa;         // AffExpr objective terms, summed (n): enters the QP with the weight of quirk C-4
   DevField lb0, ub0;   // user bounds of the scalar variables (n each): the closest-point QP honours them
-  DevField objp;       // non-quadratic objective: stack program (1 row)
-  int obj_len, obj_flags;  // its instruction count, 0 = none; bit 0: gradient by forward-mode differentiation
+  int n_ob, n_terms;   // objective blocks (0 = no non-quadratic objective term) and their terms
+  int n_in_max, nwj;   // widest term; warps that run the eigenvalue shift (each with n_in_max^2 doubles of scratch)
+  int nnz_p;           // entries of the pattern of P (P_cptr[n])
+  DevObjBlock ob[SCO_DEV_MAX_OBJ_BLOCKS];
+  const int *ob_cols;          // column maps of the objective blocks
+  const int *hv_ptr, *hv_src;  // nnz_p + 1 / per pattern entry of P: the term-model entries (H_t+) summed into it
+  const int *gq_ptr, *gq_src;  // n + 1 / per variable: the term-model entries (A_t) summed into q
   // linear rows: CSR + CSC (entry index into lin_val / Als)
   const int *lin_rowptr, *lin_col, *lin_cptr, *lin_centry, *lin_crow;
   const double *lin_val;
@@ -124,7 +144,8 @@ struct DevStruct {
   const int *pc_ptr, *pc_e, *pc_r;  // CSC over user variables: shared-memory entry index, row
   // sparsity pattern of the symmetrised objective matrix, by column (exact when Q is shared by the batch -- the
   // smoothness matrices of the trajectory configurations are block tridiagonal -- and dense otherwise; empty when
-  // there is no Q).  Column norms, P x and the assembly of S walk this instead of n entries per column.
+  // there is no Q), united with the n_in x n_in block of every objective term.  Column norms, P x and the assembly
+  // of S walk this instead of n entries per column.
   const int *P_cptr, *P_row;
   const double *shared;
   int overlap[SCO_DEV_MAX_GROUPS];  // bit g2 of overlap[g] <=> groups overlap (prob.py:139-142)
@@ -306,7 +327,7 @@ struct QPW {
   Sh red;
   ShU32 msk;
   Sh stage;
-  Sh Hq, gq;
+  Sh ot, jac, Hv, gq, oc;
   Sh ps;
   Sh xc;  // current SQP iterate, n doubles appended after the layout
   double *Sg;  // S in global memory (DevStruct::sws), else null; set by the kernel after bind()
@@ -326,7 +347,7 @@ struct QPW {
     red = Sh{L.red};
     msk = ShU32{L.msk};
     stage = Sh{L.stage};
-    Hq = Sh{L.Hq}; gq = Sh{L.gq};
+    ot = Sh{L.ot}; jac = Sh{L.jac}; Hv = Sh{L.Hv}; gq = Sh{L.gq}; oc = Sh{L.oc};
     ps = Sh{L.ps};
     xc = Sh{L.total};
     Sg = nullptr;

@@ -287,20 +287,20 @@ static __device__ double vm_fd1(const double *prog, int m, int row, Sh x, const 
   return (4.0 * est[0] - est[1]) / 3.0;
 }
 
-// d2 f / d x_i d x_j of a scalar program: central second differences at h and 2h, Richardson-combined
-// (numdifftools.Hessian as called at expr.py:108; oracle/shims/numdifftools.hessian_fd)
-static __device__ double vm_fd2(const double *prog, Sh x, int i, int j, double f0) {
-  const double xi = x[i], xj = x[j];
+// d2 f_row / d x_i d x_j: central second differences at h and 2h, Richardson-combined (numdifftools.Hessian as called
+// at expr.py:108; oracle/shims/numdifftools.hessian_fd).  i, j are local inputs of the row (x[cols[i]] with a map).
+static __device__ double vm_fd2(const double *prog, int m, int row, Sh x, const int *cols, int i, int j, double f0) {
+  const double xi = x[cols ? __ldg(cols + i) : i], xj = x[cols ? __ldg(cols + j) : j];
   const double hi0 = SCO_FD_HESS_STEP * fmax(log1p(fabs(xi)), 1.0), hj0 = SCO_FD_HESS_STEP * fmax(log1p(fabs(xj)), 1.0);
   double est[2];
   for (int k = 0; k < 2; k++) {
     const double hi = hi0 * (k ? 2.0 : 1.0), hj = hj0 * (k ? 2.0 : 1.0);
     if (i == j) {
-      est[k] = (vm_eval(prog, 1, 0, x, nullptr, i, xi + 2.0 * hi, -1, 0.0) - 2.0 * f0 + vm_eval(prog, 1, 0, x, nullptr, i, xi - 2.0 * hi, -1, 0.0)) /
+      est[k] = (vm_eval(prog, m, row, x, cols, i, xi + 2.0 * hi, -1, 0.0) - 2.0 * f0 + vm_eval(prog, m, row, x, cols, i, xi - 2.0 * hi, -1, 0.0)) /
                (4.0 * hi * hi);
     } else {
-      est[k] = (vm_eval(prog, 1, 0, x, nullptr, i, xi + hi, j, xj + hj) - vm_eval(prog, 1, 0, x, nullptr, i, xi + hi, j, xj - hj) -
-                vm_eval(prog, 1, 0, x, nullptr, i, xi - hi, j, xj + hj) + vm_eval(prog, 1, 0, x, nullptr, i, xi - hi, j, xj - hj)) /
+      est[k] = (vm_eval(prog, m, row, x, cols, i, xi + hi, j, xj + hj) - vm_eval(prog, m, row, x, cols, i, xi + hi, j, xj - hj) -
+                vm_eval(prog, m, row, x, cols, i, xi - hi, j, xj + hj) + vm_eval(prog, m, row, x, cols, i, xi - hi, j, xj - hj)) /
                (4.0 * hi * hj);
     }
   }

@@ -109,11 +109,16 @@ k_convexify(const __grid_constant__ DevStruct S, long long B, const double *__re
       const double ov = sq.objective();
       if (tid == 0) obj[b] = ov;
     }
-    if (S.obj_len) {  // Expr.convexify degree 2 of the non-quadratic objective term (expr.py:143-153)
+    if (S.n_ob) {  // Expr.convexify degree 2 of the non-quadratic objective terms, summed (expr.py:143-153)
       const int n = S.n;
-      if (Hq) for (int e = tid; e < n * n; e += TEAM) Hq[b * n * n + e] = w.Hq[e];
+      if (Hq)  // column j by one thread: zeros, then the model's entries on the pattern of P
+        for (int j = tid; j < n; j += TEAM) {
+          double *Hb = Hq + (size_t)b * n * n;
+          for (int i = 0; i < n; i++) Hb[(size_t)i * n + j] = 0.0;
+          for (int p = S.P_cptr[j]; p < S.P_cptr[j + 1]; p++) Hb[(size_t)S.P_row[p] * n + j] = w.Hv[p];
+        }
       if (gq) for (int e = tid; e < n; e += TEAM) gq[b * n + e] = w.gq[e];
-      if (cq && tid == 0) cq[b] = w.Hq[n * n];
+      if (cq && tid == 0) cq[b] = w.oc[0];
     }
     Team<TEAM>::sync();
   }

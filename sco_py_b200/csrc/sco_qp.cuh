@@ -30,7 +30,7 @@ struct QPArgs {
   double wa;          // weight of the AffExpr objective terms (S.qa) in q
   int use_pen;        // 0: no penalty rows / slacks (closest feasible point)
   int closest;        // objective |x - xs|^2
-  int has_hq;         // add the degree-2 model of a non-quadratic objective term (w.Hq, w.gq)
+  int has_hq;         // add the convex model of the non-quadratic objective terms (w.Hv on the pattern of P, w.gq)
   int tail;           // the launch's work queue is drained: favour the latency of this problem (sco_dense.cuh)
   int warm;           // same J, b, pi, kd as the previous solve of this team (only the box changed): reuse
 };
@@ -186,12 +186,12 @@ struct QPSolver {
       W_Ep = w.Ep, W_rp = w.rp, W_lp = w.lp, W_up = w.up, W_zp = w.zp, W_yp = w.yp, W_wp = w.wp,            \
       W_bb = w.bb, W_fv = w.fv, W_dyp = w.dyp, W_s = w.s, W_Ds = w.Ds, W_sl = w.sl, W_bs = w.bs,            \
       W_zs = w.zs, W_ys = w.ys, W_Es = w.Es, W_gs = w.gs, W_hs = w.hs, W_rs = w.rs, W_dss = w.dss,          \
-      W_dys = w.dys, W_Minv = w.Minv, W_red = w.red, W_stage = w.stage, W_Hq = w.Hq, W_gq = w.gq,           \
+      W_dys = w.dys, W_Minv = w.Minv, W_red = w.red, W_stage = w.stage, W_Hv = w.Hv, W_gq = w.gq,           \
       W_xc = w.xc, W_ps = w.ps;                                                                             \
   const ShU32 W_msk = w.msk;                                                                                \
   (void)W_msk; (void)W_Js; (void)W_Sm; (void)W_Als; (void)W_x; (void)W_xt; (void)W_xt2; (void)W_qh; (void)W_D; (void)W_bx; (void)W_rb; (void)W_lb; (void)W_ub; (void)W_zb; (void)W_yb; (void)W_Eb; (void)W_dxv; (void)W_dyb; (void)W_xs; (void)W_El; (void)W_rl;\
   (void)W_ll; (void)W_ul; (void)W_zl; (void)W_yl; (void)W_wl; (void)W_dyl; (void)W_Ep; (void)W_rp; (void)W_lp; (void)W_up; (void)W_zp; (void)W_yp; (void)W_wp; (void)W_bb; (void)W_fv; (void)W_dyp; (void)W_s; (void)W_Ds; (void)W_sl; (void)W_bs;\
-  (void)W_zs; (void)W_ys; (void)W_Es; (void)W_gs; (void)W_hs; (void)W_rs; (void)W_dss; (void)W_dys; (void)W_Minv; (void)W_red; (void)W_stage; (void)W_Hq; (void)W_gq; (void)W_xc; (void)W_ps;\
+  (void)W_zs; (void)W_ys; (void)W_Es; (void)W_gs; (void)W_hs; (void)W_rs; (void)W_dss; (void)W_dys; (void)W_Minv; (void)W_red; (void)W_stage; (void)W_Hv; (void)W_gq; (void)W_xc; (void)W_ps;\
   const DevIdx S(this->S);                                                                                  \
   const DevSettings st = this->st;                                                                          \
   const QPArgs a = this->a;                                                                                 \
@@ -201,9 +201,7 @@ struct QPSolver {
   (void)SS; (void)ms; (void)rho;                                                                            \
   auto psym = [&](int i, int j) -> double {                                                                 \
     if (a.closest) return i == j ? 2.0 : 0.0;                                                               \
-    double v = Qg ? 0.5 * (Qg[i * n + j] + Qg[j * n + i]) : 0.0;                                            \
-    if (a.has_hq) v += 0.5 * (W_Hq[i * n + j] + W_Hq[j * n + i]); /* prob.py:348-367 */                     \
-    return v;                                                                                               \
+    return Qg ? 0.5 * (Qg[i * n + j] + Qg[j * n + i]) : 0.0;                                                \
   };                                                                                                        \
   auto gatherAT = [&](int j, Sh vl, Sh vp) -> double {                                                      \
     double acc = 0.0;                                                                                       \
@@ -227,11 +225,10 @@ struct QPSolver {
     for (int k = 0; k < wd; k++) acc += W_Js[so + k] * v[__ldg(S.jcol_g + (go + k))];                                 \
     return acc;                                                                                             \
   };                                                                                                        \
-  /* column j of c D |Psym| D over the pattern of Psym (closest point: 2 I; objective model: dense) */        \
+  /* column j of c D |Psym| D over the pattern of Psym (closest point: 2 I) */                               \
   auto pcol_norm = [&](int j) -> double {                                                                   \
     double cp = 0.0;                                                                                        \
     if (a.closest) cp = W_D[j] * fabs(SM_LD(j * n + j));                                                     \
-    else if (a.has_hq) { for (int i = 0; i < n; i++) cp = fmax(cp, W_D[i] * fabs(SM_LD(i * n + j))); }       \
     else for (int p = __ldg(S.P_cptr + (j)); p < __ldg(S.P_cptr + (j + 1)); p++) {                              \
       const int i = __ldg(S.P_row + (p));                                                                     \
       cp = fmax(cp, W_D[i] * fabs(SM_LD(i * n + j)));                                                      \
@@ -242,7 +239,7 @@ struct QPSolver {
   auto psym_dot = [&](int j, Sh v) -> double {                                                              \
     double px = 0.0;                                                                                        \
     if (a.closest) px = 2.0 * v[j];                                                                         \
-    else if (a.has_hq) { for (int k = 0; k < n; k++) px += psym(k, j) * v[k]; }                             \
+    else if (a.has_hq) px = this->psym_dot_model(j, v);                                                     \
     else if (Qg) for (int p = __ldg(S.P_cptr + (j)); p < __ldg(S.P_cptr + (j + 1)); p++) {                      \
       const int k = __ldg(S.P_row + (p));                                                                     \
       px += 0.5 * (Qg[k * n + j] + Qg[j * n + k]) * v[k];                                                   \
@@ -251,16 +248,45 @@ struct QPSolver {
   };                                                                                                        \
   (void)psym; (void)gatherAT; (void)lin_row_dot; (void)pen_row_dot; (void)pcol_norm; (void)psym_dot;
 
+  // (Psym v)_j with the objective model: Q's part and the model's on the pattern of P, entry by entry (prob.py:348-367)
+  __device__ __noinline__ double psym_dot_model(int j, Sh v) const {
+    const double *const Qg = this->Qg;
+    const int n = this->n;
+    double px = 0.0;
+    for (int p = __ldg(S.P_cptr + (j)); p < __ldg(S.P_cptr + (j + 1)); p++) {
+      const int k = __ldg(S.P_row + (p));
+      double pv = Qg ? 0.5 * (Qg[k * n + j] + Qg[j * n + k]) : 0.0;
+      pv += w.Hv[p];
+      px += pv * v[k];
+    }
+    return px;
+  }
+
   // ================================================================== setup
   // expects (unscaled): W_lb/W_ub bounds on x, W_bb = b, W_msk, W_xs (closest point target)
 #undef SM_GLOBAL
 #define SM_GLOBAL SG  // compile-time in the two setup functions: no test per matrix element
+  // Sm <- the unscaled Psym: Q's part everywhere, then the objective model's on the pattern (no barrier at the end)
+  template <bool SG>
+  __device__ __forceinline__ void load_psym() {
+    SCO_QP_LOCALS
+    for (int e = tid; e < n * n; e += TEAM) SM_ST(e, psym(e / n, e % n));
+    if (a.has_hq) {
+      sync();
+      for (int j = tid; j < n; j += TEAM)
+        for (int p = __ldg(S.P_cptr + (j)); p < __ldg(S.P_cptr + (j + 1)); p++) {
+          const int e = __ldg(S.P_row + (p)) * n + j;
+          SM_ST(e, SM_LD(e) + W_Hv[p]);
+        }
+    }
+  }
+
   template <bool SG>
   __device__ __noinline__ void load_and_scale() {
     SCO_QP_LOCALS
     const double *qg = field_ptr(SS, SS.q, a.prm), *qag = field_ptr(SS, SS.qa, a.prm);
     const double *llg = field_ptr(SS, SS.lin_l, a.prm), *ulg = field_ptr(SS, SS.lin_u, a.prm);
-    for (int e = tid; e < n * n; e += TEAM) SM_ST(e, psym(e / n, e % n));
+    load_psym<SG>();
     for (int j = tid; j < n; j += TEAM) {
       W_qh[j] = a.closest ? -2.0 * W_xs[j]
                           : (qg ? qg[j] : 0.0) + (qag ? a.wa * qag[j] : 0.0) + (a.has_hq ? W_gq[j] : 0.0);
@@ -403,6 +429,11 @@ struct QPSolver {
   __device__ __noinline__ void assemble_and_invert(bool reload) {
     SCO_QP_LOCALS
     const double sigma = st.sigma;
+    if (reload && a.has_hq) {  // the objective model's entries are not a function of (i, j): fetch Psym into Sm first
+      load_psym<SG>();
+      sync();
+      reload = false;
+    }
     for (int i = tid; i < m_nl; i += TEAM) {
       const double kr = a.kd * W_rp[i];
       const double s1 = W_sl[i], b1 = W_bs[i];
@@ -787,14 +818,16 @@ struct QPSolver {
           k0 = wq.Eb[j]; k1 = wq.D[j];
           if (INL && f.inline_test) {
             if (this->a.closest) { pq[0] = 2.0; pa[0] = f.o_xt + j; }
-            else if (this->Qg) {
+            else if (this->Qg || this->a.has_hq) {
               const double *Qg_ = this->Qg;
               const int p0 = __ldg(SS.P_cptr + (j)), p1 = __ldg(SS.P_cptr + (j + 1));
 #pragma unroll
               for (int k = 0; k < 4; k++)
                 if (p0 + k < p1) {
                   const int r = __ldg(SS.P_row + (p0 + k));
-                  pq[k] = 0.5 * (Qg_[r * n + j] + Qg_[j * n + r]);
+                  double v = Qg_ ? 0.5 * (Qg_[r * n + j] + Qg_[j * n + r]) : 0.0;
+                  if (this->a.has_hq) v += wq.Hv[p0 + k];
+                  pq[k] = v;
                   pa[k] = f.o_xt + r;
                 }
             }
@@ -1153,7 +1186,7 @@ struct QPSolver {
     f.o_red = wq.red.off; f.c = this->c;
     f.eps_abs = this->st.eps_abs; f.eps_rel = this->st.eps_rel; f.eps_pinf = this->st.eps_prim_inf; f.eps_dinf = this->st.eps_dual_inf;
     // in-loop test: the objective matrix has at most four entries per column (or is the closest-point 2 I)
-    f.inline_test = (this->a.closest || this->S.p_narrow) && !this->a.has_hq;
+    f.inline_test = this->a.closest || this->S.p_narrow;
     for (int e = tid; e < f.K3 * n; e += TEAM) wq.ps[e] = 0.0;  // segments beyond n contribute exact zeros
     // ADMM starts from x = z = y = 0 (osqp_utils.py:195 builds a new OSQP object per call) unless the opt-in warm
     // start applies; fast_role reads its iterates from these arrays

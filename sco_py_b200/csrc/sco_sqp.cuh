@@ -57,102 +57,192 @@ struct SqpSolver {
     return v[0] + (cg ? cg[0] : 0.0);
   }
 
-  // exact objective: quadratic terms + the non-quadratic term (prob.py:573-574)
+  // term t of the objective blocks: its block and row
+  __device__ __forceinline__ const DevObjBlock &obj_term(int t, int &r) const {
+    int b = 0;
+    while (b + 1 < S.n_ob && t >= S.ob[b + 1].t0) b++;
+    r = t - S.ob[b].t0;
+    return S.ob[b];
+  }
+  // term t's model in the term-model area (DevObjBlock)
+  __device__ __forceinline__ Sh obj_model(const DevObjBlock &B, int r) const {
+    return w.ot + (B.toff + r * (B.n_in * (B.n_in + 1) / 2 + B.n_in + 1));
+  }
+  // entry (i, j) of a term's packed upper triangle, i <= j
+  static __device__ __forceinline__ int tri(int i, int j, int nn) { return i * nn - i * (i - 1) / 2 + (j - i); }
+
+  // exact objective: quadratic terms + the non-quadratic terms, sum_t f_t (prob.py:573-574)
   __device__ double objective() {
     double v = objective_quad();
-    if (S.obj_len) v += vm_eval(field_ptr(S, S.objp, prm), 1, 0, xc, nullptr, -1, 0.0, -1, 0.0);
+    if (S.n_ob) {
+      double t[1] = {0.0};
+      for (int k = tid; k < S.n_terms; k += TEAM) {
+        int r;
+        const DevObjBlock &B = obj_term(k, r);
+        t[0] += vm_eval(field_ptr(S, B.prog, prm), B.m, r, xc, S.ob_cols + B.coff + r * B.n_in, -1, 0.0, -1, 0.0);
+      }
+      Team<TEAM>::reduce_sum(t, w.red);
+      v += t[0];
+    }
     return v;
   }
 
-  // objective of the convex model: quadratic terms + the degree-2 model of the non-quadratic term at
-  // the last convexification (prob.py:624-626)
+  // objective of the convex model: quadratic terms + the sum of the terms' degree-2 models at the last
+  // convexification (prob.py:624-626), from the assembled model (w.Hv on the pattern of P, w.gq, w.oc)
   __device__ double objective_model() {
     double v = objective_quad();
-    if (S.obj_len) {
+    if (S.n_ob) {
       double t[1] = {0.0};
       for (int k = tid; k < n; k += TEAM) {
         double acc = 0.0;
-        for (int j = 0; j < n; j++) acc += w.Hq[j * n + k] * xc[j];
+        for (int p = __ldg(S.P_cptr + k); p < __ldg(S.P_cptr + k + 1); p++) acc += w.Hv[p] * xc[__ldg(S.P_row + p)];
         t[0] += xc[k] * (0.5 * acc + w.gq[k]);
       }
       Team<TEAM>::reduce_sum(t, w.red);
-      v += t[0] + w.Hq[n * n];
+      v += t[0] + w.oc[0];
     }
     return v;
   }
 
-  // Expr.convexify degree 2 of the non-quadratic objective term at xc (expr.py:143-153):
-  // H = numeric Hessian shifted by -min(lambda_min, 0) I, A = grad - x'H, b = 0.5 x'Hx - grad.x + f.
-  // Leaves H in w.Hq (n x n), b in w.Hq[n*n], A in w.gq.  Uses w.Sm as scratch.
+  // Expr.convexify degree 2 of every non-quadratic objective term at xc, each on its own (expr.py:143-153):
+  // H_t = numeric Hessian over the term's inputs shifted by -min(lambda_min, 0) I, A_t = grad - x'H_t,
+  // b_t = 0.5 x'H_t x - grad.x + f_t.  Leaves the per-term models in w.ot, their sum on the pattern of P in w.Hv, its
+  // linear term in w.gq and its constant (sum_t b_t) in w.oc.  Every sum runs in a fixed order (no atomics).
   __device__ void convexify_objective() {
-    const double *prog = field_ptr(S, S.objp, prm);
-    const double f0 = vm_eval(prog, 1, 0, xc, nullptr, -1, 0.0, -1, 0.0);
-    for (int e = tid; e < n * n; e += TEAM) {
-      const int i = e / n, j = e % n;
-      if (i <= j) {
-        const double h = vm_fd2(prog, xc, i, j, f0);
-        w.Hq[i * n + j] = h; w.Hq[j * n + i] = h;
-        w.Sm[i * n + j] = h; w.Sm[j * n + i] = h;
-      }
+    const int NT = S.n_terms;
+    int nh = 0, ng_ = 0;  // Hessian entries (upper triangles) and gradient entries of all terms
+    for (int b = 0; b < S.n_ob; b++) {
+      nh += S.ob[b].m * (S.ob[b].n_in * (S.ob[b].n_in + 1) / 2);
+      ng_ += S.ob[b].m * S.ob[b].n_in;
     }
-    for (int j = tid; j < n; j += TEAM) {  // gradient: finite differences, or the program's own derivative
-      if (S.obj_flags & 1) { double d; vm_eval_dual(prog, 1, 0, xc, nullptr, j, &d); w.xt[j] = d; }
-      else w.xt[j] = vm_fd1(prog, 1, 0, xc, nullptr, j);
+    for (int k = tid; k < NT; k += TEAM) {
+      int r;
+      const DevObjBlock &B = obj_term(k, r);
+      obj_model(B, r)[B.n_in * (B.n_in + 1) / 2 + B.n_in] =
+          vm_eval(field_ptr(S, B.prog, prm), B.m, r, xc, S.ob_cols + B.coff + r * B.n_in, -1, 0.0, -1, 0.0);
     }
     sync();
-    if (tid < 32) {
-      // smallest eigenvalue: cyclic Jacobi on the scratch copy, warp 0.  The rotations come in the serial (p, q) order
-      // and every element is computed by the formula of a one-thread sweep; the lanes only share the n elements of the
-      // two columns, then of the two rows, a rotation touches.
-      const int lane = tid;
-      for (int sweep = 0; sweep < 50; sweep++) {
-        double off = 0.0, dg = 0.0;
-        for (int p = lane; p < n; p += 32)
-          for (int q = 0; q < n; q++) (p == q ? dg : off) += w.Sm[p * n + q] * w.Sm[p * n + q];
-        off = warp_sum(off); dg = warp_sum(dg);
-        if (off <= 1e-30 * dg || off == 0.0) break;
-        for (int p = 0; p < n - 1; p++)
-          for (int q = p + 1; q < n; q++) {
-            const double apq = w.Sm[p * n + q], app = w.Sm[p * n + p], aqq = w.Sm[q * n + q];
-            __syncwarp();
-            if (apq == 0.0) continue;
-            const double theta = (aqq - app) / (2.0 * apq);
-            const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
-            const double c = 1.0 / sqrt(t * t + 1.0), sn = t * c;
-            for (int k = lane; k < n; k += 32) {  // columns p, q
-              const double akp = w.Sm[k * n + p], akq = w.Sm[k * n + q];
-              w.Sm[k * n + p] = c * akp - sn * akq;
-              w.Sm[k * n + q] = sn * akp + c * akq;
-            }
-            __syncwarp();
-            for (int k = lane; k < n; k += 32) {  // rows p, q
-              const double apk = w.Sm[p * n + k], aqk = w.Sm[q * n + k];
-              w.Sm[p * n + k] = c * apk - sn * aqk;
-              w.Sm[q * n + k] = sn * apk + c * aqk;
-            }
-            __syncwarp();
+    for (int e = tid; e < nh + ng_; e += TEAM) {
+      int b = 0, q = e < nh ? e : e - nh;
+      const bool hess = e < nh;
+      for (;;) {  // the block of entry q
+        const int cnt = S.ob[b].m * (hess ? S.ob[b].n_in * (S.ob[b].n_in + 1) / 2 : S.ob[b].n_in);
+        if (q < cnt || b + 1 == S.n_ob) break;
+        q -= cnt;
+        b++;
+      }
+      const DevObjBlock &B = S.ob[b];
+      const int nn = B.n_in, ntri = nn * (nn + 1) / 2;
+      const int r = q / (hess ? ntri : nn);
+      q -= r * (hess ? ntri : nn);
+      const double *prog = field_ptr(S, B.prog, prm);
+      const int *cols = S.ob_cols + B.coff + r * nn;
+      const Sh h = obj_model(B, r);
+      if (hess) {
+        int i = 0;
+        while (q >= nn - i) { q -= nn - i; i++; }
+        h[tri(i, i + q, nn)] = vm_fd2(prog, B.m, r, xc, cols, i, i + q, h[ntri + nn]);
+      } else if (B.flags & 1) {  // gradient: the program's own derivative, or finite differences
+        double d;
+        vm_eval_dual(prog, B.m, r, xc, cols, q, &d);
+        h[ntri + q] = d;
+      } else {
+        h[ntri + q] = vm_fd1(prog, B.m, r, xc, cols, q);
+      }
+    }
+    sync();
+    {
+      // smallest eigenvalue of every H_t: cyclic Jacobi on a scratch copy, one warp per term.  The rotations come in the
+      // serial (p, q) order and every element is computed by the formula of a one-thread sweep; the lanes only share the
+      // elements of the two columns, then of the two rows, a rotation touches.
+      const int wid = tid >> 5, lane = tid & 31;
+      if (wid < S.nwj) {
+        const Sh A = w.jac + wid * S.n_in_max * S.n_in_max;
+        for (int k = wid; k < NT; k += S.nwj) {
+          int r;
+          const DevObjBlock &B = obj_term(k, r);
+          const int nn = B.n_in;
+          const Sh h = obj_model(B, r);
+          for (int e = lane; e < nn * nn; e += 32) {
+            const int i = e / nn, j = e % nn;
+            A[e] = h[i <= j ? tri(i, j, nn) : tri(j, i, nn)];
           }
-      }
-      if (lane == 0) {
-        double lam = w.Sm[0];
-        for (int p = 1; p < n; p++) lam = fmin(lam, w.Sm[p * n + p]);
-        w.Hq[n * n + 1] = lam;
+          __syncwarp();
+          for (int sweep = 0; sweep < 50; sweep++) {
+            double off = 0.0, dg = 0.0;
+            for (int p = lane; p < nn; p += 32)
+              for (int q = 0; q < nn; q++) (p == q ? dg : off) += A[p * nn + q] * A[p * nn + q];
+            off = warp_sum(off); dg = warp_sum(dg);
+            if (off <= 1e-30 * dg || off == 0.0) break;
+            for (int p = 0; p < nn - 1; p++)
+              for (int q = p + 1; q < nn; q++) {
+                const double apq = A[p * nn + q], app = A[p * nn + p], aqq = A[q * nn + q];
+                __syncwarp();
+                if (apq == 0.0) continue;
+                const double theta = (aqq - app) / (2.0 * apq);
+                const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
+                const double c = 1.0 / sqrt(t * t + 1.0), sn = t * c;
+                for (int k2 = lane; k2 < nn; k2 += 32) {  // columns p, q
+                  const double akp = A[k2 * nn + p], akq = A[k2 * nn + q];
+                  A[k2 * nn + p] = c * akp - sn * akq;
+                  A[k2 * nn + q] = sn * akp + c * akq;
+                }
+                __syncwarp();
+                for (int k2 = lane; k2 < nn; k2 += 32) {  // rows p, q
+                  const double apk = A[p * nn + k2], aqk = A[q * nn + k2];
+                  A[p * nn + k2] = c * apk - sn * aqk;
+                  A[q * nn + k2] = sn * apk + c * aqk;
+                }
+                __syncwarp();
+              }
+          }
+          double lam = A[0];
+          for (int p = 1; p < nn; p++) lam = fmin(lam, A[p * nn + p]);
+          if (lam < 0.0)
+            for (int j = lane; j < nn; j += 32) h[tri(j, j, nn)] -= lam;
+          __syncwarp();
+        }
       }
     }
-    sync();
-    const double lam = w.Hq[n * n + 1];
-    if (lam < 0.0)
-      for (int j = tid; j < n; j += TEAM) w.Hq[j * n + j] -= lam;
     sync();
     double t[1] = {0.0};
-    for (int k = tid; k < n; k += TEAM) {
+    for (int e = tid; e < ng_; e += TEAM) {
+      int b = 0, q = e;
+      while (b + 1 < S.n_ob && q >= S.ob[b].m * S.ob[b].n_in) { q -= S.ob[b].m * S.ob[b].n_in; b++; }
+      const DevObjBlock &B = S.ob[b];
+      const int nn = B.n_in, ntri = nn * (nn + 1) / 2, r = q / nn, k = q - r * nn;
+      const int *cols = S.ob_cols + B.coff + r * nn;
+      const Sh h = obj_model(B, r);
       double acc = 0.0;
-      for (int j = 0; j < n; j++) acc += w.Hq[j * n + k] * xc[j];  // (x'H)_k
-      w.gq[k] = w.xt[k] - acc;
-      t[0] += xc[k] * (0.5 * acc - w.xt[k]);
+      for (int j = 0; j < nn; j++) acc += h[j <= k ? tri(j, k, nn) : tri(k, j, nn)] * xc[__ldg(cols + j)];  // (x'H)_k
+      const double g = h[ntri + k], xk = xc[__ldg(cols + k)];
+      h[ntri + k] = g - acc;
+      t[0] += xk * (0.5 * acc - g);
     }
     Team<TEAM>::reduce_sum(t, w.red);
-    if (tid == 0) w.Hq[n * n] = t[0] + f0;
+    if (tid == 0) {
+      double f = 0.0;
+      for (int k = 0; k < NT; k++) {
+        int r;
+        const DevObjBlock &B = obj_term(k, r);
+        const double fk = obj_model(B, r)[B.n_in * (B.n_in + 1) / 2 + B.n_in];
+        f = k ? f + fk : fk;
+      }
+      w.oc[0] = t[0] + f;
+    }
+    // the model's sum on the pattern of P and on q: every entry from its list of term entries, in term order
+    for (int p = tid; p < S.nnz_p; p += TEAM) {
+      const int a0 = __ldg(S.hv_ptr + p), a1 = __ldg(S.hv_ptr + p + 1);
+      double v = a0 < a1 ? w.ot[__ldg(S.hv_src + a0)] : 0.0;
+      for (int a = a0 + 1; a < a1; a++) v += w.ot[__ldg(S.hv_src + a)];
+      w.Hv[p] = v;
+    }
+    for (int j = tid; j < n; j += TEAM) {
+      const int a0 = __ldg(S.gq_ptr + j), a1 = __ldg(S.gq_ptr + j + 1);
+      double v = a0 < a1 ? w.ot[__ldg(S.gq_src + a0)] : 0.0;
+      for (int a = a0 + 1; a < a1; a++) v += w.ot[__ldg(S.gq_src + a)];
+      w.gq[j] = v;
+    }
     sync();
   }
 
@@ -201,7 +291,7 @@ struct SqpSolver {
 
   // Prob.convexify at xc: fv, Jg, bb = f - J x - val ; first call freezes the sparsity masks
   __device__ void convexify(bool &mask_set) {
-    if (S.obj_len) convexify_objective();
+    if (S.n_ob) convexify_objective();
     eval_blocks<TEAM>(S, prm, xc, w.fv, Jg, w.stage);
     for (int bi = 0; bi < S.n_blocks; bi++) {
       const DevBlock &B = S.blocks[bi];
@@ -300,7 +390,7 @@ struct SqpSolver {
             for (int j = tid; j < n; j += TEAM) { w.lb[j] = w.xs[j] - delta; w.ub[j] = w.xs[j] + delta; }
             sync();
             QPArgs a;
-            a.prm = prm; a.Jg = Jg; a.pi = pi; a.kd = kd; a.wa = wa; a.use_pen = 1; a.closest = 0; a.has_hq = S.obj_len != 0;
+            a.prm = prm; a.Jg = Jg; a.pi = pi; a.kd = kd; a.wa = wa; a.use_pen = 1; a.closest = 0; a.has_hq = S.n_ob != 0;
             // warm_start 1: QPs of one trust-region loop (same J, b, weights; only the box moves); 2: every penalty QP
             // after the problem's first one
             a.warm = (st.warm_start == 1 && !first_qp) || (st.warm_start >= 2 && o.qp_solves > 1) ? 1 : 0;
@@ -324,7 +414,7 @@ struct SqpSolver {
             }
             model_sums(ms_);
             const double obj_new = objective();
-            const double model_merit = (S.obj_len ? objective_model() : obj_new) + mu * ms_[0];
+            const double model_merit = (S.n_ob ? objective_model() : obj_new) + mu * ms_[0];
             eval_blocks<TEAM>(S, prm, xc, w.fv, nullptr, w.stage);
             violation_sums(vs);
             const double new_merit = obj_new + mu * vs[0];

@@ -84,6 +84,12 @@ class Engine(object):
             if b.cols is not None:
                 cb.n_in = int(np.shape(b.cols)[1])
                 cb.cols = hold(b.cols, np.int32)
+        cs.n_obj_blocks = len(st.obj_blocks)
+        for i, ob in enumerate(st.obj_blocks):
+            co = cs.obj_blocks[i]
+            co.m, co.n_in, co.n_instr, co.flags = ob.m, ob.n_in, ob.n_instr, ob.flags
+            co.prog = _field(ob.prog)
+            co.cols = hold(ob.cols, np.int32)
         h = ctypes.c_void_p()
         _lib.check(self.lib.sco_create(ctypes.byref(cs), device, ctypes.byref(h)))
         self.h = h
@@ -174,7 +180,8 @@ class Engine(object):
         return f, J, b, obj
 
     def convexify_model(self, params, x):
-        """Degree-2 model of the non-quadratic objective term at x: (H+ [B,n,n], A [B,n], b [B])."""
+        """Convex model of the non-quadratic objective terms at x, each term convexified on its own and the models
+        summed (expr.py:143-153): (sum_t H_t+ [B,n,n], sum_t A_t [B,n], sum_t b_t [B])."""
         params, x = self._dev(params), self._dev(x)
         B = x.shape[0]
         H = torch.empty((B, self.n, self.n), dtype=torch.float64, device=self.device)

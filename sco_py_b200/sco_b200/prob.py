@@ -109,7 +109,7 @@ class Prob(object):
     def convexify(self):
         """Affine models of the nonlinear constraints at the current value (prob.py:522-544)."""
         s = self._dev()
-        if s["st"].obj_prog_len:
+        if s["st"].obj_prog_len or s["st"].obj_blocks:
             raise NotImplementedError("the step-by-step methods do not carry the degree-2 model of a non-quadratic "
                                       "objective between calls; use Solver.solve (one kernel does the whole SQP)")
         if s["st"].m_nl == 0:

@@ -29,6 +29,8 @@ CNT_EQ = 1         # EqExpr   -> abs penalty,   2 slacks per row  (expr.py:314-3
 
 MAX_BLOCKS = 16
 MAX_GROUPS = 8
+MAX_OBJ_BLOCKS = 4
+MAX_OBJ_INPUTS = 64
 
 
 @dataclass
@@ -56,6 +58,18 @@ class Block:
 
 
 @dataclass
+class ObjBlock:
+    """Non-quadratic objective terms of one input count and derivative mode (include/sco_b200.h
+    sco_obj_block_desc): one scalar program row per term, term r reads x[cols[r]]."""
+    prog: Field                      # m row offsets, then 2 * n_instr (like a VM constraint block)
+    m: int
+    n_in: int
+    n_instr: int
+    flags: int                       # bit 0: forward-mode gradient (SymExpr analytic=True)
+    cols: np.ndarray                 # (m, n_in) int32
+
+
+@dataclass
 class Structure:
     n: int
     stride: int                      # doubles per problem block
@@ -78,6 +92,7 @@ class Structure:
     qa: Field = field(default_factory=Field)        # n: summed A rows of AffExpr objective terms (quirk C-4 weight in the QP)
     lb0: Field = field(default_factory=Field)       # n: user lower bounds of the scalar variables (closest-point QP)
     ub0: Field = field(default_factory=Field)       # n: user upper bounds
+    obj_blocks: List[ObjBlock] = field(default_factory=list)  # objective terms bound to Variables (or obj_prog)
 
     @property
     def m_nl(self):
