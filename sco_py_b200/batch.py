@@ -31,8 +31,7 @@ class Compiled(object):
         self.c = 0.0
         self.lin_A = self.lin_l = self.lin_u = None
         self.blocks = []         # device blocks: (family expr, cnt_type, val[m], group ids, column map [m, n_in] or None)
-        self.obj_prog = None     # SymExpr of a non-quadratic objective over all variables in QP order (one term)
-        self.obj_blocks = []     # every other case: (PackedRows of scalar SymExpr terms, column map [m, n_in])
+        self.obj_blocks = []     # non-quadratic objective: (PackedRows of scalar SymExpr terms, column map [m, n_in])
         self.gids = []
 
 
@@ -159,22 +158,18 @@ def compile_problem(prob):
                                          "(n_in x n_in Hessian model per term in shared memory, n_in^2 / 2 program "
                                          "evaluations per convexification)" % (cols.size, MAX_OBJ_INPUTS))
             terms.append((e, cols))
-        e, cols = terms[0]
-        if len(terms) == 1 and cols.size == n and np.array_equal(cols, np.arange(n)):
-            cp.obj_prog = e  # one term over every variable in QP order: the structure of earlier versions
-        else:
-            packs = {}  # terms of one input count and derivative mode -> index into cp.obj_blocks
-            for e, cols in terms:
-                key = (e.n, bool(e.analytic))
-                if key not in packs:
-                    packs[key] = len(cp.obj_blocks)
-                    cp.obj_blocks.append(([], []))
-                cp.obj_blocks[packs[key]][0].append(e)
-                cp.obj_blocks[packs[key]][1].append(cols)
-            if len(cp.obj_blocks) > MAX_OBJ_BLOCKS:
-                raise UnsupportedProblem("%d objective blocks (scalar SymExpr terms of one input count and derivative "
-                                         "mode share one): the limit is %d" % (len(cp.obj_blocks), MAX_OBJ_BLOCKS))
-            cp.obj_blocks = [(PackedRows(parts), np.vstack(maps)) for parts, maps in cp.obj_blocks]
+        packs = {}  # terms of one input count and derivative mode -> index into cp.obj_blocks
+        for e, cols in terms:
+            key = (e.n, bool(e.analytic))
+            if key not in packs:
+                packs[key] = len(cp.obj_blocks)
+                cp.obj_blocks.append(([], []))
+            cp.obj_blocks[packs[key]][0].append(e)
+            cp.obj_blocks[packs[key]][1].append(cols)
+        if len(cp.obj_blocks) > MAX_OBJ_BLOCKS:
+            raise UnsupportedProblem("%d objective blocks (scalar SymExpr terms of one input count and derivative "
+                                     "mode share one): the limit is %d" % (len(cp.obj_blocks), MAX_OBJ_BLOCKS))
+        cp.obj_blocks = [(PackedRows(parts), np.vstack(maps)) for parts, maps in cp.obj_blocks]
     # ---- linear constraints
     rows_A, rows_l, rows_u = [], [], []
     for b, kind in prob._lin_cnt_exprs:
@@ -257,14 +252,7 @@ def group_key(cp):
             None if cp.lin_A is None else (cp.lin_A.shape, cp.lin_A.tobytes()), tuple(cp.gids),
             tuple((b[0].family, b[0].m, b[1], tuple(b[0].ipar), tuple(b[3])) +
                   (() if b[4] is None else (b[4].shape, b[4].tobytes())) for b in cp.blocks),
-            None if cp.obj_prog is None else (cp.obj_prog.n_instr, cp.obj_prog.analytic)) + _obj_key(cp)
-
-
-def _obj_key(cp):
-    """Identity of the objective blocks (empty without any, so that other keys stay as they were)."""
-    if not cp.obj_blocks:
-        return ()
-    return (tuple((pk.m, pk.n, pk.n_instr, int(pk.ipar[3]), cols.tobytes()) for pk, cols in cp.obj_blocks),)
+            tuple((pk.m, pk.n, pk.n_instr, int(pk.ipar[3]), cols.tobytes()) for pk, cols in cp.obj_blocks))
 
 
 def compile_batch(probs, compiled=None):
@@ -274,18 +262,9 @@ def compile_batch(probs, compiled=None):
     c0 = cps[0]
     n = c0.x0.size
     B = len(cps)
+    key0 = group_key(c0)
     for i, c in enumerate(cps[1:], 1):
-        same = (c.x0.size == n and len(c.blocks) == len(c0.blocks) and c.gids == c0.gids and
-                (c.lin_A is None) == (c0.lin_A is None) and
-                (c.lin_A is None or (c.lin_A.shape == c0.lin_A.shape and np.array_equal(c.lin_A, c0.lin_A))) and
-                all(a[0].family == b[0].family and a[0].m == b[0].m and a[1] == b[1] and a[3] == b[3] and
-                    list(a[0].ipar) == list(b[0].ipar) and (a[4] is None) == (b[4] is None) and
-                    (a[4] is None or np.array_equal(a[4], b[4])) for a, b in zip(c.blocks, c0.blocks)) and
-                (c.obj_prog is None) == (c0.obj_prog is None) and (c.qa is None) == (c0.qa is None) and
-                (c.lb0 is None) == (c0.lb0 is None) and
-                (c.obj_prog is None or (c.obj_prog.n_instr == c0.obj_prog.n_instr and c.obj_prog.analytic == c0.obj_prog.analytic)) and
-                _obj_key(c) == _obj_key(c0))
-        if not same:
+        if group_key(c) != key0:
             raise UnsupportedProblem("problem %d of the batch does not share the structure of problem 0" % i)
     shared_parts, shared_off = [], 0
 
@@ -334,14 +313,6 @@ def compile_batch(probs, compiled=None):
         fills.append((lf, lambda c: c.lin_l))
         fills.append((uf, lambda c: c.lin_u))
         kw.update(m_lin=m_lin, lin_rowptr=rp, lin_col=ci, lin_val=cv, lin_l=lf, lin_u=uf)
-    if c0.obj_prog is not None:
-        p0 = c0.obj_prog.params()
-        if B > 1 and all(np.array_equal(c.obj_prog.params(), p0) for c in cps[1:]):
-            of = shared_field(p0)
-        else:
-            of = own_field(p0.size)
-            fills.append((of, lambda c: c.obj_prog.params()))
-        kw.update(obj_prog=of, obj_prog_len=c0.obj_prog.n_instr, obj_prog_flags=int(c0.obj_prog.analytic))
     obj_blocks = []
     for oi, (pk, cols) in enumerate(c0.obj_blocks):
         p0 = pk.params()
@@ -352,6 +323,10 @@ def compile_batch(probs, compiled=None):
             fills.append((of, lambda c, oi=oi: c.obj_blocks[oi][0].params()))
         obj_blocks.append(ObjBlock(of, pk.m, pk.n, pk.n_instr, int(pk.ipar[3]),
                                    np.ascontiguousarray(cols, dtype=np.int32)))
+    if len(obj_blocks) == 1 and obj_blocks[0].m == 1 and np.array_equal(obj_blocks[0].cols[0], np.arange(n)):
+        # one term over every variable in QP order: the obj_prog structure of earlier versions
+        ob = obj_blocks.pop()
+        kw.update(obj_prog=ob.prog, obj_prog_len=ob.n_instr, obj_prog_flags=ob.flags)
     blocks = []
     for bi, (fam, ctype, val, gids, cols) in enumerate(c0.blocks):
         p0 = fam.params()

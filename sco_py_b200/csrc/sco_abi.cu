@@ -6,6 +6,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <vector>
 
 #include "sco_b200.h"
@@ -189,125 +190,173 @@ static DevSettings to_dev(const sco_settings *s) {
   return d;
 }
 
-extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle **out) {
-  if (!desc || !out) return fail(SCO_ERR_ARG, "null argument");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-    return fail(SCO_ERR_CUDA, "no CUDA device: the engine has no CPU fallback");
-  if (device < 0 || device >= ndev) return fail(SCO_ERR_ARG, "device %d out of range", device);
+// ------------------------------------------------------------------------------------ structure compiler
+// sco_create runs in stages: check_desc refuses a bad descriptor, build_index builds the index arrays on the host,
+// choose_paths picks the ADMM loop, team and layout, setup_device uploads and configures.  Nothing is allocated on
+// the device before the last stage.
+
+static bool has_obj_prog(const sco_structure_desc *desc) { return desc->obj_prog_len > 0 && desc->obj_prog.off >= 0; }
+
+// A column map: m rows of n_in indices in [0, n), none repeated within a row.  The messages name row r of block blk
+// "<what> <blk> <row> <r>": "block 2 row 5", "objective block 0 term 3".
+static int check_map(const int32_t *cols, int m, int n_in, int n, const char *what, int blk, const char *row) {
+  for (int r = 0; r < m; r++) {
+    const int32_t *c = cols + (size_t)r * n_in;
+    for (int i = 0; i < n_in; i++) {
+      if (c[i] < 0 || c[i] >= n) return fail(SCO_ERR_ARG, "%s %d %s %d: column %d outside [0, %d)", what, blk, row, r, c[i], n);
+      if (std::find(c, c + i, c[i]) != c + i) return fail(SCO_ERR_ARG, "%s %d %s %d: column %d repeats", what, blk, row, r, c[i]);
+    }
+  }
+  return 0;
+}
+
+// Every refusal of a descriptor, before anything is built or allocated.
+static int check_desc(const sco_structure_desc *desc) {
   if (desc->n <= 0 || desc->n_blocks < 0 || desc->n_blocks > SCO_MAX_BLOCKS)
     return fail(SCO_ERR_ARG, "bad n / n_blocks");
   // n_groups = 0: no constraint belongs to a group -- the reference then skips the per-group test (solver.py:209)
   if (desc->n_groups < 0 || desc->n_groups > SCO_MAX_GROUPS) return fail(SCO_ERR_ARG, "bad n_groups");
   if (desc->m_lin < 0 || desc->stride <= 0 || desc->shared_len < 0) return fail(SCO_ERR_ARG, "negative m_lin / stride / shared_len");
   if (desc->shared_len > 0 && !desc->shared) return fail(SCO_ERR_ARG, "shared_len > 0 but shared is null");
-  {
-    // every field must lie inside the block it lives in (out-of-range offsets would be device reads out of bounds)
-    const long long n_ = desc->n;
-    auto field_ok = [&](const sco_field &f, long long len) {
-      if (f.off < 0) return true;
-      const long long lim = f.shared ? (long long)desc->shared_len : (long long)desc->stride;
-      return f.off + len <= lim;
-    };
-    bool okf = field_ok(desc->Q, n_ * n_) && field_ok(desc->q, n_) && field_ok(desc->c, 1) &&
-               field_ok(desc->lin_l, desc->m_lin) && field_ok(desc->lin_u, desc->m_lin) && field_ok(desc->qa, n_) &&
-               field_ok(desc->lb0, n_) && field_ok(desc->ub0, n_) &&
-               (desc->obj_prog_len <= 0 || field_ok(desc->obj_prog, 1 + 2LL * desc->obj_prog_len));
-    if (desc->n_obj_blocks < 0 || desc->n_obj_blocks > SCO_MAX_OBJ_BLOCKS)
-      return fail(SCO_ERR_ARG, "n_obj_blocks = %d outside [0, %d]", desc->n_obj_blocks, SCO_MAX_OBJ_BLOCKS);
-    if (desc->obj_prog_len > 0 && desc->n_obj_blocks > 0)
-      return fail(SCO_ERR_ARG, "obj_prog and objective blocks are both set: a structure has one or the other");
-    for (int oi = 0; oi < desc->n_obj_blocks && okf; oi++) {
-      const sco_obj_block_desc &o = desc->obj_blocks[oi];
-      if (o.m <= 0 || o.n_instr <= 0) return fail(SCO_ERR_ARG, "objective block %d: m and n_instr must be positive", oi);
-      if (o.n_in < 1 || o.n_in > 64)
-        return fail(SCO_ERR_ARG, "objective block %d: n_in = %d outside [1, 64] (inputs per term)", oi, o.n_in);
-      if (!o.cols) return fail(SCO_ERR_ARG, "objective block %d: cols is null", oi);
-      for (int r = 0; r < o.m; r++) {
-        const int32_t *c = o.cols + (size_t)r * o.n_in;
-        for (int i = 0; i < o.n_in; i++) {
-          if (c[i] < 0 || c[i] >= n_)
-            return fail(SCO_ERR_ARG, "objective block %d term %d: column %d outside [0, %d)", oi, r, c[i], (int)n_);
-          for (int k = 0; k < i; k++)
-            if (c[k] == c[i]) return fail(SCO_ERR_ARG, "objective block %d term %d: column %d repeats", oi, r, c[i]);
-        }
-      }
-      if (o.prog.off < 0) return fail(SCO_ERR_ARG, "objective block %d: the program is missing", oi);
-      if (!field_ok(o.prog, o.m + 2LL * o.n_instr))
-        return fail(SCO_ERR_ARG, "objective block %d: the program field lies outside its parameter block", oi);
-    }
-    for (int bi = 0; bi < desc->n_blocks && okf; bi++) {
-      const sco_block_desc &b = desc->blocks[bi];
-      if (b.m <= 0) return fail(SCO_ERR_ARG, "block %d: m must be positive", bi);
-      if (desc->n_groups < 32 && (b.group_mask >> desc->n_groups) != 0)
-        return fail(SCO_ERR_ARG, "block %d: group_mask names a group >= n_groups", bi);
-      if (b.cols) {
-        const int want = b.family == SCO_FAM_CIRCLE2D ? 2 : b.family == SCO_FAM_FK7 ? 7 : b.n_in;
-        if (b.n_in <= 0 || b.n_in > n_ || b.n_in != want)
-          return fail(SCO_ERR_ARG, "block %d: n_in = %d is wrong for family %d (CIRCLE2D 2, FK7 7, else 1..n)", bi, b.n_in,
-                      b.family);
-        if (b.family == SCO_FAM_FK7 && b.m % 3 != 0) return fail(SCO_ERR_ARG, "block %d: FK7 with a map needs m %% 3 == 0", bi);
-        for (int r = 0; r < b.m; r++) {
-          const int32_t *c = b.cols + (size_t)r * b.n_in;
-          for (int i = 0; i < b.n_in; i++) {
-            if (c[i] < 0 || c[i] >= n_) return fail(SCO_ERR_ARG, "block %d row %d: column %d outside [0, %d)", bi, r, c[i], (int)n_);
-            for (int k = 0; k < i; k++)
-              if (c[k] == c[i]) return fail(SCO_ERR_ARG, "block %d row %d: column %d repeats", bi, r, c[i]);
-            if (b.family == SCO_FAM_FK7 && r % 3 != 0 && c[i] != c[i - (r % 3) * 7])
-              return fail(SCO_ERR_ARG, "block %d: rows of FK7 instance %d have different maps", bi, r / 3);
-          }
-        }
-      }
-      const long long nb = b.cols ? b.n_in : n_;  // inputs of a row
-      long long plen = 0;
-      if (b.family == SCO_FAM_QUADFORM) plen = (long long)b.m * (nb * (nb + 1) / 2 + nb);
-      else if (b.family == SCO_FAM_CIRCLE2D) plen = 3LL * b.ipar[1];
-      else if (b.family == SCO_FAM_FK7) plen = 30;
-      else if (b.family == SCO_FAM_VM) plen = b.m + 2LL * b.ipar[2];
-      if (b.par.off < 0) return fail(SCO_ERR_ARG, "block %d: parameters are missing", bi);
-      okf = field_ok(b.par, plen) && field_ok(b.val, b.m);
-    }
-    if (!okf) return fail(SCO_ERR_ARG, "a field lies outside its parameter block (offset + length > stride / shared_len)");
-    if (desc->m_lin > 0 && (desc->lin_l.off < 0 || desc->lin_u.off < 0)) return fail(SCO_ERR_ARG, "m_lin > 0 needs lin_l and lin_u");
+  // every field must lie inside the block it lives in (out-of-range offsets would be device reads out of bounds)
+  const int n = desc->n;
+  auto field_ok = [&](const sco_field &f, long long len) {
+    if (f.off < 0) return true;
+    const long long lim = f.shared ? (long long)desc->shared_len : (long long)desc->stride;
+    return f.off + len <= lim;
+  };
+  static const char outside[] = "a field lies outside its parameter block (offset + length > stride / shared_len)";
+  if (desc->n_obj_blocks < 0 || desc->n_obj_blocks > SCO_MAX_OBJ_BLOCKS)
+    return fail(SCO_ERR_ARG, "n_obj_blocks = %d outside [0, %d]", desc->n_obj_blocks, SCO_MAX_OBJ_BLOCKS);
+  if (desc->obj_prog_len > 0 && desc->n_obj_blocks > 0)
+    return fail(SCO_ERR_ARG, "obj_prog and objective blocks are both set: a structure has one or the other");
+  if (!(field_ok(desc->Q, (long long)n * n) && field_ok(desc->q, n) && field_ok(desc->c, 1) &&
+        field_ok(desc->lin_l, desc->m_lin) && field_ok(desc->lin_u, desc->m_lin) && field_ok(desc->qa, n) &&
+        field_ok(desc->lb0, n) && field_ok(desc->ub0, n) &&
+        (desc->obj_prog_len <= 0 || field_ok(desc->obj_prog, 1 + 2LL * desc->obj_prog_len))))
+    return fail(SCO_ERR_ARG, "%s", outside);
+  for (int oi = 0; oi < desc->n_obj_blocks; oi++) {
+    const sco_obj_block_desc &o = desc->obj_blocks[oi];
+    if (o.m <= 0 || o.n_instr <= 0) return fail(SCO_ERR_ARG, "objective block %d: m and n_instr must be positive", oi);
+    if (o.n_in < 1 || o.n_in > 64)
+      return fail(SCO_ERR_ARG, "objective block %d: n_in = %d outside [1, 64] (inputs per term)", oi, o.n_in);
+    if (!o.cols) return fail(SCO_ERR_ARG, "objective block %d: cols is null", oi);
+    if (int rc = check_map(o.cols, o.m, o.n_in, n, "objective block", oi, "term")) return rc;
+    if (o.prog.off < 0) return fail(SCO_ERR_ARG, "objective block %d: the program is missing", oi);
+    if (!field_ok(o.prog, o.m + 2LL * o.n_instr))
+      return fail(SCO_ERR_ARG, "objective block %d: the program field lies outside its parameter block", oi);
   }
-  CUDA_TRY(cudaSetDevice(device));
-  cudaDeviceProp prop;
-  CUDA_TRY(cudaGetDeviceProperties(&prop, device));
-  if (prop.major != 10) return fail(SCO_ERR_CUDA, "device is sm_%d%d; this library is built for sm_100a only", prop.major, prop.minor);
+  for (int bi = 0; bi < desc->n_blocks; bi++) {
+    const sco_block_desc &b = desc->blocks[bi];
+    if (b.m <= 0) return fail(SCO_ERR_ARG, "block %d: m must be positive", bi);
+    if (desc->n_groups < 32 && (b.group_mask >> desc->n_groups) != 0)
+      return fail(SCO_ERR_ARG, "block %d: group_mask names a group >= n_groups", bi);
+    const bool mapped = b.cols != nullptr;
+    if (mapped) {
+      const int want = b.family == SCO_FAM_CIRCLE2D ? 2 : b.family == SCO_FAM_FK7 ? 7 : b.n_in;
+      if (b.n_in <= 0 || b.n_in > n || b.n_in != want)
+        return fail(SCO_ERR_ARG, "block %d: n_in = %d is wrong for family %d (CIRCLE2D 2, FK7 7, else 1..n)", bi, b.n_in, b.family);
+      if (b.family == SCO_FAM_FK7 && b.m % 3 != 0) return fail(SCO_ERR_ARG, "block %d: FK7 with a map needs m %% 3 == 0", bi);
+      if (int rc = check_map(b.cols, b.m, b.n_in, n, "block", bi, "row")) return rc;
+      for (int r = 0; b.family == SCO_FAM_FK7 && r < b.m; r++)  // the three rows of an instance are one position
+        if (r % 3 != 0 && memcmp(b.cols + (size_t)r * 7, b.cols + (size_t)(r - r % 3) * 7, 7 * sizeof(int32_t)) != 0)
+          return fail(SCO_ERR_ARG, "block %d: rows of FK7 instance %d have different maps", bi, r / 3);
+    }
+    const long long nb = mapped ? b.n_in : n;  // inputs of a row
+    long long plen = 0;
+    if (b.family == SCO_FAM_QUADFORM) plen = (long long)b.m * (nb * (nb + 1) / 2 + nb);
+    else if (b.family == SCO_FAM_CIRCLE2D) plen = 3LL * b.ipar[1];
+    else if (b.family == SCO_FAM_FK7) plen = 30;
+    else if (b.family == SCO_FAM_VM) plen = b.m + 2LL * b.ipar[2];
+    else return fail(SCO_ERR_UNSUPPORTED, "unknown constraint family %d", b.family);
+    if (b.par.off < 0) return fail(SCO_ERR_ARG, "block %d: parameters are missing", bi);
+    if (!field_ok(b.par, plen) || !field_ok(b.val, b.m)) return fail(SCO_ERR_ARG, "%s", outside);
+    if (b.family == SCO_FAM_CIRCLE2D && (b.ipar[1] <= 0 || b.ipar[0] * b.ipar[1] != b.m || (!mapped && 2 * b.ipar[0] > n)))
+      return fail(SCO_ERR_ARG, "CIRCLE2D: m != T*K or 2T > n");
+    if (b.family == SCO_FAM_FK7 && ((!mapped && b.m != 3) || n < 7))
+      return fail(SCO_ERR_ARG, "FK7: m must be 3 (without a map) and n >= 7");
+    if (b.family == SCO_FAM_VM && (b.ipar[0] != nb || b.ipar[1] != b.m || b.ipar[2] <= 0))
+      return fail(SCO_ERR_ARG, "VM: ipar must be {n (n_in with a map), m, instructions}");
+  }
+  if (desc->m_lin > 0 && (desc->lin_l.off < 0 || desc->lin_u.off < 0)) return fail(SCO_ERR_ARG, "m_lin > 0 needs lin_l and lin_u");
+  if (has_obj_prog(desc) && n > 64) return fail(SCO_ERR_UNSUPPORTED, "non-quadratic objectives are limited to 64 variables");
+  if (desc->m_lin > 0) {
+    if (!desc->lin_rowptr || !desc->lin_col || !desc->lin_val) return fail(SCO_ERR_ARG, "m_lin > 0 but CSR arrays are null");
+    for (int r = 0; r < desc->m_lin; r++)
+      for (int p = desc->lin_rowptr[r]; p < desc->lin_rowptr[r + 1]; p++)
+        if (desc->lin_col[p] < 0 || desc->lin_col[p] >= n) return fail(SCO_ERR_ARG, "linear row column out of range");
+  }
+  return 0;
+}
 
-  sco_handle *h = new sco_handle();
-  h->device = device;
-  h->sm_count = prop.multiProcessorCount;
-  DevStruct &S = h->S;
+// What sco_create hands to the device, built on the host: DevStruct's sizes and tables, the index arrays, the team
+// and the shared memory per problem.  The device sums along pc_*, lin_c*, hv_src and gq_src in list order, so the
+// order of every list is part of the results: rows ascending, and within a row its stored entries ascending.
+struct HostStruct {
+  DevStruct S;  // device pointers unset
+  std::vector<int> row_goff, row_soff, row_w, row_eq, row_gmask, jcol, pc_ptr, pc_e, pc_r;  // penalty rows
+  std::vector<int> lrp, lcol, lin_w, lcptr, lcentry, lcrow;                                 // linear rows
+  std::vector<double> lval, shared;
+  std::vector<int> ob_cols, P_cptr, P_row, hv_ptr, hv_src, gq_ptr, gq_src;                  // objective
+  bool any_map = false;
+  int team = 0; size_t smem_bytes = 0;  // choose_paths
+};
+
+// lists[i] -> ptr (ptr[i + 1] - ptr[i] = lists[i].size()) and src, the lists concatenated in order
+static void flatten(const std::vector<std::vector<int>> &lists, std::vector<int> &ptr, std::vector<int> &src) {
+  ptr.assign(lists.size() + 1, 0);
+  for (size_t i = 0; i < lists.size(); i++) {
+    ptr[i + 1] = ptr[i] + (int)lists[i].size();
+    src.insert(src.end(), lists[i].begin(), lists[i].end());
+  }
+}
+
+// CSC over the n user variables of a row pattern whose row r holds w[r] entries, entry e0[r] + k in column
+// col[c0[r] + k]: per column its (entry, row) pairs, rows ascending and a row's entries ascending
+static void to_csc(int n, const std::vector<int> &col, const std::vector<int> &c0, const std::vector<int> &e0,
+                   const std::vector<int> &w, std::vector<int> &ptr, std::vector<int> &ent, std::vector<int> &row) {
+  std::vector<std::vector<int>> ents(n), rows(n);
+  for (size_t r = 0; r < w.size(); r++)
+    for (int k = 0; k < w[r]; k++) {
+      ents[col[c0[r] + k]].push_back(e0[r] + k);
+      rows[col[c0[r] + k]].push_back((int)r);
+    }
+  flatten(ents, ptr, ent);
+  flatten(rows, ptr, row);
+}
+
+// max - min of the w columns col[c0 ..]: the band a row adds to S = P + A'RA (0 for an empty row)
+static int col_span(const std::vector<int> &col, int c0, int w) {
+  if (w <= 0) return 0;
+  const auto mm = std::minmax_element(col.begin() + c0, col.begin() + c0 + w);
+  return *mm.second - *mm.first;
+}
+
+static void build_index(const sco_structure_desc *desc, HostStruct &ix) {
+  DevStruct &S = ix.S;
   memset(&S, 0, sizeof(S));
   const int n = desc->n;
-  S.n = n;
-  S.m_lin = desc->m_lin;
-  S.n_blocks = desc->n_blocks;
-  S.n_groups = desc->n_groups;
-  S.stride = desc->stride;
+  S.n = n; S.m_lin = desc->m_lin; S.n_blocks = desc->n_blocks; S.n_groups = desc->n_groups; S.stride = desc->stride;
   S.Q = cvt(desc->Q); S.q = cvt(desc->q); S.c = cvt(desc->c);
   S.lin_l = cvt(desc->lin_l); S.lin_u = cvt(desc->lin_u);
   S.qa = cvt(desc->qa); S.lb0 = cvt(desc->lb0); S.ub0 = cvt(desc->ub0);
   // objective terms: the one-term obj_prog becomes a block of one term over all n variables in QP order
-  const bool legacy_obj = desc->obj_prog_len > 0 && desc->obj_prog.off >= 0;
-  if (legacy_obj && n > 64) { delete h; return fail(SCO_ERR_UNSUPPORTED, "non-quadratic objectives are limited to 64 variables"); }
-  std::vector<int> ob_cols;
-  S.n_ob = legacy_obj ? 1 : desc->n_obj_blocks;
-  for (int oi = 0, t0 = 0, toff = 0; oi < S.n_ob; oi++) {
+  std::vector<int32_t> all(n);
+  for (int j = 0; j < n; j++) all[j] = j;
+  const sco_obj_block_desc prog = {1, n, desc->obj_prog_len, desc->obj_prog_flags, desc->obj_prog, all.data()};
+  std::vector<int> pidx((size_t)n * n, -1);  // (i, j) -> entry of the pattern of P (below)
+  S.n_ob = has_obj_prog(desc) ? 1 : desc->n_obj_blocks;
+  for (int oi = 0, toff = 0; oi < S.n_ob; oi++) {
+    const sco_obj_block_desc &o = has_obj_prog(desc) ? prog : desc->obj_blocks[oi];
     DevObjBlock &d = S.ob[oi];
-    if (legacy_obj) {
-      d.m = 1; d.n_in = n; d.flags = desc->obj_prog_flags; d.prog = cvt(desc->obj_prog);
-      for (int j = 0; j < n; j++) ob_cols.push_back(j);
-    } else {
-      const sco_obj_block_desc &o = desc->obj_blocks[oi];
-      d.m = o.m; d.n_in = o.n_in; d.flags = o.flags; d.prog = cvt(o.prog);
-      ob_cols.insert(ob_cols.end(), o.cols, o.cols + (size_t)o.m * o.n_in);
-    }
-    d.t0 = t0; d.toff = toff; d.coff = (int)ob_cols.size() - d.m * d.n_in;
-    t0 += d.m;
+    d.m = o.m; d.n_in = o.n_in; d.flags = o.flags; d.prog = cvt(o.prog);
+    d.t0 = S.n_terms; d.toff = toff; d.coff = (int)ix.ob_cols.size();
+    ix.ob_cols.insert(ix.ob_cols.end(), o.cols, o.cols + (size_t)o.m * o.n_in);
+    for (int r = 0; r < o.m; r++)  // the term's n_in x n_in block is in the pattern of P
+      for (int a = 0; a < o.n_in; a++)
+        for (int b = 0; b < o.n_in; b++) pidx[(size_t)o.cols[r * o.n_in + a] * n + o.cols[r * o.n_in + b]] = 0;
+    S.n_terms += d.m;
     toff += d.m * (d.n_in * (d.n_in + 1) / 2 + d.n_in + 1);
-    S.n_terms = t0;
     S.n_in_max = std::max(S.n_in_max, d.n_in);
   }
   for (int g = 0; g < desc->n_groups; g++) {
@@ -318,10 +367,7 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
     S.overlap[g] = bits;
   }
   // ---- penalty rows
-  std::vector<int> row_goff, row_soff, row_w, row_eq, row_gmask, jcol;
-  int m_nl = 0, jnnz = 0, sj = 0, n_slack = 0, any_eq = 0, max_stage = 0;
-  int max_jw = 1;
-  bool any_map = false;
+  int m_nl = 0, jnnz = 0, sj = 0, n_slack = 0, max_stage = 0, max_jw = 1;
   for (int bi = 0; bi < desc->n_blocks; bi++) {
     const sco_block_desc &b = desc->blocks[bi];
     DevBlock &d = S.blocks[bi];
@@ -331,191 +377,117 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
     d.par = cvt(b.par); d.val = cvt(b.val);
     const bool mapped = b.cols != nullptr;
     const int nb = mapped ? b.n_in : n;  // inputs of a row
-    any_map = any_map || mapped;
+    ix.any_map = ix.any_map || mapped;
     d.n_in = mapped ? b.n_in : 0;
-    int jw = 0;
-    if (b.family == SCO_FAM_QUADFORM) {
-      jw = nb;
-      // a map's inputs are gathered into the staging buffer behind P_r
+    const int jw = b.family == SCO_FAM_CIRCLE2D ? 2 : b.family == SCO_FAM_FK7 ? 7 : nb;  // QUADFORM, VM: every input
+    if (b.family == SCO_FAM_QUADFORM)  // a map's inputs are gathered into the staging buffer behind P_r
       max_stage = std::max(max_stage, nb * (nb + 1) / 2 + (mapped ? nb : 0));
-    } else if (b.family == SCO_FAM_CIRCLE2D) {
-      jw = 2;
-      if (b.ipar[1] <= 0 || b.ipar[0] * b.ipar[1] != b.m || (!mapped && 2 * b.ipar[0] > n)) { sco_destroy(h); return fail(SCO_ERR_ARG, "CIRCLE2D: m != T*K or 2T > n"); }
-    } else if (b.family == SCO_FAM_FK7) {
-      jw = 7;
-      if (mapped) max_stage = std::max(max_stage, 106);  // 98 doubles of finite differences + the gathered joints
-      if ((!mapped && b.m != 3) || n < 7) { sco_destroy(h); return fail(SCO_ERR_ARG, "FK7: m must be 3 (without a map) and n >= 7"); }
-    } else if (b.family == SCO_FAM_VM) {
-      jw = nb;
-      if (b.ipar[0] != nb || b.ipar[1] != b.m || b.ipar[2] <= 0) { sco_destroy(h); return fail(SCO_ERR_ARG, "VM: ipar must be {n (n_in with a map), m, instructions}"); }
-    } else { sco_destroy(h); return fail(SCO_ERR_UNSUPPORTED, "unknown constraint family %d", b.family); }
+    if (b.family == SCO_FAM_FK7 && mapped)  // 98 doubles of finite differences + the gathered joints
+      max_stage = std::max(max_stage, 106);
     max_jw = std::max(max_jw, jw);
     d.jw = jw;
     const int ldj = (jw % 2 == 0) ? jw + 1 : jw;
     for (int r = 0; r < b.m; r++) {
-      row_goff.push_back(jnnz + r * jw);
-      row_soff.push_back(sj + r * ldj);
-      row_w.push_back(jw);
-      row_eq.push_back(b.cnt_type == SCO_CNT_EQ ? 1 : 0);
-      row_gmask.push_back(b.group_mask);
+      ix.row_goff.push_back(jnnz + r * jw);
+      ix.row_soff.push_back(sj + r * ldj);
+      ix.row_w.push_back(jw);
+      ix.row_eq.push_back(b.cnt_type == SCO_CNT_EQ ? 1 : 0);
+      ix.row_gmask.push_back(b.group_mask);
       for (int k = 0; k < jw; k++) {
         int col = 0;
         if (mapped) col = b.cols[(size_t)r * b.n_in + k];
         else if (b.family == SCO_FAM_QUADFORM || b.family == SCO_FAM_VM) col = k;
         else if (b.family == SCO_FAM_CIRCLE2D) col = 2 * (r / b.ipar[1]) + k;
         else col = n - 7 + k;
-        jcol.push_back(col);
+        ix.jcol.push_back(col);
       }
     }
-    if (b.cnt_type == SCO_CNT_EQ) any_eq = 1;
     n_slack += b.m * (b.cnt_type == SCO_CNT_EQ ? 2 : 1);
     m_nl += b.m;
     jnnz += b.m * jw;
     sj += b.m * ldj;
   }
   S.m_nl = m_nl; S.jnnz = jnnz; S.sjnnz = sj; S.n_slack = n_slack; S.n_q = n + n_slack;
-  S.nsl = any_eq ? 2 : 1;
+  S.nsl = n_slack > m_nl ? 2 : 1;  // an equality row has two slacks
   S.stage_per_warp = (max_stage + 1) & ~1;
   S.mw = (max_jw + 31) / 32;
-  // CSC over user variables of the stored Jacobian pattern
-  std::vector<int> pc_ptr(n + 1, 0), pc_e, pc_r;
-  {
-    std::vector<std::vector<std::pair<int, int>>> cols(n);
-    for (int i = 0; i < m_nl; i++)
-      for (int k = 0; k < row_w[i]; k++) cols[jcol[row_goff[i] + k]].push_back({row_soff[i] + k, i});
-    for (int j = 0; j < n; j++) {
-      pc_ptr[j + 1] = pc_ptr[j] + (int)cols[j].size();
-      for (auto &pr : cols[j]) { pc_e.push_back(pr.first); pc_r.push_back(pr.second); }
-    }
-  }
-  // linear rows
-  std::vector<int> lrp(desc->m_lin + 1, 0), lcol, lcptr(n + 1, 0), lcentry, lcrow;
-  std::vector<double> lval;
-  if (desc->m_lin > 0) {
-    if (!desc->lin_rowptr || !desc->lin_col || !desc->lin_val) { sco_destroy(h); return fail(SCO_ERR_ARG, "m_lin > 0 but CSR arrays are null"); }
-    lrp.assign(desc->lin_rowptr, desc->lin_rowptr + desc->m_lin + 1);
-    const int nnz = lrp[desc->m_lin];
-    lcol.assign(desc->lin_col, desc->lin_col + nnz);
-    lval.assign(desc->lin_val, desc->lin_val + nnz);
-    std::vector<std::vector<std::pair<int, int>>> cols(n);
-    for (int r = 0; r < desc->m_lin; r++)
-      for (int p = lrp[r]; p < lrp[r + 1]; p++) {
-        if (lcol[p] < 0 || lcol[p] >= n) { sco_destroy(h); return fail(SCO_ERR_ARG, "linear row column out of range"); }
-        cols[lcol[p]].push_back({p, r});
-      }
-    for (int j = 0; j < n; j++) {
-      lcptr[j + 1] = lcptr[j] + (int)cols[j].size();
-      for (auto &pr : cols[j]) { lcentry.push_back(pr.first); lcrow.push_back(pr.second); }
-    }
-    S.nnz_lin = nnz;
-  }
-  std::vector<double> shared_v;
-  if (desc->shared_len > 0 && desc->shared) shared_v.assign(desc->shared, desc->shared + desc->shared_len);
-  // pattern of Psym = (Q + Q') / 2 by column: exact for a shared Q, dense for a per-problem Q, empty without Q; united
-  // with the n_in x n_in block of every objective term
-  std::vector<int> P_cptr(n + 1, 0), P_row;
-  std::vector<int> hv_ptr, hv_src, gq_ptr(n + 1, 0), gq_src;
-  {
-    std::vector<int> pidx((size_t)n * n, -1);  // (i, j) -> pattern entry
-    if (desc->Q.off >= 0)
-      for (int j = 0; j < n; j++)
-        for (int i = 0; i < n; i++) {
-          bool nz = true;
-          if (desc->Q.shared) nz = shared_v[desc->Q.off + (size_t)i * n + j] != 0.0 || shared_v[desc->Q.off + (size_t)j * n + i] != 0.0;
-          if (nz) pidx[(size_t)i * n + j] = 0;
-        }
-    for (int oi = 0; oi < S.n_ob; oi++) {
-      const DevObjBlock &d = S.ob[oi];
-      for (int r = 0; r < d.m; r++) {
-        const int *c = ob_cols.data() + d.coff + (size_t)r * d.n_in;
-        for (int a = 0; a < d.n_in; a++)
-          for (int b = 0; b < d.n_in; b++) pidx[(size_t)c[a] * n + c[b]] = 0;
-      }
-    }
-    for (int j = 0; j < n; j++) {
-      for (int i = 0; i < n; i++)
-        if (pidx[(size_t)i * n + j] >= 0) {
-          pidx[(size_t)i * n + j] = (int)P_row.size();
-          P_row.push_back(i);
-        }
-      P_cptr[j + 1] = (int)P_row.size();
-    }
-    // the term-model entries summed into each pattern entry of P and each entry of q, in term order
-    std::vector<std::vector<int>> hv(P_row.size()), gv(n);
-    for (int oi = 0; oi < S.n_ob; oi++) {
-      const DevObjBlock &d = S.ob[oi];
-      const int nn = d.n_in, ntri = nn * (nn + 1) / 2;
-      for (int r = 0; r < d.m; r++) {
-        const int *c = ob_cols.data() + d.coff + (size_t)r * nn;
-        const int base = d.toff + r * (ntri + nn + 1);
-        for (int a = 0; a < nn; a++) {
-          for (int b = 0; b < nn; b++) {
-            const int lo = std::min(a, b), hi = std::max(a, b);
-            hv[pidx[(size_t)c[a] * n + c[b]]].push_back(base + lo * nn - lo * (lo - 1) / 2 + (hi - lo));
-          }
-          gv[c[a]].push_back(base + ntri + a);
-        }
-      }
-    }
-    hv_ptr.assign(P_row.size() + 1, 0);
-    for (size_t p = 0; p < hv.size(); p++) {
-      hv_ptr[p + 1] = hv_ptr[p] + (int)hv[p].size();
-      hv_src.insert(hv_src.end(), hv[p].begin(), hv[p].end());
-    }
-    for (int j = 0; j < n; j++) {
-      gq_ptr[j + 1] = gq_ptr[j] + (int)gv[j].size();
-      gq_src.insert(gq_src.end(), gv[j].begin(), gv[j].end());
-    }
-    S.nnz_p = (int)P_row.size();
-  }
-  int rc = 0;
-  rc |= upload(h, row_goff, &S.row_goff); rc |= upload(h, row_soff, &S.row_soff);
-  rc |= upload(h, row_w, &S.row_w); rc |= upload(h, row_eq, &S.row_eq);
-  rc |= upload(h, row_gmask, &S.row_gmask); rc |= upload(h, jcol, &S.jcol_g);
-  rc |= upload(h, pc_ptr, &S.pc_ptr); rc |= upload(h, pc_e, &S.pc_e); rc |= upload(h, pc_r, &S.pc_r);
-  rc |= upload(h, lrp, &S.lin_rowptr); rc |= upload(h, lcol, &S.lin_col); rc |= upload(h, lval, &S.lin_val);
-  rc |= upload(h, lcptr, &S.lin_cptr); rc |= upload(h, lcentry, &S.lin_centry); rc |= upload(h, lcrow, &S.lin_crow);
-  rc |= upload(h, shared_v, &S.shared);
-  rc |= upload(h, P_cptr, &S.P_cptr); rc |= upload(h, P_row, &S.P_row);
-  rc |= upload(h, ob_cols, &S.ob_cols); rc |= upload(h, hv_ptr, &S.hv_ptr); rc |= upload(h, hv_src, &S.hv_src);
-  rc |= upload(h, gq_ptr, &S.gq_ptr); rc |= upload(h, gq_src, &S.gq_src);
-  {
-    int bw = 0;
+  to_csc(n, ix.jcol, ix.row_goff, ix.row_soff, ix.row_w, ix.pc_ptr, ix.pc_e, ix.pc_r);
+  // ---- linear rows
+  ix.lrp.assign(1, 0);  // without linear rows the CSR arrays may be null
+  if (desc->m_lin > 0) ix.lrp.assign(desc->lin_rowptr, desc->lin_rowptr + desc->m_lin + 1);
+  S.nnz_lin = ix.lrp[desc->m_lin];
+  ix.lcol.assign(desc->lin_col, desc->lin_col + S.nnz_lin);
+  ix.lval.assign(desc->lin_val, desc->lin_val + S.nnz_lin);
+  for (int r = 0; r < desc->m_lin; r++) ix.lin_w.push_back(ix.lrp[r + 1] - ix.lrp[r]);
+  to_csc(n, ix.lcol, ix.lrp, ix.lrp, ix.lin_w, ix.lcptr, ix.lcentry, ix.lcrow);
+  if (desc->shared_len > 0 && desc->shared) ix.shared.assign(desc->shared, desc->shared + desc->shared_len);
+  // ---- pattern of Psym = (Q + Q') / 2 by column: exact for a shared Q, dense for a per-problem Q, empty without Q;
+  // united with the n_in x n_in block of every objective term (marked above)
+  ix.P_cptr.assign(n + 1, 0);
+  if (desc->Q.off >= 0)
     for (int j = 0; j < n; j++)
-      for (int p = P_cptr[j]; p < P_cptr[j + 1]; p++) bw = std::max(bw, std::abs(P_row[p] - j));
-    for (int r = 0; r < desc->m_lin; r++)
-      if (lrp[r + 1] > lrp[r]) {
-        int lo = n, hi = -1;
-        for (int p = lrp[r]; p < lrp[r + 1]; p++) { lo = std::min(lo, lcol[p]); hi = std::max(hi, lcol[p]); }
-        bw = std::max(bw, hi - lo);
+      for (int i = 0; i < n; i++)
+        if (!desc->Q.shared || ix.shared[desc->Q.off + (size_t)i * n + j] != 0.0 || ix.shared[desc->Q.off + (size_t)j * n + i] != 0.0)
+          pidx[(size_t)i * n + j] = 0;
+  for (int j = 0; j < n; j++) {
+    for (int i = 0; i < n; i++)
+      if (pidx[(size_t)i * n + j] >= 0) {
+        pidx[(size_t)i * n + j] = (int)ix.P_row.size();
+        ix.P_row.push_back(i);
       }
-    for (int i = 0; i < m_nl; i++)
-      if (row_w[i] > 0) {
-        int lo = n, hi = -1;
-        for (int k = 0; k < row_w[i]; k++) { lo = std::min(lo, jcol[row_goff[i] + k]); hi = std::max(hi, jcol[row_goff[i] + k]); }
-        bw = std::max(bw, hi - lo);
-      }
-    S.s_bw = std::min(bw, n - 1);
-    // thread-per-entity ADMM loop (sco_qp.cuh: fast_role keeps SCO_EN = 8 row entries / SCO_EH = 4 + 4 column entries
-    // in registers and has no path for more)
-    bool ok = true;
-    for (int r = 0; r < desc->m_lin; r++) ok = ok && lrp[r + 1] - lrp[r] <= 8;
-    for (int i = 0; i < m_nl; i++) ok = ok && row_w[i] <= 8;
-    for (int j = 0; j < n; j++) ok = ok && lcptr[j + 1] - lcptr[j] <= 4 && pc_ptr[j + 1] - pc_ptr[j] <= 4;
-    S.fast_ok = ok ? 1 : 0;
-    bool narrow = true;
-    for (int j = 0; j < n; j++) narrow = narrow && P_cptr[j + 1] - P_cptr[j] <= 4;
-    S.p_narrow = narrow ? 1 : 0;
-    bool dense = desc->m_lin == 0 && n <= 32 && m_nl > 0 && m_nl <= 48;
-    for (int i = 0; i < m_nl; i++) dense = dense && row_w[i] == n;
-    dense = dense && !any_map;  // its kernels assume rows over all n variables in column order
-    S.fast_dense = dense && !ok ? 1 : 0;
+    ix.P_cptr[j + 1] = (int)ix.P_row.size();
   }
-  if (rc) { sco_destroy(h); return SCO_ERR_CUDA; }
+  S.nnz_p = (int)ix.P_row.size();
+  // the term-model entries summed into each pattern entry of P and each entry of q, in term order
+  std::vector<std::vector<int>> hv(ix.P_row.size()), gv(n);
+  for (int oi = 0; oi < S.n_ob; oi++) {
+    const DevObjBlock &d = S.ob[oi];
+    const int nn = d.n_in, ntri = nn * (nn + 1) / 2;
+    for (int r = 0; r < d.m; r++) {
+      const int *c = ix.ob_cols.data() + d.coff + (size_t)r * nn;
+      const int base = d.toff + r * (ntri + nn + 1);
+      for (int a = 0; a < nn; a++) {
+        for (int b = 0; b < nn; b++) {
+          const int lo = std::min(a, b), hi = std::max(a, b);
+          hv[pidx[(size_t)c[a] * n + c[b]]].push_back(base + lo * nn - lo * (lo - 1) / 2 + (hi - lo));
+        }
+        gv[c[a]].push_back(base + ntri + a);
+      }
+    }
+  }
+  flatten(hv, ix.hv_ptr, ix.hv_src);
+  flatten(gv, ix.gq_ptr, ix.gq_src);
+  // ---- structural half-bandwidth of S = P + A'RA
+  int bw = 0;
+  for (int j = 0; j < n; j++)
+    for (int p = ix.P_cptr[j]; p < ix.P_cptr[j + 1]; p++) bw = std::max(bw, std::abs(ix.P_row[p] - j));
+  for (int r = 0; r < desc->m_lin; r++) bw = std::max(bw, col_span(ix.lcol, ix.lrp[r], ix.lin_w[r]));
+  for (int i = 0; i < m_nl; i++) bw = std::max(bw, col_span(ix.jcol, ix.row_goff[i], ix.row_w[i]));
+  S.s_bw = std::min(bw, n - 1);
+}
+
+// The ADMM loop a structure takes (fast_ok, p_narrow, fast_dense, dense_kind), its team size and its shared-memory
+// layout (sws when S has to move out).  Refuses a structure whose working set does not fit shared memory.
+static int choose_paths(const sco_structure_desc *desc, HostStruct &ix, size_t smem_optin) {
+  DevStruct &S = ix.S;
+  const int n = S.n, m_nl = S.m_nl;
+  // thread-per-entity ADMM loop (sco_qp.cuh: fast_role keeps SCO_EN = 8 row entries / SCO_EH = 4 + 4 column entries
+  // in registers and has no path for more)
+  bool ok = true;
+  for (int w : ix.lin_w) ok = ok && w <= 8;
+  for (int w : ix.row_w) ok = ok && w <= 8;
+  for (int j = 0; j < n; j++) ok = ok && ix.lcptr[j + 1] - ix.lcptr[j] <= 4 && ix.pc_ptr[j + 1] - ix.pc_ptr[j] <= 4;
+  S.fast_ok = ok ? 1 : 0;
+  bool narrow = true;
+  for (int j = 0; j < n; j++) narrow = narrow && ix.P_cptr[j + 1] - ix.P_cptr[j] <= 4;
+  S.p_narrow = narrow ? 1 : 0;
+  bool dense = desc->m_lin == 0 && n <= 32 && m_nl > 0 && m_nl <= 48;
+  for (int w : ix.row_w) dense = dense && w == n;
+  dense = dense && !ix.any_map;  // its kernels assume rows over all n variables in column order
+  S.fast_dense = dense && !ok ? 1 : 0;
   // ---- dense fast path: one dense hinge block over all variables, no linear rows, sizes within the instantiated table
-  S.dense_kind = 0;
   if (desc->m_lin == 0 && S.n_ob == 0 && desc->n_blocks == 1 && desc->blocks[0].family == SCO_FAM_QUADFORM &&
-      desc->blocks[0].cnt_type == SCO_CNT_LEQ && !any_map) {
+      desc->blocks[0].cnt_type == SCO_CNT_LEQ && !ix.any_map) {
     static const int table[][2] = {{8, 6}, {12, 16}, {20, 30}, {32, 32}};  // keep in sync with QPSolver::solve in sco_qp.cuh
     for (int k = 0; k < 4; k++)
       if (n <= table[k][0] && m_nl <= table[k][1]) { S.dense_kind = k + 1; break; }
@@ -523,58 +495,85 @@ extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle
   // ---- team size and shared-memory layout
   const int work = std::max(std::max(n, m_nl), desc->m_lin);
   int team = work <= 40 ? 32 : work <= 96 ? 64 : work <= 192 ? 128 : 256;
-  {
-    // one thread per entity (variable / linear row / penalty row) is what the fast ADMM loop wants (sco_qp.cuh:
-    // fast_loop); structures with more than 512 entities stay on the strided shared-memory loop
-    // (every role starts on a warp boundary)
-    const int entities = ((n + 31) & ~31) + ((desc->m_lin + 31) & ~31) + ((m_nl + 31) & ~31);
-    if (entities <= 512) team = entities <= 32 ? 32 : entities <= 64 ? 64 : entities <= 128 ? 128 : entities <= 256 ? 256 : 512;
-  }
+  // one thread per entity (variable / linear row / penalty row) is what the fast ADMM loop wants (sco_qp.cuh:
+  // fast_loop); structures with more than 512 entities stay on the strided shared-memory loop
+  // (every role starts on a warp boundary)
+  const int entities = ((n + 31) & ~31) + ((desc->m_lin + 31) & ~31) + ((m_nl + 31) & ~31);
+  if (entities <= 512) team = entities <= 32 ? 32 : entities <= 64 ? 64 : entities <= 128 ? 128 : entities <= 256 ? 256 : 512;
   if (S.dense_kind) team = 64;  // two warps per problem: rows | variables (sco_dense.cuh)
+  ix.team = team;
   for (;;) {
     build_layout(S, team);
-    h->smem_bytes = (size_t)(S.L.total + ((n + 1) & ~1)) * sizeof(double);
-    if (h->smem_bytes <= (size_t)prop.sharedMemPerBlockOptin) break;
-    if (!S.sws && !S.dense_kind && !S.n_ob) {  // objective terms stay in the resident regime
-      // the n x n matrix S (and its inverse) moves to a global workspace per resident team: the ADMM loop streams it
-      // from L2 / HBM in every iteration (strided loop only); everything else stays in shared memory
-      S.sws = n * n;
-      continue;
-    }
-    sco_destroy(h);
-    return fail(SCO_ERR_UNSUPPORTED, "problem working set (%zu B) exceeds shared memory per block (%zu B)",
-                h->smem_bytes, (size_t)prop.sharedMemPerBlockOptin);
+    ix.smem_bytes = (size_t)(S.L.total + ((n + 1) & ~1)) * sizeof(double);
+    if (ix.smem_bytes <= smem_optin) return 0;
+    if (S.sws || S.dense_kind || S.n_ob)  // objective terms stay in the resident regime
+      return fail(SCO_ERR_UNSUPPORTED, "problem working set (%zu B) exceeds shared memory per block (%zu B)",
+                  ix.smem_bytes, smem_optin);
+    // the n x n matrix S (and its inverse) moves to a global workspace per resident team: the ADMM loop streams it
+    // from L2 / HBM in every iteration (strided loop only); everything else stays in shared memory
+    S.sws = n * n;
   }
-  h->team = team;
+}
+
+// Uploads, kernel selection and configuration, launch-slot and staging scratch.  On failure the caller destroys h.
+static int setup_device(sco_handle *h, const HostStruct &ix) {
+  DevStruct &S = h->S = ix.S;
+  h->team = ix.team;
+  h->smem_bytes = ix.smem_bytes;
+  int rc = 0;
+  rc |= upload(h, ix.row_goff, &S.row_goff); rc |= upload(h, ix.row_soff, &S.row_soff);
+  rc |= upload(h, ix.row_w, &S.row_w); rc |= upload(h, ix.row_eq, &S.row_eq);
+  rc |= upload(h, ix.row_gmask, &S.row_gmask); rc |= upload(h, ix.jcol, &S.jcol_g);
+  rc |= upload(h, ix.pc_ptr, &S.pc_ptr); rc |= upload(h, ix.pc_e, &S.pc_e); rc |= upload(h, ix.pc_r, &S.pc_r);
+  rc |= upload(h, ix.lrp, &S.lin_rowptr); rc |= upload(h, ix.lcol, &S.lin_col); rc |= upload(h, ix.lval, &S.lin_val);
+  rc |= upload(h, ix.lcptr, &S.lin_cptr); rc |= upload(h, ix.lcentry, &S.lin_centry); rc |= upload(h, ix.lcrow, &S.lin_crow);
+  rc |= upload(h, ix.shared, &S.shared);
+  rc |= upload(h, ix.P_cptr, &S.P_cptr); rc |= upload(h, ix.P_row, &S.P_row);
+  rc |= upload(h, ix.ob_cols, &S.ob_cols); rc |= upload(h, ix.hv_ptr, &S.hv_ptr); rc |= upload(h, ix.hv_src, &S.hv_src);
+  rc |= upload(h, ix.gq_ptr, &S.gq_ptr); rc |= upload(h, ix.gq_src, &S.gq_src);
+  if (rc) return SCO_ERR_CUDA;
+  const int team = ix.team;
   h->gen_ops = team == 32 ? sco_team_ops_32() : team == 64 ? sco_team_ops_64() : team == 128 ? sco_team_ops_128()
                : team == 256 ? sco_team_ops_256() : sco_team_ops_512();
   h->ops = h->gen_ops;
   if (S.dense_kind)
     h->ops = S.dense_kind == 1 ? sco_dense_ops_1() : S.dense_kind == 2 ? sco_dense_ops_2() : S.dense_kind == 3 ? sco_dense_ops_3() : sco_dense_ops_4();
-  {
-    int occ = 0;
-    cudaError_t ce = h->gen_ops->configure(h->smem_bytes, &occ, &h->carve_gen);
-    h->carve_ops = h->carve_gen;
-    if (ce == cudaSuccess && h->ops != h->gen_ops) ce = h->ops->configure(h->smem_bytes, &occ, &h->carve_ops);
-    if (ce != cudaSuccess) {
-      sco_destroy(h);
-      return fail(SCO_ERR_CUDA, "kernel configuration failed: %s", cudaGetErrorString(ce));
-    }
-    h->occupancy = std::max(occ, 1);
-  }
+  int occ = 0;
+  cudaError_t ce = h->gen_ops->configure(h->smem_bytes, &occ, &h->carve_gen);
+  h->carve_ops = h->carve_gen;
+  if (ce == cudaSuccess && h->ops != h->gen_ops) ce = h->ops->configure(h->smem_bytes, &occ, &h->carve_ops);
+  if (ce != cudaSuccess) return fail(SCO_ERR_CUDA, "kernel configuration failed: %s", cudaGetErrorString(ce));
+  h->occupancy = std::max(occ, 1);
   h->Jscr_ctas = (size_t)h->sm_count * h->occupancy;
   bool ok = cudaMalloc(&h->counter, sco_handle::NSLOT * sizeof(unsigned long long)) == cudaSuccess &&
             cudaMalloc(&h->order_err, sco_handle::NSLOT * sizeof(int)) == cudaSuccess;
   for (int k = 0; k < sco_handle::NSLOT && ok; k++)
-    ok = cudaMalloc(&h->Jscr[k], std::max<size_t>(h->Jscr_ctas * (size_t)std::max(jnnz + S.sws, 1), 1) * sizeof(double)) == cudaSuccess &&
+    ok = cudaMalloc(&h->Jscr[k], std::max<size_t>(h->Jscr_ctas * (size_t)std::max(S.jnnz + S.sws, 1), 1) * sizeof(double)) == cudaSuccess &&
          cudaEventCreateWithFlags(&h->slot_done[k], cudaEventDisableTiming) == cudaSuccess;
   for (int k = 0; k < sco_handle::NSTG && ok; k++)
     ok = cudaEventCreateWithFlags(&h->stg[k].done, cudaEventDisableTiming) == cudaSuccess;
-  if (!ok) {
-    sco_destroy(h);
-    return fail(SCO_ERR_CUDA, "cudaMalloc of scratch failed");
-  }
-  *out = h;
+  if (!ok) return fail(SCO_ERR_CUDA, "cudaMalloc of scratch failed");
+  return SCO_OK;
+}
+
+extern "C" int sco_create(const sco_structure_desc *desc, int device, sco_handle **out) {
+  if (!desc || !out) return fail(SCO_ERR_ARG, "null argument");
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail(SCO_ERR_CUDA, "no CUDA device: the engine has no CPU fallback");
+  if (device < 0 || device >= ndev) return fail(SCO_ERR_ARG, "device %d out of range", device);
+  if (int rc = check_desc(desc)) return rc;
+  CUDA_TRY(cudaSetDevice(device));
+  cudaDeviceProp prop;
+  CUDA_TRY(cudaGetDeviceProperties(&prop, device));
+  if (prop.major != 10) return fail(SCO_ERR_CUDA, "device is sm_%d%d; this library is built for sm_100a only", prop.major, prop.minor);
+  HostStruct ix;
+  build_index(desc, ix);
+  if (int rc = choose_paths(desc, ix, (size_t)prop.sharedMemPerBlockOptin)) return rc;
+  std::unique_ptr<sco_handle, decltype(&sco_destroy)> h(new sco_handle(), &sco_destroy);  // released on success
+  h->device = device; h->sm_count = prop.multiProcessorCount;
+  if (int rc = setup_device(h.get(), ix)) return rc;
+  *out = h.release();
   return SCO_OK;
 }
 

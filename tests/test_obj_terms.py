@@ -96,9 +96,14 @@ def test_subset_in_permuted_order_and_two_input_counts():
 def test_legacy_objective_keeps_its_fields_and_signature():
     for n in (20, 40):
         for analytic in (False, True):
-            st, _, _, _ = _compile([CAPS.build_chain(p, analytic=analytic)[0] for p in CAPS.chain_points(2, n)])
+            st, params, _, cps = _compile([CAPS.build_chain(p, analytic=analytic)[0] for p in CAPS.chain_points(2, n)])
             assert st.obj_prog_len > 0 and st.obj_blocks == [] and st.obj_prog_flags == int(analytic)
             assert hashlib.sha256(repr(batch.signature(st)).encode()).hexdigest() == SIGNATURES[(n, analytic)]
+            for c, row in zip(cps, params):  # the program of the one-term block is the term's own
+                (pk, _), = c.obj_blocks
+                (term,) = pk.parts
+                assert np.array_equal(pk.params(), term.params())
+                assert np.array_equal(st.get(st.obj_prog, row, 1 + 2 * st.obj_prog_len), term.params())
 
 
 def test_refusals_name_their_limit():
